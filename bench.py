@@ -2,7 +2,7 @@
 """bench.py — controller-steps/sec of the batched CLIK controller step on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--scenario ur5_track] [--batch 1048576] [--no-secondary]
+                    [--scenario ur5_track] [--batch 1048576] [--no-secondary] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (PseudoInverseController.solve for every instance of the
 batch — reference casclik/controllers/pseudo_inverse.py:512-556) over one batch of synthetic
@@ -21,6 +21,10 @@ a global batch of 2^23 sharded over the ranks — each with its own roofline and
 
 `--impl reference` times the restated reference CPU path (oracle/clik_oracle.c, all host
 threads) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<name>.npy, so that two
+builds run with the same arguments (same seeded inputs) can be compared output for output; see
+dump_outputs.
 """
 import argparse
 import json
@@ -275,7 +279,7 @@ def _bytes_per_set(meta, is_qp, B):
 def time_device_resident(torch, dist, ctrl, scenario, B, steps, warm, rank, world, dev, min_sets=2,
                          seed_base=1000, overlap=2, plain_too=True, n_streams=1):
     """K steps of solve_batch on device-resident inputs -> (ms total max-over-ranks, n_sets, graph?, step,
-    ms of the same K steps in plain stream order | None).
+    ms of the same K steps in plain stream order | None, output buffers of the last timed step).
     Inputs and outputs rotate over enough sets to exceed L2 twice over."""
     meta = ctrl.kernel_meta
     is_qp = scenario.controller == "qp"
@@ -378,7 +382,7 @@ def time_device_resident(torch, dist, ctrl, scenario, B, steps, warm, rank, worl
             ctrl.set_input_staging(True)
         side[:] = keep
     ms, graphed = timed(overlap)
-    return ms, n_sets, graphed, step, ms_plain
+    return ms, n_sets, graphed, step, ms_plain, outs[(steps - 1) % n_sets]
 
 
 def rooflines(meta, is_qp, B, sec_per_step, hbm_peak, hbm_src, fp64_peak, counts):
@@ -422,6 +426,26 @@ def rooflines(meta, is_qp, B, sec_per_step, hbm_peak, hbm_src, fp64_peak, counts
     return max(cands, key=lambda r: r["frac"]), detail
 
 
+DUMP_LIMIT = 64 * 10 ** 6     # bytes written by --dump-outputs in all
+
+
+def dump_outputs(directory, arrays):
+    """{name: host array (rows, N) or (N,)} -> directory/<name>.npy in float64 (int32 modes, statuses and
+    active-set bit masks are exact in it).  When all N instances would exceed DUMP_LIMIT, the same fixed,
+    seeded sample of instance columns is written for every array, and its indices as instances.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items() if v is not None}
+    N = next(iter(arrays.values())).shape[-1]
+    rows = sum(1 if a.ndim == 1 else a.shape[0] for a in arrays.values())
+    if 8 * rows * N > DUMP_LIMIT:
+        keep = DUMP_LIMIT // (8 * (rows + 1))
+        idx = np.sort(np.random.default_rng(0).choice(N, size=keep, replace=False))
+        arrays = {k: a[..., idx] for k, a in arrays.items()}
+        arrays["instances"] = idx.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -442,7 +466,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the other BASELINE configs")
     ap.add_argument("--secondary-only", default="", help="(profiling) run only this secondary scenario's timed loop")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -496,9 +524,9 @@ def main():
             Bs = batch
         per = _bytes_per_set(c.kernel_meta, qp, Bs)
         k = int(max(8, min(100, (3 << 30) // max(per, 1))))          # ~3 GB of algorithmic traffic per leg
-        ms_tot, n_sets, graphed, _, ms_plain = time_device_resident(torch, dist, c, sc, Bs, k, 3, rank, world, dev,
-                                                                    seed_base=2000, overlap=args.overlap,
-                                                                    n_streams=args.streams)
+        ms_tot, n_sets, graphed, _, ms_plain, _ = time_device_resident(torch, dist, c, sc, Bs, k, 3, rank, world, dev,
+                                                                       seed_base=2000, overlap=args.overlap,
+                                                                       n_streams=args.streams)
         total = batch if mode == "strong" else batch * world
         val = total * k / (ms_tot * 1e-3)
         out = {"config": cfg, "workload": sc.description, "value": val, "unit": UNIT,
@@ -536,10 +564,14 @@ def main():
     # on the data path — instances are independent (SURVEY.md §8e)
     sampler = ClockSampler(local)
     sampler.start()
-    ms, n_sets, graphed, step, ms_plain = time_device_resident(torch, dist, ctrl, scenario, B, args.steps, args.warmup,
-                                                               rank, world, dev, min_sets=max(args.sets, 2),
-                                                               overlap=args.overlap, n_streams=args.streams)
+    ms, n_sets, graphed, step, ms_plain, last = time_device_resident(
+        torch, dist, ctrl, scenario, B, args.steps, args.warmup, rank, world, dev, min_sets=max(args.sets, 2),
+        overlap=args.overlap, n_streams=args.streams)
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # now, before the e2e loop and the untimed load steps below reuse the step buffers
+        names = ("sol", "status", "active") if is_qp else ("robot_vel", "virtual_vel", "mode")
+        dump_outputs(args.dump_outputs, {k: None if a is None else a.cpu().numpy() for k, a in zip(names, last)})
 
     # ---- end to end through the host-buffer C ABI (pinned host inputs, copies inside) --------------
     inp = scenario.sample(B, seed=1000 * rank + 77)
@@ -631,7 +663,7 @@ def main():
                                       "ms_per_step": ms_plain / args.steps}
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"], _, _ = CpuPort(scenario).measure(B, seconds_target=12.0)
-    del step
+    del step, last
     torch.cuda.empty_cache()
 
     # ---- the other BASELINE configs, same run, same timing rules ---------------------------------------

@@ -84,25 +84,27 @@ class RefSkill(ctypes.Structure):
 
 EVAL_DECL = "double t, const double* q, const double* x, const double* y"
 
+_evals = {}
+
 
 def _compile_eval(nodes, names, tag):
     """Expression graph -> plain C (the emitter's C flavour: what CasADi's code generator + `jit` do in
-    the reference) -> gcc -O2 -> function pointer `void ev(t, q, x, y, out)`."""
+    the reference) -> gcc -O2 -> function pointer `void ev(t, q, x, y, out)`.  Compiled in a temporary
+    directory that is gone once the library is loaded (bench.py runs from trees it may not write to);
+    cached per process on the source."""
     import hashlib
+    import tempfile
     from casclik_b200.codegen import emit_c_function
     src = emit_c_function("ev", names, nodes, EVAL_DECL)
-    key = hashlib.sha256(src.encode()).hexdigest()[:16]
-    build_dir = os.path.join(HERE, "_build")
-    os.makedirs(build_dir, exist_ok=True)
-    so = os.path.join(build_dir, "eval_%s_%s.so" % (tag, key))
-    if not os.path.exists(so):
-        c = so[:-3] + ".c"
-        with open(c, "w") as f:
-            f.write(src)
-        tmp = so + ".tmp%d" % os.getpid()
-        subprocess.run(["gcc", "-O2", "-shared", "-fPIC", "-o", tmp, c, "-lm"], check=True)
-        os.replace(tmp, so)
-    lib = ctypes.CDLL(so)
+    key = hashlib.sha256(src.encode()).hexdigest()
+    if key not in _evals:
+        with tempfile.TemporaryDirectory(prefix="clik_oracle_eval_") as tmp:
+            c, so = os.path.join(tmp, "eval_%s.c" % tag), os.path.join(tmp, "eval_%s.so" % tag)
+            with open(c, "w") as f:
+                f.write(src)
+            subprocess.run(["gcc", "-O2", "-shared", "-fPIC", "-o", so, c, "-lm"], check=True)
+            _evals[key] = ctypes.CDLL(so)
+    lib = _evals[key]
     return lib, ctypes.cast(lib.ev, ctypes.c_void_p)
 
 

@@ -1,9 +1,12 @@
 """bench.py's reference arm runs on host cores only, so its side of the JSON contract can be checked
-without a GPU: one JSON line, the required keys, rank != 0 silent under a multi-rank launch."""
+without a GPU: one JSON line, the required keys, rank != 0 silent under a multi-rank launch.  So can the
+host side of --dump-outputs and the argument checks."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -46,3 +49,33 @@ def test_reference_arm_only_rank_zero_works_under_a_multi_rank_launch():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, "--gpus", "2", "--no-secondary") == []
     lines = _run({"RANK": "0", "WORLD_SIZE": "2", "LOCAL_RANK": "0"}, "--gpus", "2", "--no-secondary")
     assert len(lines) == 1 and json.loads(lines[0])["n_gpus"] == 2
+
+
+def test_dump_outputs_writes_float64_and_samples_the_same_instances_when_too_large(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(1)
+    vel, mode = rng.standard_normal((6, 5000)), rng.integers(0, 4, 5000).astype(np.int32)
+    bench.dump_outputs(str(tmp_path / "all"), {"robot_vel": vel, "virtual_vel": None, "mode": mode})
+    assert sorted(os.listdir(tmp_path / "all")) == ["mode.npy", "robot_vel.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "robot_vel.npy"), vel)
+    got = np.load(tmp_path / "all" / "mode.npy")
+    assert got.dtype == np.float64 and np.array_equal(got, mode)
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 8 * 8 * 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"robot_vel": vel, "mode": mode})
+    total = sum(os.path.getsize(tmp_path / "a" / f) - 128 for f in os.listdir(tmp_path / "a"))
+    assert total <= bench.DUMP_LIMIT
+    idx = np.load(tmp_path / "a" / "instances.npy").astype(np.int64)
+    assert len(idx) == 1000 and np.array_equal(idx, np.unique(idx))
+    assert np.array_equal(np.load(tmp_path / "a" / "robot_vel.npy"), vel[:, idx])
+    assert np.array_equal(np.load(tmp_path / "a" / "mode.npy"), mode[idx])
+    for f in os.listdir(tmp_path / "a"):
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
+
+
+def test_steps_below_one_is_refused():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                       text=True, timeout=600)
+    assert p.returncode == 2 and "--steps" in p.stderr
