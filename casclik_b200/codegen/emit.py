@@ -32,9 +32,13 @@ def literal(v: float) -> str:
 class Emitter(object):
     """Emits the statements computing a set of nodes, sharing temporaries across calls."""
 
-    def __init__(self, sym_names, const_table=None, sincos_name="sincos"):
+    def __init__(self, sym_names, const_table=None, sincos_name="sincos", leaves=None):
         self.sym_names = sym_names
         self.name = {}        # node id -> C expression (temp name, symbol name or literal)
+        # computed nodes that are inputs of this program (node id -> C lvalue): used as they are, never
+        # expanded (the NLP cost functions read the decision-free values eval_nlp_pre hoisted)
+        self.leaves = dict(leaves or {})
+        self.name.update(self.leaves)
         self.lines = []
         self.counter = 0
         self.hist = {}
@@ -54,6 +58,8 @@ class Emitter(object):
         return "KC[%d]" % self.const_table.index(v)
 
     def _ref(self, n):
+        if n.id in self.leaves:          # (before symbols: a hoisted input row t / q / x / y is a leaf too)
+            return self.leaves[n.id]
         if n.op == "const":
             return self._const(n.val)
         if n.op == "sym":
@@ -69,7 +75,7 @@ class Emitter(object):
         pending = [n for n in outputs if n.op not in ("const", "sym") and n.id not in self.name]
         if not pending:
             return
-        order = [n for n in dag.topo(pending) if n.op not in ("const", "sym") and n.id not in self.name]
+        order = [n for n in self._topo(pending) if n.op not in ("const", "sym") and n.id not in self.name]
         # pair sin/cos of the same argument into one sincos call
         by_arg = {}
         for n in order:
@@ -132,6 +138,19 @@ class Emitter(object):
             t = self._tmp()
             self.lines.append("const double %s = %s;" % (t, rhs))
             self.name[n.id] = t
+
+    def _topo(self, outputs):
+        if not self.leaves:
+            return dag.topo(outputs)
+        seen, stack = {}, list(outputs)
+        while stack:
+            n = stack.pop()
+            if n.id in seen:
+                continue
+            seen[n.id] = n
+            if n.id not in self.leaves:
+                stack.extend(n.args)
+        return [seen[k] for k in sorted(seen)]
 
     def assign(self, lhs, node):
         self.require([node])
@@ -319,12 +338,18 @@ def _switch(name, values, ret="int"):
             % (ret, name, body))
 
 
-def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None):
-    """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None.
+def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None,
+               nlp=None, nlp_tol=1e-10):
+    """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None; or `nlp`:
+    NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).
     Tuning knobs (also settable through the environment for experiments): CLIK_BLOCK,
     CLIK_MINBLOCKS, CLIK_CONSTBANK (1), CLIK_FAST_SINCOS (1)."""
     if block_threads is None:
         block_threads = int(os.environ.get("CLIK_BLOCK", "128"))
+    if nlp is not None:
+        if pinv is not None or qp is not None:
+            raise ValueError("an NLP image holds the NLP kernels only")
+        return _emit_nlp(nlp, label, block_threads, nlp_tol)
     env_min_blocks = int(os.environ.get("CLIK_MINBLOCKS", "0"))
     if min_blocks is None:
         min_blocks = env_min_blocks
@@ -704,6 +729,130 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     out.append("  " + " ".join("o[%d] = (int)0x%xu;" % (8 + k, v) for k, v in enumerate(tuple(pm) + tuple(qm))))
     out.append("  o[16] = %d; o[17] = %s;" % (meta.get("pinv_static_modes", 1),
                                              "clik::GroupGeometry<Skill>::BLOCK" if meta.get("pinv_group") else "0"))
+    out.append("}")
+    return "\n".join(out) + "\n", meta
+
+
+def nlp_hoisted(nlp):
+    """The maximal decision-free subexpressions the cost graph (F, g, H) consumes: every non-constant
+    argument without a decision symbol below it of a node that has one, and every output without one.
+    eval_nlp_pre computes them once per step; the SQP iteration only reads them."""
+    dec = {n.id for n in nlp.dec}
+    outs = [nlp.F] + list(nlp.g) + list(nlp.H)
+    dep = {}
+    for n in dag.topo(outs):
+        dep[n.id] = n.id in dec or any(dep[a.id] for a in n.args)
+    P, seen = [], set()
+
+    def want(n):
+        if n.op != "const" and not dep[n.id] and n.id not in seen:
+            seen.add(n.id)
+            P.append(n)
+    for n in dag.topo(outs):
+        if dep[n.id]:
+            for a in n.args:
+                want(a)
+    for o in outs:
+        want(o)
+    return P
+
+
+def _emit_nlp(nlp, label, block_threads, tol):
+    """Translation unit of the reactive-NLP controller (csrc/clik_nlp.cuh instantiated on the skill)."""
+    const_table = [] if os.environ.get("CLIK_CONSTBANK", "1") == "1" else None
+    sincos_name = "clik::sincos_fast" if os.environ.get("CLIK_FAST_SINCOS", "1") == "1" else "sincos"
+    nq, nxv, ny, nx, m = nlp.n_rob, nlp.n_virt, nlp.n_in, nlp.nx, nlp.m
+    P = nlp_hoisted(nlp)
+    npar = len(P)
+    meta = {"label": label, "n_robot": nq, "n_virtual": nxv, "n_input": ny,
+            "has_pinv": False, "has_qp": False, "has_nlp": True,
+            "n_modes": 1, "qp_n": nx, "qp_m": m, "block_threads": block_threads,
+            "nlp_quadratic": bool(nlp.quadratic), "nlp_hoisted": npar, "nlp_tol": float(tol)}
+    out = ["// generated by casclik_b200.codegen for skill %r -- do not edit" % label,
+           '#include "clik_math.cuh"',
+           '#include "clik_qp.cuh"',
+           '#include "clik_nlp.cuh"',
+           ""]
+    pre_struct = []
+    struct_at = len(out)
+    out.append("struct Skill {")
+    out.append("  static constexpr int NQ = %d, NX = %d, NY = %d, NS = %d;" % (nq, nxv, ny, nq + nxv))
+    out.append("  static constexpr int BLOCK = %d;   // threads per CTA of the step kernels" % block_threads)
+    out.append("  static constexpr int NN = %d, NM = %d, NP = %d;   // decision variables, rows, hoisted values"
+               % (nx, m, npar))
+    out.append("  static constexpr bool NLP_QUADRATIC = %s;   // Hessian free of decision variables: one subproblem"
+               % ("true" if nlp.quadratic else "false"))
+    out.append("  static constexpr double NLP_TOL = %s;" % literal(float(tol)))
+    out.append("  static constexpr int NLP_QP_ITER = %d;   // iteration cap of each subproblem" % (10 * (nx + m)))
+    sig = ("const double t, const double (&q)[%d], const double (&x)[%d], const double (&y)[%d]"
+           % (max(nq, 1), max(nxv, 1), max(ny, 1)))
+    # once per step: the constraint rows and the hoisted values
+    em = Emitter(nlp.syms.names, const_table, sincos_name)
+    for r in range(m):
+        for j in range(nx):
+            em.assign("d.A[%d]" % (r * nx + j), nlp.A[r][j])
+        em.assign("d.lb[%d]" % r, nlp.lb[r])
+        em.assign("d.ub[%d]" % r, nlp.ub[r])
+    for k, n in enumerate(P):
+        em.assign("d.P[%d]" % k, n)
+    out.append("  __device__ static __forceinline__ void eval_nlp_pre(%s, clik::NlpData<Skill>& d) {" % sig)
+    out += ["    " + ln for ln in em.finish()]
+    out.append("  }")
+    meta["nlp_read_masks"] = em.read_masks(nlp.syms)
+    pre_counts = em.counts()
+    # per SQP iteration / line-search trial: F (and g, H) from the decision variables and the hoisted values
+    dec_names = {n.id: "v[%d]" % j for j, n in enumerate(nlp.dec)}
+    leaves = {n.id: "P[%d]" % k for k, n in enumerate(P)}
+    psig = "const double (&P)[%d], const double (&v)[%d]" % (max(npar, 1), nx)
+    emf = Emitter(dec_names, const_table, sincos_name, leaves=leaves)
+    emf.assign("f_", nlp.F)
+    out.append("  __device__ static __forceinline__ double eval_nlp_f(%s) {" % psig)
+    out.append("    double f_;")
+    out += ["    " + ln for ln in emf.finish()]
+    out.append("    return f_;")
+    out.append("  }")
+    emg = Emitter(dec_names, const_table, sincos_name, leaves=leaves)
+    emg.assign("f_", nlp.F)
+    for j in range(nx):
+        emg.assign("g[%d]" % j, nlp.g[j])
+    for k, n in enumerate(nlp.H):
+        emg.assign("H[%d]" % k, n)
+    out.append("  __device__ static __forceinline__ double eval_nlp_fgH(%s, double (&g)[%d], double (&H)[%d]) {"
+               % (psig, nx, nx * (nx + 1) // 2))
+    out.append("    double f_;")
+    out += ["    " + ln for ln in emg.finish()]
+    out.append("    return f_;")
+    out.append("  }")
+    meta["nlp_eval"] = {"pre": pre_counts, "f": emf.counts(), "fgH": emg.counts()}
+    out.append("  static constexpr unsigned NLP_READ_T = %du, NLP_READ_Q = 0x%xu, NLP_READ_X = 0x%xu, NLP_READ_Y = 0x%xu;"
+               % meta["nlp_read_masks"])
+    meta["nlp_inputs_read"] = em.inputs_read()
+    out.append("};")
+    out.append("")
+    if const_table:
+        pre_struct.append("__constant__ double KC[%d] = {%s};" % (
+            len(const_table), ", ".join(literal(v) for v in const_table)))
+    out[struct_at:struct_at] = pre_struct
+    out.append('extern "C" __global__ void __launch_bounds__(%d) clik_nlp_kernel(' % block_threads)
+    out.append("    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,")
+    out.append("    const double* y, const double* x0, double* sol, int* status, int* iters, unsigned* active,")
+    out.append("    int max_iter) {")
+    out.append("  clik::nlp_step<Skill>(N, ld, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter);")
+    out.append("}")
+    out.append('extern "C" __global__ void __launch_bounds__(%d) clik_nlp_rollout_kernel(' % block_threads)
+    out.append("    long long N, long long ld, int steps, double dt, const double* t0, int t_stride, double* q, double* x,")
+    out.append("    const double* y, double vmax_q, double vmax_x, double* sol_last, int* n_failed, int max_iter) {")
+    out.append("  clik::nlp_rollout<Skill>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last, n_failed,")
+    out.append("                           max_iter);")
+    out.append("}")
+    out.append('extern "C" __global__ void clik_sizes_kernel(int* o) {')
+    out.append("  // manifest: sizes (o[4], o[5]: NLP variables and rows), flags (256 NLP step + rollout kernels)")
+    out.append("  o[0] = %d; o[1] = %d; o[2] = %d; o[3] = 1; o[4] = %d; o[5] = %d; o[6] = 1; o[7] = 256;"
+               % (nq, nxv, ny, nx, m))
+    full = (1, 0xffffffff, 0xffffffff, 0xffffffff)
+    out.append("  // input rows the kernels read (t, q, x, y bit masks): (no pinv kernel) then NLP")
+    out.append("  " + " ".join("o[%d] = (int)0x%xu;" % (8 + k, v) for k, v in enumerate(full + tuple(meta["nlp_read_masks"]))))
+    out.append("  o[16] = 1; o[17] = 0;")
     out.append("}")
     return "\n".join(out) + "\n", meta
 

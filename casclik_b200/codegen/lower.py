@@ -64,6 +64,68 @@ class Symbols(object):
                              "variables of the skill: %s" % (what, sorted(set(free))))
 
 
+def _constraint_rows(spec, n_rob, n_virt, n_slack):
+    """Rows of  lb <= A x <= ub  over x = [robot vel; virtual vel; slack], one per constraint row:
+    [de/dq | de/dx | -1 on the row's own slack if soft]            reactive_qp.py:191-246.
+    -> (A as lists of nodes, lb nodes, ub nodes, row labels)."""
+    A, lbs, ubs, labels = [], [], [], []
+    slack_ind = 0
+    for c in spec.constraints:
+        kind = kind_of(c)
+        e = c.expression
+        rows = e.size()[0]
+        Jq = cs.jacobian(e, spec.robot_var)
+        Jx = cs.jacobian(e, spec.virtual_var) if spec.virtual_var is not None else None
+        Jt = cs.jacobian(e, spec.time_var)
+        lb = -Jt
+        ub = -Jt
+        if kind == KIND_EQ:
+            ke = c.gain_times(e)
+            lb = lb + (-ke)
+            ub = ub + (-ke)
+        elif kind == KIND_SET:
+            smin = cs.MX(cs.vertcat(*_col(c.set_min, rows, "set_min", c.label)))
+            smax = cs.MX(cs.vertcat(*_col(c.set_max, rows, "set_max", c.label)))
+            lb = lb + c.gain_times(smin - e)
+            ub = ub + c.gain_times(smax - e)
+        elif kind == KIND_VELEQ:
+            tg = cs.MX(cs.vertcat(*_col(c.target, rows, "target", c.label)))
+            lb = lb + tg
+            ub = ub + tg
+        else:
+            lb = lb + cs.MX(cs.vertcat(*_col(c.set_min, rows, "set_min", c.label)))
+            ub = ub + cs.MX(cs.vertcat(*_col(c.set_max, rows, "set_max", c.label)))
+        soft = c.constraint_type == "soft"
+        for r in range(rows):
+            row = [Jq._a[r, k] for k in range(n_rob)]
+            if Jx is not None:
+                row += [Jx._a[r, k] for k in range(n_virt)]
+            srow = [dag.ZERO] * n_slack
+            if soft:
+                srow[slack_ind + r] = dag.MINUS_ONE
+            A.append(row + srow)
+            labels.append("%s[%d]" % (c.label, r))
+        if soft:
+            slack_ind += rows
+        lbs += lb.nodes()
+        ubs += ub.nodes()
+    return A, lbs, ubs, labels
+
+
+def _classify_rows(A):
+    """Row structure: a "unit" row has exactly one structural non-zero and it is a constant (bounds on
+    a single variable: joint limits, speed limits); everything else is dense.
+    -> ([(row, column, coefficient)], [dense row indices])."""
+    unit_rows, dense_rows = [], []
+    for r, row in enumerate(A):
+        nz = [(j, n) for j, n in enumerate(row) if n is not dag.ZERO]
+        if len(nz) == 1 and nz[0][1].is_const and nz[0][1].val != 0.0:
+            unit_rows.append((r, nz[0][0], nz[0][1].val))
+        else:
+            dense_rows.append(r)
+    return unit_rows, dense_rows
+
+
 class PinvProgram(object):
     """Per-constraint numeric blocks for the pseudo-inverse controller."""
 
@@ -190,57 +252,68 @@ class QpProgram(object):
         self.h = cs.vertcat(*parts).nodes()
         if len(self.h) != self.nx:
             raise ValueError("weights do not match the number of optimisation variables")
-        # constraints                                                    reactive_qp.py:191-246
-        self.A, self.lb, self.ub, self.labels = [], [], [], []
-        slack_ind = 0
-        for c in spec.constraints:
-            kind = kind_of(c)
-            e = c.expression
-            rows = e.size()[0]
-            Jq = cs.jacobian(e, spec.robot_var)
-            Jx = cs.jacobian(e, spec.virtual_var) if spec.virtual_var is not None else None
-            Jt = cs.jacobian(e, spec.time_var)
-            lb = -Jt
-            ub = -Jt
-            if kind == KIND_EQ:
-                ke = c.gain_times(e)
-                lb = lb + (-ke)
-                ub = ub + (-ke)
-            elif kind == KIND_SET:
-                smin = cs.MX(cs.vertcat(*_col(c.set_min, rows, "set_min", c.label)))
-                smax = cs.MX(cs.vertcat(*_col(c.set_max, rows, "set_max", c.label)))
-                lb = lb + c.gain_times(smin - e)
-                ub = ub + c.gain_times(smax - e)
-            elif kind == KIND_VELEQ:
-                tg = cs.MX(cs.vertcat(*_col(c.target, rows, "target", c.label)))
-                lb = lb + tg
-                ub = ub + tg
-            else:
-                lb = lb + cs.MX(cs.vertcat(*_col(c.set_min, rows, "set_min", c.label)))
-                ub = ub + cs.MX(cs.vertcat(*_col(c.set_max, rows, "set_max", c.label)))
-            soft = c.constraint_type == "soft"
-            for r in range(rows):
-                row = [Jq._a[r, k] for k in range(self.n_rob)]
-                if Jx is not None:
-                    row += [Jx._a[r, k] for k in range(self.n_virt)]
-                srow = [dag.ZERO] * self.n_slack
-                if soft:
-                    srow[slack_ind + r] = dag.MINUS_ONE
-                self.A.append(row + srow)
-                self.labels.append("%s[%d]" % (c.label, r))
-            if soft:
-                slack_ind += rows
-            self.lb += lb.nodes()
-            self.ub += ub.nodes()
+        self.A, self.lb, self.ub, self.labels = _constraint_rows(spec, self.n_rob, self.n_virt, self.n_slack)
         self.m = len(self.A)
         nodes = self.h + self.lb + self.ub + [n for r in self.A for n in r]
         self.syms.check_closed(nodes, "QP matrices")
-        # row structure: a "unit" row has exactly one structural non-zero and it is a constant
-        # (bounds on a single variable: joint limits, speed limits); everything else is dense
-        self.unit_rows, self.dense_rows = [], []
-        for r, row in enumerate(self.A):
-            nz = [(j, n) for j, n in enumerate(row) if n is not dag.ZERO]
-            if len(nz) == 1 and nz[0][1].is_const and nz[0][1].val != 0.0:
-                self.unit_rows.append((r, nz[0][0], nz[0][1].val))
-            else:
-                self.dense_rows.append(r)
+        self.unit_rows, self.dense_rows = _classify_rows(self.A)
+
+
+#: capacity of the in-kernel NLP solver (the tiers of the dense QP core it calls, clik_qp_dense)
+NLP_MAX_NX, NLP_MAX_M = 32, 64
+
+
+class NlpProgram(object):
+    """Linearly constrained NLP of the reactive NLP controller over x = [robot vel; virtual vel; slack]:
+
+        min F(x)   s.t.  lb <= A x <= ub
+
+    with A, lb, ub exactly as QpProgram builds them.  `objective` is the whole scalar F, as
+    ReactiveNLPController.get_cost_expr composes it (the one place that states the cost convention).
+    Holds F, its gradient `g` and the lower triangle of H = d2F/dx2 (row-major packed:
+    H[i*(i+1)/2 + j], j <= i) as scalar nodes over the decision symbols `dec` (robot_vel_var;
+    virtual_vel_var; slack_var) and t, q, x, y; `quadratic` is true when no entry of H depends on a
+    decision symbol."""
+
+    def __init__(self, spec, objective):
+        self.syms = Symbols(spec)
+        self.n_rob = spec.n_robot_var
+        self.n_virt = spec.n_virtual_var if spec.virtual_var is not None else 0
+        self.n_slack = spec.n_slack_var
+        self.nx = self.n_rob + self.n_virt + self.n_slack
+        if not isinstance(objective, cs.GenericMatrixCommon):
+            objective = cs.DM(objective)
+        if tuple(objective.size()) != (1, 1):
+            raise ValueError("the cost must be a scalar (1x1) expression, got %dx%d" % tuple(objective.size()))
+        self.dec = list(spec.robot_vel_var.nodes())
+        if self.n_virt > 0:
+            self.dec += spec.virtual_vel_var.nodes()
+        if self.n_slack > 0:
+            self.dec += spec.slack_var.nodes()
+        cost = objective.nodes()[0]
+        # a cost that reads the input although no constraint does: the input rows become kernel inputs
+        if spec.input_var is not None and not self.syms.y:
+            yn = spec.input_var.nodes()
+            if dag.depends_on([cost], yn):
+                self.syms.y = yn
+                for i, n in enumerate(yn):
+                    self.syms.names[n.id] = "y[%d]" % i
+        self.n_in = len(self.syms.y)
+        dec_ids = {n.id for n in self.dec}
+        free = [s.name for s in dag.symbols_of([cost]) if s.id not in self.syms.names and s.id not in dec_ids]
+        if free:
+            raise ValueError("the cost depends on symbols that are not time/robot/virtual/input variables or "
+                             "decision variables (robot_vel_var, virtual_vel_var, slack_var) of the skill: %s"
+                             % sorted(set(free)))
+        self.A, self.lb, self.ub, self.labels = _constraint_rows(spec, self.n_rob, self.n_virt, self.n_slack)
+        self.m = len(self.A)
+        if self.nx > NLP_MAX_NX or self.m > NLP_MAX_M:
+            raise ValueError("the NLP controller supports at most %d decision variables and %d constraint rows "
+                             "(this skill: %d x %d)" % (NLP_MAX_NX, NLP_MAX_M, self.nx, self.m))
+        self.syms.check_closed(self.lb + self.ub + [n for r in self.A for n in r], "NLP constraints")
+        self.unit_rows, self.dense_rows = _classify_rows(self.A)
+        self.F = cost
+        self.g = dag.jacobian([cost], self.dec)[0]
+        Hfull = dag.jacobian(self.g, self.dec)
+        self.H = [Hfull[i][j] for i in range(self.nx) for j in range(i + 1)]
+        self.quadratic = not dag.depends_on(self.H, self.dec)

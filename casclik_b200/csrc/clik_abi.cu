@@ -90,12 +90,13 @@ struct clik_skill {
   clik_skill_desc desc;
   cudaLibrary_t lib = nullptr;
   KernelInfo pinv, pinv_tma, pinv_rollout, pinv_fast, pinv_group, qp, qp_fast, qp_tail, qp_tail_capped, qp_rollout;
+  KernelInfo nlp, nlp_rollout;   // NLP images (manifest flag 256)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
   bool pinv_group_all = false;  // CLIK_PINV_GROUP=1: whole batches through the sub-warp mapping (A/B measurements)
   int n_static = 1;           // statically compiled modes: where the group pass resumes the search
-  ReadMask pinv_reads, qp_reads;
+  ReadMask pinv_reads, qp_reads;   // (an NLP image reports its rows in the QP slots)
   bool use_tma = false;  // clik_skill_set_staging / CLIK_TMA=1: the TMA-staged persistent pinv kernel (device-resident batches)
   // programmatic dependent launch (clik_skill_set_overlap / CLIK_PDL): 0 = plain stream order,
   // 1 = the second launch of a two-launch step is scheduled while the first drains (it waits for the first
@@ -471,6 +472,11 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
     if (st == CLIK_OK && (flags & 128)) st = setup_kernel(s, "clik_qp_tail_capped_kernel", &s->qp_tail_capped);
     if (const char* e = getenv("CLIK_QP_TAIL_PICK")) s->qp_tail_pick = atoi(e);
     if (const char* e = getenv("CLIK_QP_SPLIT")) s->qp_split = atoi(e) != 0;
+  }
+  if (st == CLIK_OK && (flags & 256)) {
+    s->qp_reads = ReadMask{(unsigned)hsz[12], (unsigned)hsz[13], (unsigned)hsz[14], (unsigned)hsz[15]};
+    st = setup_kernel(s, "clik_nlp_kernel", &s->nlp);
+    if (st == CLIK_OK) st = setup_kernel(s, "clik_nlp_rollout_kernel", &s->nlp_rollout);
   }
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
@@ -983,6 +989,155 @@ clik_status clik_qp_solve_one(const clik_skill* cs, double t, const double* q, c
   const int* hi = (const int*)(h + o_int);
   if (status) *status = hi[0];
   if (active) { active[0] = (uint32_t)hi[1]; active[1] = (uint32_t)hi[2]; }
+  return CLIK_OK;
+}
+
+}  // extern "C"
+
+// ---- reactive NLP controller ------------------------------------------------------------------------------
+namespace {
+
+constexpr int NLP_DEFAULT_MAX_ITER = 50;
+
+clik_status nlp_step_impl(const clik_skill* s, int64_t N, int64_t ld, const double* t, int32_t t_stride,
+                          const double* q, const double* x, const double* y, const double* x0, double* sol,
+                          int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter, void* stream) {
+  clik_status st = check_common(s, N, t, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (ld < N) return fail(CLIK_ERR_INVALID, "row stride ld (%lld) < N (%lld)", (long long)ld, (long long)N);
+  if (!s->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
+  if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = ld;
+  int ts = t_stride ? 1 : 0;
+  int mi = max_iter > 0 ? max_iter : NLP_DEFAULT_MAX_ITER;
+  void* args[] = {&n, &l, &t, &ts, &q, &x, &y, &x0, &sol, &status, &iters, &active, &mi};
+  CK(launch(s->nlp, grid_for(s->nlp, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_nlp_step(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                          const double* x, const double* y, const double* x0, double* sol, int32_t* status,
+                          int32_t* iters, uint32_t* active, int32_t max_iter, void* stream) {
+  return nlp_step_impl(s, N, N, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter, stream);
+}
+
+clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t, int32_t t_stride,
+                               const double* q, const double* x, const double* y, const double* x0,
+                               double* sol, int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter) {
+  clik_skill* s = const_cast<clik_skill*>(cs);
+  clik_status st = check_common(s, N, t, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!s->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
+  if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
+  const clik_skill_desc& d = s->desc;
+  if (zero_copy_enabled()) {
+    const void *dt, *dq, *dx, *dy, *dx0, *dsol, *dst, *dit, *dact;
+    ON_DEVICE(d.device);
+    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
+        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(x0, &dx0) && device_alias(sol, &dsol) &&
+        device_alias(status, &dst) && device_alias(iters, &dit) && device_alias(active, &dact)) {
+      std::lock_guard<std::mutex> lock(s->mu);
+      clik_status zs = ensure_scratch(s, 0, 256);
+      if (zs != CLIK_OK) return zs;
+      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
+      zs = nlp_step_impl(s, N, N, (const double*)dt, t_stride, (const double*)dq, (const double*)dx,
+                         (const double*)dy, (const double*)dx0, (double*)dsol, (int32_t*)dst, (int32_t*)dit,
+                         (uint32_t*)dact, max_iter, s->scratch.stream[0]);
+      if (zs != CLIK_OK) return zs;
+      CK(cudaStreamSynchronize(s->scratch.stream[0]));
+      return CLIK_OK;
+    }
+  }
+  std::vector<Field> f;
+  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
+  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
+  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
+  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
+  f[0].rowmask = s->qp_reads.t;
+  f[1].rowmask = s->qp_reads.q;
+  f[2].rowmask = s->qp_reads.x;
+  f[3].rowmask = s->qp_reads.y;
+  f.push_back({x0, nullptr, d.qp_n, 8, 1, 0});
+  f.push_back({nullptr, sol, d.qp_n, 8, 1, 0});
+  f.push_back({nullptr, status, 1, 4, 1, 0});
+  f.push_back({nullptr, iters, 1, 4, 1, 0});
+  f.push_back({nullptr, active, 2, 4, 1, 0});
+  return run_host_pipeline(s, N, 0, N, f, [&](char* base, int64_t c, cudaStream_t stream) {
+    return nlp_step_impl(s, c, c, (const double*)(base + f[0].dev_off), t_stride,
+                         (const double*)(base + f[1].dev_off),
+                         d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
+                         d.n_input ? (const double*)(base + f[3].dev_off) : nullptr,
+                         x0 ? (const double*)(base + f[4].dev_off) : nullptr, (double*)(base + f[5].dev_off),
+                         status ? (int32_t*)(base + f[6].dev_off) : nullptr,
+                         iters ? (int32_t*)(base + f[7].dev_off) : nullptr,
+                         active ? (uint32_t*)(base + f[8].dev_off) : nullptr, max_iter, stream);
+  });
+}
+
+clik_status clik_nlp_solve_one(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
+                               const double* x0, double* sol, int32_t* status, int32_t* iters, uint32_t* active,
+                               int32_t max_iter) {
+  clik_skill* s = const_cast<clik_skill*>(cs);
+  if (!s || !q || !sol) return fail(CLIK_ERR_INVALID, "NULL argument");
+  if (!s->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
+  const clik_skill_desc& d = s->desc;
+  if (d.n_virtual > 0 && !x) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x is required");
+  if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
+  ON_DEVICE(d.device);
+  std::lock_guard<std::mutex> lock(s->mu);
+  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n;
+  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3));
+  if (st != CLIK_OK) return st;
+  double* h = s->one_host;
+  // slot: t | q | x | y | x0 | sol | status, iters, active_up, active_lo (four int cells in two doubles)
+  h[0] = t;
+  std::memcpy(h + 1, q, sizeof(double) * nq);
+  if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
+  if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
+  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn;
+  if (x0) std::memcpy(h + o_x0, x0, sizeof(double) * qn);
+  double* dv = s->one_dev;
+  long long n = 1, l = 1;
+  int ts = 0;
+  int mi = max_iter > 0 ? max_iter : NLP_DEFAULT_MAX_ITER;
+  const double *dt = dv, *dq = dv + 1, *dx = nx ? dv + 1 + nq : nullptr, *dy = ny ? dv + 1 + nq + nx : nullptr;
+  const double* dx0 = x0 ? dv + o_x0 : nullptr;
+  double* dsol = dv + o_sol;
+  int* dst = (int*)(dv + o_int);
+  int* dit = dst + 1;
+  unsigned* dact = (unsigned*)(dst + 2);      // active[0], active[ld = 1]
+  void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dx0, &dsol, &dst, &dit, &dact, &mi};
+  CK(cudaLaunchKernel((const void*)s->nlp.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
+  CK(cudaStreamSynchronize(s->one_stream));
+  std::memcpy(sol, h + o_sol, sizeof(double) * qn);
+  const int* hi = (const int*)(h + o_int);
+  if (status) *status = hi[0];
+  if (iters) *iters = hi[1];
+  if (active) { active[0] = (uint32_t)hi[2]; active[1] = (uint32_t)hi[3]; }
+  return CLIK_OK;
+}
+
+clik_status clik_nlp_rollout(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                             int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                             double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                             void* stream) {
+  clik_status st = check_common(s, N, t0, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!s->nlp_rollout.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP rollout kernel");
+  if (steps < 0) return fail(CLIK_ERR_INVALID, "steps < 0");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0, k = steps;
+  int mi = max_iter > 0 ? max_iter : NLP_DEFAULT_MAX_ITER;
+  void* args[] = {&n, &l, &k, &dt, &t0, &ts, &q, &x, &y, &max_robot_speed, &max_virtual_speed,
+                  &sol_last, &n_failed, &mi};
+  CK(cudaLaunchKernel((const void*)s->nlp_rollout.kernel, dim3(grid_for(s->nlp_rollout, N)),
+                      dim3(s->nlp_rollout.block), args, 0, (cudaStream_t)stream));
   return CLIK_OK;
 }
 

@@ -16,6 +16,7 @@ _c_uint32_p = ctypes.POINTER(ctypes.c_uint32)
 
 ABI_VERSION = 2
 QP_SOLVED, QP_MAXITER, QP_INFEASIBLE, QP_INVALID = 0, 1, 2, 4
+NLP_STALLED = 5   # NLP step: the line search found no decrease (other codes as the QP's)
 
 
 class ClikError(RuntimeError):
@@ -35,6 +36,7 @@ EXPORTS = (
     "clik_pinv_step_host", "clik_qp_step_host", "clik_skill_launch_info",
     "clik_pinv_step_ld", "clik_qp_step_ld", "clik_pinv_step_host_multi", "clik_qp_step_host_multi",
     "clik_pinv_solve_one", "clik_qp_solve_one", "clik_skill_set_overlap", "clik_skill_get_overlap",
+    "clik_nlp_step", "clik_nlp_step_host", "clik_nlp_solve_one", "clik_nlp_rollout",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -99,6 +101,15 @@ def load_library():
     lib.clik_qp_step_host.argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32]
     lib.clik_qp_dense.restype = i32
     lib.clik_qp_dense.argtypes = [i32, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
+    lib.clik_nlp_step.restype = i32
+    lib.clik_nlp_step.argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
+    lib.clik_nlp_step_host.restype = i32
+    lib.clik_nlp_step_host.argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32]
+    lib.clik_nlp_solve_one.restype = i32
+    lib.clik_nlp_solve_one.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, vp, i32]
+    lib.clik_nlp_rollout.restype = i32
+    lib.clik_nlp_rollout.argtypes = [vp, i64, i32, ctypes.c_double, vp, i32, vp, vp, vp,
+                                     ctypes.c_double, ctypes.c_double, vp, vp, i32, vp]
     lib.clik_skill_launch_info.restype = i32
     lib.clik_skill_launch_info.argtypes = [vp, i32, _c_int32_p, _c_int32_p, _c_int32_p, _c_int32_p]
     lib.clik_skill_set_overlap.restype = i32

@@ -8,6 +8,11 @@ __graft_entry__.py and the tests, so all three measure and check exactly the sam
   iiwa_multitask  configs[2]: 7 joint-limit SetConstraints + 4-row pose EqualityConstraint
   ur5_qp          configs[3]: soft position Eq (K = 50) + joint limits + joint speed limits
   ur5_moe2016     configs[4]: 3 scalar box sets (K = 500) + time-varying 3-row path Eq (K = 0.15)
+
+NLP_REGISTRY holds the scenarios of ReactiveNLPController (no BASELINE config; tools/nlp_bench.py):
+
+  ur5_nlp_taskspeed  ur5_qp's constraints, cost |J_p(q) dq|^2 + mu |dq|^2 (quadratic, q-dependent Hessian)
+  ur5_nlp_quartic    ur5_qp's constraints, cost mu |dq|^2 + sum_j (dq_j / 0.3)^4 (convex, not quadratic)
 """
 import math
 
@@ -21,12 +26,16 @@ from .sym import dag
 
 
 class Scenario(object):
-    def __init__(self, name, spec, controller, options, sampler, description):
+    def __init__(self, name, spec, controller, options, sampler, description, cost_expr=None):
         self.name, self.spec, self.controller = name, spec, controller
         self.options, self.sampler, self.description = options, sampler, description
+        self.cost_expr = cost_expr       # the NLP controller's cost
 
     def make_controller(self):
-        from .controllers import PseudoInverseController, ReactiveQPController
+        from .controllers import PseudoInverseController, ReactiveQPController, ReactiveNLPController
+        if self.controller == "nlp":
+            return ReactiveNLPController(self.spec, self.cost_expr,
+                                         options=dict(self.options) if self.options else None)
         cls = {"pinv": PseudoInverseController, "qp": ReactiveQPController}[self.controller]
         return cls(skill_spec=self.spec, options=dict(self.options) if self.options else None)
 
@@ -202,5 +211,31 @@ REGISTRY = {
 }
 
 
+def ur5_nlp(cost):
+    """ur5_qp's skill (9 variables x 15 rows) with a general cost of the NLP controller."""
+    base = ur5_qp()
+    spec = base.spec
+    q, dq = spec.robot_var, spec.robot_vel_var
+    mu = 0.001
+    if cost == "taskspeed":
+        J = cs.jacobian(fk.ur5()["T_fk"](q)[:3, 3], q)
+        v = cs.mtimes(J, dq)
+        expr = cs.dot(v, v) + mu * cs.dot(dq, dq)
+        what = "|J_p(q) dq|^2 + mu |dq|^2 (quadratic, configuration-dependent Hessian)"
+    else:
+        u2 = (dq / 0.3) * (dq / 0.3)
+        expr = mu * cs.dot(dq, dq) + cs.sum1(u2 * u2)
+        what = "mu |dq|^2 + sum_j (dq_j / 0.3)^4 (convex, not quadratic)"
+    return Scenario("ur5_nlp_" + cost, spec, "nlp", None, base.sampler,
+                    "UR5 ReactiveNLPController on ur5_qp's constraints (9 variables x 15 rows), cost " + what,
+                    cost_expr=expr)
+
+
+NLP_REGISTRY = {
+    "ur5_nlp_taskspeed": lambda: ur5_nlp("taskspeed"),
+    "ur5_nlp_quartic": lambda: ur5_nlp("quartic"),
+}
+
+
 def get(name):
-    return REGISTRY[name]()
+    return REGISTRY[name]() if name in REGISTRY else NLP_REGISTRY[name]()

@@ -10,7 +10,7 @@ from .matrix import (  # noqa: F401
     sum1, sum2, trace, diag, reshape, vec, cross,
     sin, cos, tan, asin, acos, atan, atan2, exp, log, sqrt, fabs, sign, floor, ceil,
     fmin, fmax, power, logic_and, logic_or, logic_not, if_else,
-    jacobian, jtimes, gradient, substitute, depends_on, symvar,
+    jacobian, jtimes, gradient, hessian, substitute, depends_on, symvar,
     solve, inv, det, pinv,
 )
 

@@ -722,6 +722,13 @@ def gradient(expr, var):
     return jacobian(expr, var).T
 
 
+def hessian(expr, var):
+    """-> (H, g): the Hessian of the scalar `expr` with respect to `var` and its gradient, as
+    casadi.hessian returns them (H = jacobian(gradient(expr, var), var))."""
+    g = gradient(expr, var)
+    return jacobian(g, var), g
+
+
 def substitute(expr, var, val):
     e = _mat(expr)
     syms = _sym_list(var)

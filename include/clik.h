@@ -47,7 +47,14 @@ typedef enum {
 #define CLIK_QP_INFEASIBLE 2
 #define CLIK_QP_INVALID 4 /* non-finite data or solution (NaN input, non-positive cost weight); 3 is internal */
 
-/* Sizes of a compiled skill; must match the constants baked into the cubin (checked at load). */
+/* Per-instance NLP outcome written to `status[i]` by clik_nlp_step*: CLIK_QP_SOLVED, CLIK_QP_MAXITER (SQP
+ * iteration cap or the cap of a subproblem), CLIK_QP_INFEASIBLE, CLIK_QP_INVALID (also a non-finite cost,
+ * gradient or Hessian at an iterate, or a Hessian no tried shift makes positive definite), or: */
+#define CLIK_NLP_STALLED 5 /* the line search found no sufficient decrease of the cost */
+
+/* Sizes of a compiled skill; must match the constants baked into the cubin (checked at load).
+ * An image of the NLP controller (manifest flag 256) loads with has_pinv = has_qp = 0; qp_n / qp_m then
+ * carry the NLP's decision variables and constraint rows. */
 typedef struct {
   int32_t abi_version; /* CLIK_ABI_VERSION */
   int32_t device;      /* CUDA device ordinal the skill lives on */
@@ -152,6 +159,44 @@ clik_status clik_qp_dense(int32_t device, int64_t N, int32_t nx, int32_t m, cons
                           const double* A, const double* lb, const double* ub, const double* x0,
                           double* sol, int32_t* status, uint32_t* active, int32_t max_iter,
                           void* stream);
+
+/* ReactiveNLPController.solve (the reference's cs.nlpsol / IPOPT call, reactive_nlp.py:469-534) for N
+ * instances of an NLP image: min F(x) s.t. lb <= A x <= ub with the QP's rows, by SQP with the exact Hessian,
+ * one instance per thread.
+ *   x0     [qp_n * N] start point of the iteration, or NULL (start at 0); the first subproblem restores
+ *          feasibility from it
+ *   sol    [qp_n * N] out: [robot vel; virtual vel; slack]
+ *   status [N] out, may be NULL: CLIK_QP_* / CLIK_NLP_STALLED
+ *   iters  [N] out, may be NULL: SQP iterations (subproblems solved)
+ *   active [2 * N] out, may be NULL: working set of the last subproblem, format of clik_qp_step
+ *   max_iter <= 0 selects the default SQP cap 50.
+ * Solved (0) means |p|_inf * max(1, delta) <= tol * (1 + |x|_inf) for the last SQP step p (delta: the shift that
+ * made the Hessian positive definite, tol compiled into the image, default 1e-10), or a step with
+ * |p|_inf <= 100 * tol * (1 + |x|_inf) that left the cost unchanged within its rounding (1e-15 relative). */
+clik_status clik_nlp_step(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                          const double* q, const double* x, const double* y, const double* x0, double* sol,
+                          int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter, void* stream);
+
+/* The same call on HOST pointers, synchronous (the chunked pipeline or, on page-locked buffers, the kernel
+ * on the mapped memory, as clik_qp_step_host).  Bit-identical to clik_nlp_step. */
+clik_status clik_nlp_step_host(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                               const double* q, const double* x, const double* y, const double* x0,
+                               double* sol, int32_t* status, int32_t* iters, uint32_t* active,
+                               int32_t max_iter);
+
+/* One instance, HOST pointers (the reference's single solve() call), synchronous, as clik_qp_solve_one. */
+clik_status clik_nlp_solve_one(const clik_skill* skill, double t, const double* q, const double* x,
+                               const double* y, const double* x0, double* sol, int32_t* status,
+                               int32_t* iters, uint32_t* active, int32_t max_iter);
+
+/* The simulation loop with the NLP controller (see clik_qp_rollout): every step starts from the previous
+ * step's solution; a step that is not solved applies zero velocity, is counted in n_failed, and the next
+ * step starts from 0.
+ *   sol_last [qp_n * N] out, may be NULL: solution of the last step (robot / virtual parts clipped) */
+clik_status clik_nlp_rollout(const clik_skill* skill, int64_t N, int32_t steps, double dt,
+                             const double* t0, int32_t t_stride, double* q, double* x, const double* y,
+                             double max_robot_speed, double max_virtual_speed, double* sol_last,
+                             int32_t* n_failed, int32_t max_iter, void* stream);
 
 /* Host-buffer variants (same argument meaning, HOST pointers, synchronous).  Pageable memory goes
  * through a chunked H2D / kernel / D2H pipeline on internal streams; if every buffer is page-locked

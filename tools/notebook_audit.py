@@ -2,7 +2,7 @@
 """Drop-in audit (build container only — it reads the reference's notebooks from /root/reference):
 execute the code cells of examples/notebooks/*.ipynb with `casadi`, `casclik` and `urdf2casadi`
 resolved to this package, up to — not including — anything that needs a GPU (controller.solve calls
-and what depends on their results), plotting or the out-of-scope NLP / MPC controllers.  Controllers
+and what depends on their results), plotting or the out-of-scope MPC controller.  Controllers
 are set up with load=False: lowered, emitted and compiled by nvcc, not loaded.  Prints per notebook
 which cells ran, which were skipped and why, and every exception.
 
@@ -70,7 +70,7 @@ sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
 sys.modules["matplotlib"].animation = sys.modules["matplotlib.animation"]
 
 # controllers: build, do not load (no GPU here)
-for cls in (cc.PseudoInverseController, cc.ReactiveQPController):
+for cls in (cc.PseudoInverseController, cc.ReactiveQPController, cc.ReactiveNLPController):
     orig = cls.setup_problem_functions
     cls.setup_problem_functions = (lambda o: lambda self, load=False: o(self, load=False))(orig)
     cls.setup_solver = (lambda o: lambda self: o(self, load=False))(orig)
@@ -99,7 +99,7 @@ def _fake_initial(self, time_var0, robot_var0, virtual_var0=None, robot_vel_var0
 
 
 class _OutOfScopeController(object):
-    """ReactiveNLPController / ModelPredictiveController (IPOPT; not part of this package)."""
+    """ModelPredictiveController (an NLP over a horizon; not part of this package)."""
 
     def __init__(self, skill_spec, *a, **k):
         self.skill_spec = skill_spec
@@ -114,11 +114,11 @@ class _OutOfScopeController(object):
     solve_initial_problem = _fake_initial
 
 
-for cls in (cc.PseudoInverseController, cc.ReactiveQPController):
+for cls in (cc.PseudoInverseController, cc.ReactiveQPController, cc.ReactiveNLPController):
     cls.solve = _fake_solve
     cls.solve_initial_problem = _fake_initial
     cls.setup_initial_problem_solver = lambda self: None
-cc.ReactiveNLPController = cc.ModelPredictiveController = _OutOfScopeController
+cc.ModelPredictiveController = _OutOfScopeController
 
 NEEDS_GPU = re.compile(r"a^")       # (nothing: solve() is faked above)
 OUT_OF_SCOPE = re.compile(r"a^")
