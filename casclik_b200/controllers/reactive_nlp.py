@@ -21,7 +21,7 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
-from .base_controller import BaseController, Batch, as_vector, dm_column
+from .base_controller import BaseController, Batch, as_vector, dm_column, resolve_devices, skill_handle_array
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -166,17 +166,22 @@ class ReactiveNLPController(BaseController):
 
     # ---- step --------------------------------------------------------------------------------------
     def solve_batch(self, time_var, robot_var, virtual_var=None, input_var=None, warmstart=None, out=None,
-                    max_iter=None):
+                    max_iter=None, devices=None):
         """NLP controller step for N instances (layout of ReactiveQPController.solve_batch): torch CUDA
         tensors run on their device (asynchronously on the current stream), NumPy arrays go through the
         host entry point.  warmstart: optional (nx, N) start point of the SQP iteration (the first
         subproblem restores feasibility from it).
+        devices: as in PseudoInverseController.solve_batch (host arrays sharded over several GPUs,
+        bit-identical to one GPU).
         Returns (sol (nx, N), status (N,) int32, active (2, N) int32 bit masks [upper; lower] of the last
         subproblem's working set, iterations (N,) int32)."""
         spec = self.skill_spec
         b = Batch(spec.n_robot_var, self._nxv, self._ny, time_var, robot_var, virtual_var,
                   input_var if self._ny else None)
-        skill = self._skill(b.device_index)
+        devs = resolve_devices(devices)
+        if devs is not None and b.on_device:
+            raise ValueError("devices= applies to host arrays; CUDA tensors run on the device they live on")
+        skill = self._skill(b.device_index if devs is None else devs[0])
         if out is None:
             sol, status, active, iters = b.empty(self._qn), b.empty(0, "i32"), b.empty(2, "i32"), b.empty(0, "i32")
         else:
@@ -198,6 +203,10 @@ class ReactiveNLPController(BaseController):
         if b.on_device:
             runtime.check(lib.clik_nlp_step(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, x0p,
                                             solp, stp, itp, acp, mi, b.stream()))
+        elif devs is not None and len(devs) > 1:
+            skills = [self._skill(d) for d in devs]
+            runtime.check(lib.clik_nlp_step_host_multi(skill_handle_array(skills), len(skills), b.N, b.tp,
+                                                       b.t_stride, b.qp, b.xp, b.yp, x0p, solp, stp, itp, acp, mi))
         else:
             runtime.check(lib.clik_nlp_step_host(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, x0p,
                                                  solp, stp, itp, acp, mi))

@@ -1016,25 +1016,12 @@ clik_status nlp_step_impl(const clik_skill* s, int64_t N, int64_t ld, const doub
   return CLIK_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-clik_status clik_nlp_step(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
-                          const double* x, const double* y, const double* x0, double* sol, int32_t* status,
-                          int32_t* iters, uint32_t* active, int32_t max_iter, void* stream) {
-  return nlp_step_impl(s, N, N, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter, stream);
-}
-
-clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t, int32_t t_stride,
-                               const double* q, const double* x, const double* y, const double* x0,
-                               double* sol, int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter) {
-  clik_skill* s = const_cast<clik_skill*>(cs);
-  clik_status st = check_common(s, N, t, q, x, y);
-  if (st != CLIK_OK || N == 0) return st;
-  if (!s->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
-  if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
+// Instances [lo, lo + cnt) of a host batch of N (as qp_host_range).
+clik_status nlp_host_range(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, const double* t, int32_t t_stride,
+                           const double* q, const double* x, const double* y, const double* x0, double* sol,
+                           int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter) {
   const clik_skill_desc& d = s->desc;
+  if (cnt <= 0) return CLIK_OK;
   if (zero_copy_enabled()) {
     const void *dt, *dq, *dx, *dy, *dx0, *dsol, *dst, *dit, *dact;
     ON_DEVICE(d.device);
@@ -1044,10 +1031,12 @@ clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t,
       std::lock_guard<std::mutex> lock(s->mu);
       clik_status zs = ensure_scratch(s, 0, 256);
       if (zs != CLIK_OK) return zs;
+      auto off = [lo](const void* p) { return p ? (const double*)p + lo : nullptr; };
       GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
-      zs = nlp_step_impl(s, N, N, (const double*)dt, t_stride, (const double*)dq, (const double*)dx,
-                         (const double*)dy, (const double*)dx0, (double*)dsol, (int32_t*)dst, (int32_t*)dit,
-                         (uint32_t*)dact, max_iter, s->scratch.stream[0]);
+      zs = nlp_step_impl(s, cnt, N, t_stride ? off(dt) : (const double*)dt, t_stride, off(dq), off(dx), off(dy),
+                         off(dx0), (double*)off(dsol), dst ? (int32_t*)dst + lo : nullptr,
+                         dit ? (int32_t*)dit + lo : nullptr, dact ? (uint32_t*)dact + lo : nullptr, max_iter,
+                         s->scratch.stream[0]);
       if (zs != CLIK_OK) return zs;
       CK(cudaStreamSynchronize(s->scratch.stream[0]));
       return CLIK_OK;
@@ -1067,7 +1056,7 @@ clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t,
   f.push_back({nullptr, status, 1, 4, 1, 0});
   f.push_back({nullptr, iters, 1, 4, 1, 0});
   f.push_back({nullptr, active, 2, 4, 1, 0});
-  return run_host_pipeline(s, N, 0, N, f, [&](char* base, int64_t c, cudaStream_t stream) {
+  return run_host_pipeline(s, N, lo, cnt, f, [&](char* base, int64_t c, cudaStream_t stream) {
     return nlp_step_impl(s, c, c, (const double*)(base + f[0].dev_off), t_stride,
                          (const double*)(base + f[1].dev_off),
                          d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
@@ -1076,6 +1065,42 @@ clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t,
                          status ? (int32_t*)(base + f[6].dev_off) : nullptr,
                          iters ? (int32_t*)(base + f[7].dev_off) : nullptr,
                          active ? (uint32_t*)(base + f[8].dev_off) : nullptr, max_iter, stream);
+  });
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_nlp_step(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                          const double* x, const double* y, const double* x0, double* sol, int32_t* status,
+                          int32_t* iters, uint32_t* active, int32_t max_iter, void* stream) {
+  return nlp_step_impl(s, N, N, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter, stream);
+}
+
+clik_status clik_nlp_step_ld(const clik_skill* s, int64_t N, int64_t ld, const double* t, int32_t t_stride,
+                             const double* q, const double* x, const double* y, const double* x0, double* sol,
+                             int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter, void* stream) {
+  return nlp_step_impl(s, N, ld, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter, stream);
+}
+
+clik_status clik_nlp_step_host(const clik_skill* cs, int64_t N, const double* t, int32_t t_stride,
+                               const double* q, const double* x, const double* y, const double* x0,
+                               double* sol, int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter) {
+  return clik_nlp_step_host_multi(&cs, 1, N, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter);
+}
+
+clik_status clik_nlp_step_host_multi(const clik_skill* const* skills, int32_t n_skills, int64_t N,
+                                     const double* t, int32_t t_stride, const double* q, const double* x,
+                                     const double* y, const double* x0, double* sol, int32_t* status,
+                                     int32_t* iters, uint32_t* active, int32_t max_iter) {
+  if (!skills || n_skills < 1 || !skills[0]) return fail(CLIK_ERR_INVALID, "no skill handles");
+  clik_status st = check_common(skills[0], N, t, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!skills[0]->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
+  if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
+  return run_sharded(skills, n_skills, N, [&](clik_skill* s, int64_t lo, int64_t cnt) {
+    return nlp_host_range(s, N, lo, cnt, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter);
   });
 }
 

@@ -37,6 +37,7 @@ EXPORTS = (
     "clik_pinv_step_ld", "clik_qp_step_ld", "clik_pinv_step_host_multi", "clik_qp_step_host_multi",
     "clik_pinv_solve_one", "clik_qp_solve_one", "clik_skill_set_overlap", "clik_skill_get_overlap",
     "clik_nlp_step", "clik_nlp_step_host", "clik_nlp_solve_one", "clik_nlp_rollout",
+    "clik_nlp_step_ld", "clik_nlp_step_host_multi",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -105,6 +106,11 @@ def load_library():
     lib.clik_nlp_step.argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.clik_nlp_step_host.restype = i32
     lib.clik_nlp_step_host.argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32]
+    lib.clik_nlp_step_ld.restype = i32
+    lib.clik_nlp_step_ld.argtypes = [vp, i64, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
+    lib.clik_nlp_step_host_multi.restype = i32
+    lib.clik_nlp_step_host_multi.argtypes = [ctypes.POINTER(vp), i32, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp,
+                                             vp, i32]
     lib.clik_nlp_solve_one.restype = i32
     lib.clik_nlp_solve_one.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, vp, i32]
     lib.clik_nlp_rollout.restype = i32

@@ -177,6 +177,14 @@ clik_status clik_nlp_step(const clik_skill* skill, int64_t N, const double* t, i
                           const double* q, const double* x, const double* y, const double* x0, double* sol,
                           int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter, void* stream);
 
+/* Shard variant of clik_nlp_step (see clik_pinv_step_ld): N instances in place, rows `ld` elements apart
+ * (ld >= N), every pointer (t when t_stride = 1, q, x, y, x0, sol, status, iters, active) already at the shard's
+ * first instance; active[i] / active[ld + i].  clik_nlp_step(..N..) == clik_nlp_step_ld(..N, N..). */
+clik_status clik_nlp_step_ld(const clik_skill* skill, int64_t N, int64_t ld, const double* t,
+                             int32_t t_stride, const double* q, const double* x, const double* y,
+                             const double* x0, double* sol, int32_t* status, int32_t* iters,
+                             uint32_t* active, int32_t max_iter, void* stream);
+
 /* The same call on HOST pointers, synchronous (the chunked pipeline or, on page-locked buffers, the kernel
  * on the mapped memory, as clik_qp_step_host).  Bit-identical to clik_nlp_step. */
 clik_status clik_nlp_step_host(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
@@ -229,7 +237,10 @@ clik_status clik_qp_solve_one(const clik_skill* skill, double t, const double* q
  * copy on page-locked buffers — the SMs of device k read/write only shard k of the host arrays over that
  * device's PCIe link — or the chunked pipeline on pageable ones), and the call returns when every
  * result is in the caller's host arrays: the "final host gather" of the north star, with no collective
- * and no intermediate copy.  Results are bit-identical to the single-device call. */
+ * and no intermediate copy.  Results are bit-identical to the single-device call.  The handles stay owned by
+ * the caller; several of them may live on one device (their shards then share it).  The NLP form takes the
+ * arguments of clik_nlp_step_host; clik_*_step_host(skill, ...) is clik_*_step_host_multi(&skill, 1, ...), so a
+ * NULL skill there fails with CLIK_ERR_INVALID, "no skill handles". */
 clik_status clik_pinv_step_host_multi(const clik_skill* const* skills, int32_t n_skills, int64_t N,
                                       const double* t, int32_t t_stride, const double* q,
                                       const double* x, const double* y, double* qdot, double* xdot,
@@ -238,6 +249,10 @@ clik_status clik_qp_step_host_multi(const clik_skill* const* skills, int32_t n_s
                                     const double* t, int32_t t_stride, const double* q, const double* x,
                                     const double* y, const double* x0, const uint32_t* active0,
                                     double* sol, int32_t* status, uint32_t* active, int32_t max_iter);
+clik_status clik_nlp_step_host_multi(const clik_skill* const* skills, int32_t n_skills, int64_t N,
+                                     const double* t, int32_t t_stride, const double* q, const double* x,
+                                     const double* y, const double* x0, double* sol, int32_t* status,
+                                     int32_t* iters, uint32_t* active, int32_t max_iter);
 
 /* Overlap of launches on one stream (programmatic dependent launch, sm_90+; replaces nothing in the
  * reference — its loop is sequential, casclik/controllers/pseudo_inverse.py:512-556 — it is the batched
