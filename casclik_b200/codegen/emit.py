@@ -729,8 +729,47 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     out.append("  " + " ".join("o[%d] = (int)0x%xu;" % (8 + k, v) for k, v in enumerate(tuple(pm) + tuple(qm))))
     out.append("  o[16] = %d; o[17] = %s;" % (meta.get("pinv_static_modes", 1),
                                              "clik::GroupGeometry<Skill>::BLOCK" if meta.get("pinv_group") else "0"))
+    meta["duals"] = qp is not None and 0 < qp.m <= DUALS_MAX_ROWS
+    if meta["duals"]:
+        out.append("  o[18] = 1;   // multiplier kernels (1 QP, 2 NLP)")
     out.append("}")
+    if meta["duals"]:
+        out += _emit_qp_duals(qp, sig, sincos_name, block_threads, meta["qp_structured"])
     return "\n".join(out) + "\n", meta
+
+
+#: the working-set masks of the step kernels describe rows below 32 only (clik_duals.cuh)
+DUALS_MAX_ROWS = 32
+
+
+def _emit_qp_duals(qp, sig, sincos_name, block_threads, structured):
+    """clik_qp_duals_kernel, appended after the manifest so that nothing emitted before changes.  A structured
+    skill (eval_qps: dense rows + unit rows, 1/sqrt(h)) also gets the dense eval_qp the kernel reads, in a struct
+    derived from Skill; its constants are literals, so the constant bank of the step kernels stays as it is."""
+    out = ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
+           '#include "clik_duals.cuh"']
+    skill = "Skill"
+    if structured:
+        skill = "SkillDuals"
+        em = Emitter(qp.syms.names, None, sincos_name)
+        for r in range(qp.m):
+            for j in range(qp.nx):
+                em.assign("d.A[%d]" % (r * qp.nx + j), qp.A[r][j])
+            em.assign("d.lb[%d]" % r, qp.lb[r])
+            em.assign("d.ub[%d]" % r, qp.ub[r])
+        for j in range(qp.nx):
+            em.assign("d.h[%d]" % j, qp.h[j])
+        out.append("struct SkillDuals : Skill {")
+        out.append("  __device__ static __forceinline__ void eval_qp(%s, clik::QpData<SkillDuals>& d) {" % sig)
+        out += ["    " + ln for ln in em.finish()]
+        out.append("  }")
+        out.append("};")
+    out.append('extern "C" __global__ void __launch_bounds__(%d) clik_qp_duals_kernel(' % block_threads)
+    out.append("    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,")
+    out.append("    const double* y, const double* sol, const int* status, const unsigned* active, double* lam) {")
+    out.append("  clik::qp_duals<%s>(N, ld, t, t_stride, q, x, y, sol, status, active, lam);" % skill)
+    out.append("}")
+    return out
 
 
 def nlp_hoisted(nlp):
@@ -853,7 +892,18 @@ def _emit_nlp(nlp, label, block_threads, tol):
     out.append("  // input rows the kernels read (t, q, x, y bit masks): (no pinv kernel) then NLP")
     out.append("  " + " ".join("o[%d] = (int)0x%xu;" % (8 + k, v) for k, v in enumerate(full + tuple(meta["nlp_read_masks"]))))
     out.append("  o[16] = 1; o[17] = 0;")
+    meta["duals"] = 0 < m <= DUALS_MAX_ROWS
+    if meta["duals"]:
+        out.append("  o[18] = 2;   // multiplier kernels (1 QP, 2 NLP)")
     out.append("}")
+    if meta["duals"]:
+        out += ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
+                '#include "clik_duals.cuh"',
+                'extern "C" __global__ void __launch_bounds__(%d) clik_nlp_duals_kernel(' % block_threads,
+                "    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,",
+                "    const double* y, const double* sol, const int* status, const unsigned* active, double* lam) {",
+                "  clik::nlp_duals<Skill>(N, ld, t, t_stride, q, x, y, sol, status, active, lam);",
+                "}"]
     return "\n".join(out) + "\n", meta
 
 

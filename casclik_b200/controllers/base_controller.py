@@ -37,6 +37,44 @@ def resolve_devices(devices):
     return devs
 
 
+def multipliers_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, out):
+    """Shared body of ReactiveQPController / ReactiveNLPController.multipliers_batch (`kind` "qp" or "nlp"):
+    validates the step's inputs and outputs like solve_batch and calls clik_<kind>_duals[_host]."""
+    if ctrl._cubin is None:
+        raise RuntimeError("call setup_problem_functions() / setup_solver() before multipliers_batch()")
+    if not ctrl.kernel_meta.get("duals"):
+        raise ValueError("multipliers need at most 32 constraint rows and at least one (the skill has %d)" % ctrl._qm)
+    spec = ctrl.skill_spec
+    b = Batch(spec.n_robot_var, ctrl._nxv, ctrl._ny, time_var, robot_var, virtual_var,
+              input_var if ctrl._ny else None)
+    lam = b.empty(ctrl._qm) if out is None else out
+    lamp = b.out_ptr(lam, ctrl._qm, "f64", "out (lam)")
+    if sol is None or status is None or active is None:
+        raise ValueError("sol, status and active of the step are required")
+    if b.on_device:
+        if not all(runtime._is_torch(a) for a in (sol, status, active)):
+            raise ValueError("sol, status and active must be CUDA tensors when the inputs are CUDA tensors")
+        solp = runtime.dev_ptr(sol, "f64", ctrl._qn * b.N, "sol")
+        stp = runtime.dev_ptr(status, "i32", b.N, "status")
+        acp = runtime.dev_ptr(active, "u32", 2 * b.N, "active")
+        if any(a.device != b.device for a in (sol, status, active)):
+            raise ValueError("sol, status and active must live on %s like robot_var" % b.device)
+    else:
+        solp, sol = runtime.host_ptr(sol, np.float64, ctrl._qn * b.N, "sol")
+        stp, status = runtime.host_ptr(status, np.int32, b.N, "status")
+        acp, active = runtime.host_ptr(active.view(np.int32) if getattr(active, "dtype", None) == np.uint32 else active,
+                                       np.int32, 2 * b.N, "active")
+    skill = ctrl._skill(b.device_index)
+    lib = runtime.load_library()
+    if b.on_device:
+        runtime.check(getattr(lib, "clik_%s_duals" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp,
+                                                            solp, stp, acp, lamp, b.stream()))
+    else:
+        runtime.check(getattr(lib, "clik_%s_duals_host" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp,
+                                                                 b.yp, solp, stp, acp, lamp))
+    return lam
+
+
 def skill_handle_array(skills):
     arr = (ctypes.c_void_p * len(skills))(*[s.handle for s in skills])
     return arr

@@ -21,7 +21,8 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
-from .base_controller import BaseController, Batch, as_vector, dm_column, resolve_devices, skill_handle_array
+from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
+                              skill_handle_array)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -212,6 +213,12 @@ class ReactiveNLPController(BaseController):
                                                  solp, stp, itp, acp, mi))
         return sol, status, active, iters
 
+    def multipliers_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
+        """Constraint multipliers (the reference's lam_g) of a solve_batch result, as
+        ReactiveQPController.multipliers_batch: lam (m, N) float64 with grad F + A' lam = 0 on the last
+        subproblem's working set; NaN for an instance whose status is not 0 (include/clik.h clik_nlp_duals)."""
+        return multipliers_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
+
     def rollout_batch(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
                       max_speed=None, max_virtual_speed=None, max_iter=None):
         """Closed-loop simulation on the device (see ReactiveQPController.rollout_batch): robot_var /
@@ -238,7 +245,9 @@ class ReactiveNLPController(BaseController):
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None, warmstart_slack_var=None):
         """One controller step -> (robot_vel, virtual_vel | None, slack | None).  Sets
-        self.res = {"x", "f", "status", "iterations"}; a step that did not converge does not raise."""
+        self.res = {"x", "f", "status", "iterations", "lam_g", "lam_x"}; a step that did not converge does not
+        raise.  lam_g (m x 1): the constraint multipliers (multipliers_batch; NaN when not solved, None for skills
+        with more than 32 rows); lam_x (n x 1): zeros (no simple bounds)."""
         spec = self.skill_spec
         if self._cubin is None:
             raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
@@ -271,13 +280,15 @@ class ReactiveNLPController(BaseController):
         sol = np.empty(self._qn)
         status, iters = np.zeros(1, dtype=np.int32), np.zeros(1, dtype=np.int32)
         active = np.zeros(2, dtype=np.uint32)
+        lam = np.empty(self._qm) if self.kernel_meta.get("duals") else None
         vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)  # noqa: E731
         skill = self._skill()
-        runtime.check(skill._lib.clik_nlp_solve_one(
+        runtime.check(skill._lib.clik_nlp_solve_one_lam(
             skill.handle, ctypes.c_double(float(time_var)), vp(q), vp(x), vp(y), vp(warm), vp(sol), vp(status),
-            vp(iters), vp(active), self._max_iter(None)))
+            vp(iters), vp(active), self._max_iter(None), vp(lam)))
         self.res = {"x": dm_column(sol), "f": self._objective(time_var, q, x, y, sol),
-                    "status": int(status[0]), "iterations": int(iters[0])}
+                    "status": int(status[0]), "iterations": int(iters[0]),
+                    "lam_g": None if lam is None else dm_column(lam), "lam_x": cs.DM.zeros(self._qn, 1)}
         res_robot_vel = dm_column(sol[:nrob])
         res_virtual_vel = dm_column(sol[nrob:nrob + nvirt]) if (nvirt > 0 and has_virtual) else None
         off = nrob + self._nxv

@@ -22,7 +22,8 @@ import numpy as np
 from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
-from .base_controller import BaseController, Batch, as_vector, dm_column, resolve_devices, skill_handle_array
+from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
+                              skill_handle_array)
 from .qp_solver import ConicSolver
 
 
@@ -328,6 +329,15 @@ class ReactiveQPController(BaseController):
                                                 b.yp, x0p, a0p, solp, stp, acp, mi))
         return sol, status, active
 
+    def multipliers_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
+        """Constraint multipliers (the reference's lam_a) of a solve_batch result: the step's inputs and its
+        (sol, status, active), same layout rules as solve_batch (torch CUDA tensors on their device and the
+        current stream, NumPy arrays through the host entry point; out= a (m, N) float64 buffer).
+        Returns lam (m, N) float64: > 0 at an upper bound, < 0 at a lower bound, 0 off the working set; NaN for
+        an instance that is not solved or whose working set is rank-deficient (include/clik.h clik_qp_duals).
+        Skills with more than 32 constraint rows raise ValueError."""
+        return multipliers_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
+
     def rollout_batch(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
                       max_speed=None, max_virtual_speed=None, max_iter=None):
         """Closed-loop simulation on the device (see PseudoInverseController.rollout_batch):
@@ -355,7 +365,9 @@ class ReactiveQPController(BaseController):
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None,
               warmstart_slack_var=None):
-        """One controller step -> (robot_vel, virtual_vel | None, slack | None)."""
+        """One controller step -> (robot_vel, virtual_vel | None, slack | None).  Sets self.res = {"x", "status",
+        "active_upper", "active_lower", "cost", "lam_a", "lam_x"}: lam_a (m x 1) are the constraint multipliers
+        (multipliers_batch; None for skills with more than 32 rows), lam_x (n x 1) zeros (no simple bounds)."""
         spec = self.skill_spec
         if self._cubin is None:
             raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
@@ -390,20 +402,21 @@ class ReactiveQPController(BaseController):
         # one instance: the single-instance ABI entry (page-locked mapped slot inside the library)
         import ctypes
         one = getattr(self, "_one", None)
-        if one is None or one["qn"] != self._qn:
+        if one is None or one["qn"] != self._qn or one["lam"].size != self._qm:
             buf = {"qn": self._qn, "sol": np.empty(self._qn), "status": np.zeros(1, dtype=np.int32),
-                   "active": np.zeros(2, dtype=np.uint32)}
-            for k in ("sol", "status", "active"):
+                   "active": np.zeros(2, dtype=np.uint32), "lam": np.empty(self._qm)}
+            for k in ("sol", "status", "active", "lam"):
                 buf[k + "_p"] = ctypes.c_void_p(buf[k].ctypes.data)
             one = self._one = buf
         skill = self._skill()
         mi = int(self.options.get("max_iter", 0) or 0)
-        runtime.check(skill._lib.clik_qp_solve_one(
+        duals = bool(self.kernel_meta.get("duals"))
+        runtime.check(skill._lib.clik_qp_solve_one_lam(
             skill.handle, ctypes.c_double(float(time_var)), ctypes.c_void_p(q.ctypes.data),
             ctypes.c_void_p(x.ctypes.data) if x is not None else None,
             ctypes.c_void_p(y.ctypes.data) if y is not None else None,
             ctypes.c_void_p(warm.ctypes.data) if warm is not None else None,
-            one["sol_p"], one["status_p"], one["active_p"], mi))
+            one["sol_p"], one["status_p"], one["active_p"], mi, one["lam_p"] if duals else None))
         sol, status, active = one["sol"].reshape(-1, 1).copy(), one["status"], one["active"].reshape(2, 1)
         if int(status[0]) != runtime.QP_SOLVED:
             raise RuntimeError("QP %s" % {runtime.QP_INFEASIBLE: "is infeasible",
@@ -414,7 +427,8 @@ class ReactiveQPController(BaseController):
             self.H_func(*self._numeric_args(time_var, q, x, y)).toarray()).diagonal()
         self.res = {"x": dm_column(xs), "status": int(status[0]),
                     "active_upper": int(active[0, 0]), "active_lower": int(active[1, 0]),
-                    "cost": 0.5 * float(np.sum(hdiag * xs * xs))}
+                    "cost": 0.5 * float(np.sum(hdiag * xs * xs)),
+                    "lam_a": dm_column(one["lam"]) if duals else None, "lam_x": cs.DM.zeros(self._qn, 1)}
         res_robot_vel = dm_column(xs[:nrob])
         res_virtual_vel = dm_column(xs[nrob:nrob + nvirt]) if (nvirt > 0 and has_virtual) else None
         off = nrob + self._nxv

@@ -91,6 +91,7 @@ struct clik_skill {
   cudaLibrary_t lib = nullptr;
   KernelInfo pinv, pinv_tma, pinv_rollout, pinv_fast, pinv_group, qp, qp_fast, qp_tail, qp_tail_capped, qp_rollout;
   KernelInfo nlp, nlp_rollout;   // NLP images (manifest flag 256)
+  KernelInfo qp_duals, nlp_duals;   // constraint multipliers (manifest o[18]: bit 0 QP, bit 1 NLP; at most 32 rows)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
@@ -478,6 +479,9 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
     st = setup_kernel(s, "clik_nlp_kernel", &s->nlp);
     if (st == CLIK_OK) st = setup_kernel(s, "clik_nlp_rollout_kernel", &s->nlp_rollout);
   }
+  const int duals = hsz[18];   // multiplier kernels: bit 0 QP, bit 1 NLP
+  if (st == CLIK_OK && (duals & 1)) st = setup_kernel(s, "clik_qp_duals_kernel", &s->qp_duals);
+  if (st == CLIK_OK && (duals & 2)) st = setup_kernel(s, "clik_nlp_duals_kernel", &s->nlp_duals);
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
     delete s;
@@ -952,24 +956,32 @@ clik_status clik_pinv_solve_one(const clik_skill* cs, double t, const double* q,
 
 clik_status clik_qp_solve_one(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
                               const double* x0, double* sol, int32_t* status, uint32_t* active, int32_t max_iter) {
+  return clik_qp_solve_one_lam(cs, t, q, x, y, x0, sol, status, active, max_iter, nullptr);
+}
+
+clik_status clik_qp_solve_one_lam(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
+                                  const double* x0, double* sol, int32_t* status, uint32_t* active, int32_t max_iter,
+                                  double* lam) {
   clik_skill* s = const_cast<clik_skill*>(cs);
   if (!s || !q || !sol) return fail(CLIK_ERR_INVALID, "NULL argument");
   if (!s->qp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the QP kernel");
+  if (lam && !s->qp_duals.kernel)
+    return fail(CLIK_ERR_INVALID, "multipliers need at most 32 constraint rows (the skill has %d)", s->desc.qp_m);
   const clik_skill_desc& d = s->desc;
   if (d.n_virtual > 0 && !x) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x is required");
   if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
   ON_DEVICE(d.device);
   std::lock_guard<std::mutex> lock(s->mu);
-  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n;
-  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3));
+  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n, qm = lam ? d.qp_m : 0;
+  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3 + qm));
   if (st != CLIK_OK) return st;
   double* h = s->one_host;
-  // slot: t | q | x | y | x0 | sol | status, active_up, active_lo (three int cells in two doubles)
+  // slot: t | q | x | y | x0 | sol | status, active_up, active_lo (three int cells in two doubles) | lam
   h[0] = t;
   std::memcpy(h + 1, q, sizeof(double) * nq);
   if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
   if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
-  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn;
+  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
   if (x0) std::memcpy(h + o_x0, x0, sizeof(double) * qn);
   double* dv = s->one_dev;
   long long n = 1, l = 1;
@@ -984,11 +996,18 @@ clik_status clik_qp_solve_one(const clik_skill* cs, double t, const double* q, c
   void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dx0, &da0, &dsol, &dst, &dact, &mi};
   // one instance: the single full kernel (prediction + iteration in one launch)
   CK(cudaLaunchKernel((const void*)s->qp.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
+  if (lam) {
+    // the multipliers at the step's output, same stream: one wait for both launches
+    double* dlam = dv + o_lam;
+    void* largs[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dsol, &dst, &dact, &dlam};
+    CK(cudaLaunchKernel((const void*)s->qp_duals.kernel, dim3(1), dim3(32), largs, 0, s->one_stream));
+  }
   CK(cudaStreamSynchronize(s->one_stream));
   std::memcpy(sol, h + o_sol, sizeof(double) * qn);
   const int* hi = (const int*)(h + o_int);
   if (status) *status = hi[0];
   if (active) { active[0] = (uint32_t)hi[1]; active[1] = (uint32_t)hi[2]; }
+  if (lam) std::memcpy(lam, h + o_lam, sizeof(double) * qm);
   return CLIK_OK;
 }
 
@@ -1107,24 +1126,32 @@ clik_status clik_nlp_step_host_multi(const clik_skill* const* skills, int32_t n_
 clik_status clik_nlp_solve_one(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
                                const double* x0, double* sol, int32_t* status, int32_t* iters, uint32_t* active,
                                int32_t max_iter) {
+  return clik_nlp_solve_one_lam(cs, t, q, x, y, x0, sol, status, iters, active, max_iter, nullptr);
+}
+
+clik_status clik_nlp_solve_one_lam(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
+                                   const double* x0, double* sol, int32_t* status, int32_t* iters, uint32_t* active,
+                                   int32_t max_iter, double* lam) {
   clik_skill* s = const_cast<clik_skill*>(cs);
   if (!s || !q || !sol) return fail(CLIK_ERR_INVALID, "NULL argument");
   if (!s->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
+  if (lam && !s->nlp_duals.kernel)
+    return fail(CLIK_ERR_INVALID, "multipliers need at most 32 constraint rows (the skill has %d)", s->desc.qp_m);
   const clik_skill_desc& d = s->desc;
   if (d.n_virtual > 0 && !x) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x is required");
   if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
   ON_DEVICE(d.device);
   std::lock_guard<std::mutex> lock(s->mu);
-  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n;
-  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3));
+  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n, qm = lam ? d.qp_m : 0;
+  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3 + qm));
   if (st != CLIK_OK) return st;
   double* h = s->one_host;
-  // slot: t | q | x | y | x0 | sol | status, iters, active_up, active_lo (four int cells in two doubles)
+  // slot: t | q | x | y | x0 | sol | status, iters, active_up, active_lo (four int cells in two doubles) | lam
   h[0] = t;
   std::memcpy(h + 1, q, sizeof(double) * nq);
   if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
   if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
-  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn;
+  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
   if (x0) std::memcpy(h + o_x0, x0, sizeof(double) * qn);
   double* dv = s->one_dev;
   long long n = 1, l = 1;
@@ -1138,12 +1165,18 @@ clik_status clik_nlp_solve_one(const clik_skill* cs, double t, const double* q, 
   unsigned* dact = (unsigned*)(dst + 2);      // active[0], active[ld = 1]
   void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dx0, &dsol, &dst, &dit, &dact, &mi};
   CK(cudaLaunchKernel((const void*)s->nlp.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
+  if (lam) {
+    double* dlam = dv + o_lam;
+    void* largs[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dsol, &dst, &dact, &dlam};
+    CK(cudaLaunchKernel((const void*)s->nlp_duals.kernel, dim3(1), dim3(32), largs, 0, s->one_stream));
+  }
   CK(cudaStreamSynchronize(s->one_stream));
   std::memcpy(sol, h + o_sol, sizeof(double) * qn);
   const int* hi = (const int*)(h + o_int);
   if (status) *status = hi[0];
   if (iters) *iters = hi[1];
   if (active) { active[0] = (uint32_t)hi[2]; active[1] = (uint32_t)hi[3]; }
+  if (lam) std::memcpy(lam, h + o_lam, sizeof(double) * qm);
   return CLIK_OK;
 }
 
@@ -1164,6 +1197,118 @@ clik_status clik_nlp_rollout(const clik_skill* s, int64_t N, int32_t steps, doub
   CK(cudaLaunchKernel((const void*)s->nlp_rollout.kernel, dim3(grid_for(s->nlp_rollout, N)),
                       dim3(s->nlp_rollout.block), args, 0, (cudaStream_t)stream));
   return CLIK_OK;
+}
+
+}  // extern "C"
+
+// ---- constraint multipliers of a step's output (clik_duals.cuh) -------------------------------------------
+namespace {
+
+// Arguments of a multiplier call; CLIK_OK with nothing to do when N == 0.
+clik_status duals_check(const clik_skill* s, bool nlp, int64_t N, const double* t, const double* q, const double* x,
+                        const double* y, const double* sol, const int32_t* status, const uint32_t* active,
+                        const double* lam) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  if (!(nlp ? s->nlp.kernel : s->qp.kernel))
+    return fail(CLIK_ERR_INVALID, "skill was built without the %s kernel", nlp ? "NLP" : "QP");
+  if (!(nlp ? s->nlp_duals.kernel : s->qp_duals.kernel))
+    return fail(CLIK_ERR_INVALID, "multipliers need at most 32 constraint rows (the skill has %d)", s->desc.qp_m);
+  clik_status st = check_common(s, N, t, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!sol || !status || !active || !lam) return fail(CLIK_ERR_INVALID, "sol, status, active and lam are required");
+  return CLIK_OK;
+}
+
+clik_status duals_impl(const clik_skill* s, bool nlp, int64_t N, int64_t ld, const double* t, int32_t t_stride,
+                       const double* q, const double* x, const double* y, const double* sol, const int32_t* status,
+                       const uint32_t* active, double* lam, void* stream) {
+  clik_status st = duals_check(s, nlp, N, t, q, x, y, sol, status, active, lam);
+  if (st != CLIK_OK || N == 0) return st;
+  if (ld < N) return fail(CLIK_ERR_INVALID, "row stride ld (%lld) < N (%lld)", (long long)ld, (long long)N);
+  const KernelInfo& k = nlp ? s->nlp_duals : s->qp_duals;
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = ld;
+  int ts = t_stride ? 1 : 0;
+  void* args[] = {&n, &l, &t, &ts, &q, &x, &y, &sol, &status, &active, &lam};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+// Host arrays (as nlp_host_range): the kernel on mapped memory when every buffer is page-locked, else the
+// chunked copy pipeline.
+clik_status duals_host(clik_skill* s, bool nlp, int64_t N, const double* t, int32_t t_stride, const double* q,
+                       const double* x, const double* y, const double* sol, const int32_t* status,
+                       const uint32_t* active, double* lam) {
+  clik_status st = duals_check(s, nlp, N, t, q, x, y, sol, status, active, lam);
+  if (st != CLIK_OK || N == 0) return st;
+  const clik_skill_desc& d = s->desc;
+  if (zero_copy_enabled()) {
+    const void *dt, *dq, *dx, *dy, *dsol, *dst, *dact, *dlam;
+    ON_DEVICE(d.device);
+    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
+        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(sol, &dsol) && device_alias(status, &dst) &&
+        device_alias(active, &dact) && device_alias(lam, &dlam)) {
+      std::lock_guard<std::mutex> lock(s->mu);
+      clik_status zs = ensure_scratch(s, 0, 256);
+      if (zs != CLIK_OK) return zs;
+      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
+      zs = duals_impl(s, nlp, N, N, (const double*)dt, t_stride, (const double*)dq, (const double*)dx,
+                      (const double*)dy, (const double*)dsol, (const int32_t*)dst, (const uint32_t*)dact,
+                      (double*)dlam, s->scratch.stream[0]);
+      if (zs != CLIK_OK) return zs;
+      CK(cudaStreamSynchronize(s->scratch.stream[0]));
+      return CLIK_OK;
+    }
+  }
+  std::vector<Field> f;
+  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
+  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
+  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
+  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
+  f[0].rowmask = s->qp_reads.t;
+  f[1].rowmask = s->qp_reads.q;
+  f[2].rowmask = s->qp_reads.x;
+  f[3].rowmask = s->qp_reads.y;
+  f.push_back({sol, nullptr, d.qp_n, 8, 1, 0});
+  f.push_back({status, nullptr, 1, 4, 1, 0});
+  f.push_back({active, nullptr, 2, 4, 1, 0});
+  f.push_back({nullptr, lam, d.qp_m, 8, 1, 0});
+  return run_host_pipeline(s, N, 0, N, f, [&](char* base, int64_t c, cudaStream_t stream) {
+    return duals_impl(s, nlp, c, c, (const double*)(base + f[0].dev_off), t_stride,
+                      (const double*)(base + f[1].dev_off),
+                      d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
+                      d.n_input ? (const double*)(base + f[3].dev_off) : nullptr, (const double*)(base + f[4].dev_off),
+                      (const int32_t*)(base + f[5].dev_off), (const uint32_t*)(base + f[6].dev_off),
+                      (double*)(base + f[7].dev_off), stream);
+  });
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_qp_duals(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                          const double* x, const double* y, const double* sol, const int32_t* status,
+                          const uint32_t* active, double* lam, void* stream) {
+  return duals_impl(s, false, N, N, t, t_stride, q, x, y, sol, status, active, lam, stream);
+}
+
+clik_status clik_nlp_duals(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                           const double* x, const double* y, const double* sol, const int32_t* status,
+                           const uint32_t* active, double* lam, void* stream) {
+  return duals_impl(s, true, N, N, t, t_stride, q, x, y, sol, status, active, lam, stream);
+}
+
+clik_status clik_qp_duals_host(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                               const double* x, const double* y, const double* sol, const int32_t* status,
+                               const uint32_t* active, double* lam) {
+  return duals_host(const_cast<clik_skill*>(s), false, N, t, t_stride, q, x, y, sol, status, active, lam);
+}
+
+clik_status clik_nlp_duals_host(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                                const double* x, const double* y, const double* sol, const int32_t* status,
+                                const uint32_t* active, double* lam) {
+  return duals_host(const_cast<clik_skill*>(s), true, N, t, t_stride, q, x, y, sol, status, active, lam);
 }
 
 clik_status clik_measure_fp64_peak(int32_t device, int32_t iters, double* tflops) {

@@ -38,6 +38,8 @@ EXPORTS = (
     "clik_pinv_solve_one", "clik_qp_solve_one", "clik_skill_set_overlap", "clik_skill_get_overlap",
     "clik_nlp_step", "clik_nlp_step_host", "clik_nlp_solve_one", "clik_nlp_rollout",
     "clik_nlp_step_ld", "clik_nlp_step_host_multi",
+    "clik_qp_duals", "clik_nlp_duals", "clik_qp_duals_host", "clik_nlp_duals_host",
+    "clik_qp_solve_one_lam", "clik_nlp_solve_one_lam",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -116,6 +118,16 @@ def load_library():
     lib.clik_nlp_rollout.restype = i32
     lib.clik_nlp_rollout.argtypes = [vp, i64, i32, ctypes.c_double, vp, i32, vp, vp, vp,
                                      ctypes.c_double, ctypes.c_double, vp, vp, i32, vp]
+    for name in ("clik_qp_duals", "clik_nlp_duals"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]
+    for name in ("clik_qp_duals_host", "clik_nlp_duals_host"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.clik_qp_solve_one_lam.restype = i32
+    lib.clik_qp_solve_one_lam.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, i32, vp]
+    lib.clik_nlp_solve_one_lam.restype = i32
+    lib.clik_nlp_solve_one_lam.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.clik_skill_launch_info.restype = i32
     lib.clik_skill_launch_info.argtypes = [vp, i32, _c_int32_p, _c_int32_p, _c_int32_p, _c_int32_p]
     lib.clik_skill_set_overlap.restype = i32

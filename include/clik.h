@@ -231,6 +231,43 @@ clik_status clik_qp_solve_one(const clik_skill* skill, double t, const double* q
                               const double* y, const double* x0, double* sol, int32_t* status,
                               uint32_t* active, int32_t max_iter);
 
+/* The same single-instance steps with the constraint multipliers of the result (see clik_qp_duals):
+ * lam [qp_m] out, or NULL.  The step and the multiplier kernel are launched back to back on the skill's
+ * stream with one wait.  clik_qp_solve_one / clik_nlp_solve_one are these calls with lam = NULL, with
+ * bit-identical results.  A non-NULL lam on a skill with more than 32 rows fails with CLIK_ERR_INVALID. */
+clik_status clik_qp_solve_one_lam(const clik_skill* skill, double t, const double* q, const double* x,
+                                  const double* y, const double* x0, double* sol, int32_t* status,
+                                  uint32_t* active, int32_t max_iter, double* lam);
+clik_status clik_nlp_solve_one_lam(const clik_skill* skill, double t, const double* q, const double* x,
+                                   const double* y, const double* x0, double* sol, int32_t* status,
+                                   int32_t* iters, uint32_t* active, int32_t max_iter, double* lam);
+
+/* Constraint multipliers of a step's output (the reference's lam_a of cs.conic, lam_g of cs.nlpsol), for N
+ * instances: the inputs of the step (t, q, x, y as clik_qp_step / clik_nlp_step) and its outputs
+ *   sol [qp_n * N], status [N], active [2 * N]   (all required)
+ *   lam [qp_m * N] out: lam[r*N + i], CasADi's sign convention (> 0 at an upper bound, < 0 at a lower bound,
+ *       any sign on an equality row), 0 on the rows outside the working set.
+ * lam_W = argmin |D^1/2 (g + A_W' lam)| on the working set W of `active`, by modified Gram-Schmidt QR: for the QP
+ * g = H x and D = H^-1 (exact stationarity of the face problem), for the NLP g = grad F(x) and D = I.  Every entry
+ * of instance i is NaN when status[i] is not 0 (solved), or when the rows of W are linearly dependent (a QR pivot
+ * below 1e-12 times the largest column norm).  One thread per instance.  The working-set masks describe rows
+ * below 32 only: a skill with more than 32 rows has no multiplier kernel and the call fails with
+ * CLIK_ERR_INVALID, "multipliers need at most 32 constraint rows".  clik_qp_duals takes QP images,
+ * clik_nlp_duals NLP images.  Device pointers, asynchronous on `stream`; the _host forms take host arrays and
+ * are synchronous (zero copy on page-locked buffers, else the chunked pipeline), with bit-identical results. */
+clik_status clik_qp_duals(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                          const double* q, const double* x, const double* y, const double* sol,
+                          const int32_t* status, const uint32_t* active, double* lam, void* stream);
+clik_status clik_nlp_duals(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                           const double* q, const double* x, const double* y, const double* sol,
+                           const int32_t* status, const uint32_t* active, double* lam, void* stream);
+clik_status clik_qp_duals_host(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                               const double* q, const double* x, const double* y, const double* sol,
+                               const int32_t* status, const uint32_t* active, double* lam);
+clik_status clik_nlp_duals_host(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                                const double* q, const double* x, const double* y, const double* sol,
+                                const int32_t* status, const uint32_t* active, double* lam);
+
 /* One host batch over several GPUs of the box: `skills[k]` is the same cubin loaded on device k
  * (clik_skill_load with desc.device = k); the batch is cut into n_skills contiguous shards (sizes differ
  * by at most one, shard k = [k*N/n .. )), each shard runs on its device from its own host thread (zero
