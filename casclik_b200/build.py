@@ -96,7 +96,7 @@ def build_library(force=False, verbose=False):
 
 def _kernel_headers():
     return [os.path.join(CSRC_DIR, f) for f in ("clik_pinv.cuh", "clik_pinv_group.cuh", "clik_qp.cuh", "clik_nlp.cuh",
-                                                   "clik_math.cuh", "clik_duals.cuh")]
+                                                   "clik_math.cuh", "clik_duals.cuh", "clik_vjp.cuh")]
 
 
 def source_hash(source: str) -> str:

@@ -339,9 +339,11 @@ def _switch(name, values, ret="int"):
 
 
 def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None,
-               nlp=None, nlp_tol=1e-10):
+               nlp=None, nlp_tol=1e-10, vjp=False):
     """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None; or `nlp`:
-    NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).
+    NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).  `vjp`: also append the reverse-mode
+    derivative kernel of the QP / NLP step (clik_vjp.cuh) after the multiplier kernel, for skills that have
+    one; everything emitted before it is the same text as with vjp=False.
     Tuning knobs (also settable through the environment for experiments): CLIK_BLOCK,
     CLIK_MINBLOCKS, CLIK_CONSTBANK (1), CLIK_FAST_SINCOS (1)."""
     if block_threads is None:
@@ -349,7 +351,7 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     if nlp is not None:
         if pinv is not None or qp is not None:
             raise ValueError("an NLP image holds the NLP kernels only")
-        return _emit_nlp(nlp, label, block_threads, nlp_tol)
+        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp)
     env_min_blocks = int(os.environ.get("CLIK_MINBLOCKS", "0"))
     if min_blocks is None:
         min_blocks = env_min_blocks
@@ -732,9 +734,15 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     meta["duals"] = qp is not None and 0 < qp.m <= DUALS_MAX_ROWS
     if meta["duals"]:
         out.append("  o[18] = 1;   // multiplier kernels (1 QP, 2 NLP)")
+    meta["vjp"] = bool(vjp) and meta["duals"]
+    if meta["vjp"]:
+        out.append(_VJP_MANIFEST % 1)
     out.append("}")
     if meta["duals"]:
         out += _emit_qp_duals(qp, sig, sincos_name, block_threads, meta["qp_structured"])
+    if meta["vjp"]:
+        out += _emit_vjp(qp, "qp", sig, sincos_name, block_threads,
+                         "SkillDuals" if meta["qp_structured"] else "Skill", meta["qp_read_masks"], meta)
     return "\n".join(out) + "\n", meta
 
 
@@ -772,6 +780,50 @@ def _emit_qp_duals(qp, sig, sincos_name, block_threads, structured):
     return out
 
 
+_VJP_MANIFEST = "  o[19] = %d;   // VJP kernels (1 QP, 2 NLP)"
+
+
+def _emit_vjp(prog, kind, sig, sincos_name, block_threads, base, base_masks, meta):
+    """clik_<kind>_vjp_kernel (clik_vjp.cuh), appended after the multiplier kernel: a struct derived from `base`
+    (the struct whose eval_qp / eval_nlp_pre the multiplier kernel reads) adds eval_vjp, the gradient program of
+    Phi (codegen/vjp.py), and the rows the kernel loads (those of `base_masks` and those eval_vjp reads).  Its
+    constants are literals, so the constant bank of the step kernels stays as it is."""
+    from .vjp import VjpProgram
+    vp = VjpProgram(prog, kind)
+    em = Emitter(vp.names, None, sincos_name)
+    em.assign("tb", vp.t)
+    for arr, nodes in (("qb", vp.q), ("xb", vp.x), ("yb", vp.y)):
+        for j, n in enumerate(nodes):
+            em.assign("%s[%d]" % (arr, j), n)
+    masks = tuple(a | b for a, b in zip(base_masks, em.read_masks(prog.syms)))
+    meta["vjp_eval"] = em.counts()
+    meta["vjp_read_masks"] = masks
+    n, m = prog.nx, prog.m
+    out = ["", "// ---- reverse-mode derivative of the step's output (clik_vjp.cuh) ----",
+           '#include "clik_vjp.cuh"',
+           "struct SkillVjp : %s {" % base,
+           "  using Base = %s;   // the struct whose row evaluation the kernel calls" % base,
+           "  static constexpr unsigned VJP_READ_T = %du, VJP_READ_Q = 0x%xu, VJP_READ_X = 0x%xu, VJP_READ_Y = 0x%xu;"
+           % masks,
+           "  __device__ static __forceinline__ void eval_vjp(%s," % sig,
+           "      const double (&xs_)[%d], const double (&lam_)[%d], const double (&u_)[%d], const double (&vu_)[%d],"
+           % (n, m, n, m),
+           "      const double (&vl_)[%d], double& tb, double (&qb)[%d], double (&xb)[%d], double (&yb)[%d]) {"
+           % (m, max(prog.n_rob, 1), max(prog.n_virt, 1), max(prog.n_in, 1))]
+    out += ["    " + ln for ln in em.finish()]
+    out += ["  }",
+            "};",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_vjp_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,",
+            "    const double* y, const double* sol, const int* status, const unsigned* active, const double* sol_bar,",
+            "    double* t_bar, double* q_bar, double* x_bar, double* y_bar) {",
+            "  clik::%s_vjp<SkillVjp>(N, ld, t, t_stride, q, x, y, sol, status, active, sol_bar, t_bar, q_bar, x_bar,"
+            % kind,
+            "                         y_bar);",
+            "}"]
+    return out
+
+
 def nlp_hoisted(nlp):
     """The maximal decision-free subexpressions the cost graph (F, g, H) consumes: every non-constant
     argument without a decision symbol below it of a node that has one, and every output without one.
@@ -796,7 +848,7 @@ def nlp_hoisted(nlp):
     return P
 
 
-def _emit_nlp(nlp, label, block_threads, tol):
+def _emit_nlp(nlp, label, block_threads, tol, vjp=False):
     """Translation unit of the reactive-NLP controller (csrc/clik_nlp.cuh instantiated on the skill)."""
     const_table = [] if os.environ.get("CLIK_CONSTBANK", "1") == "1" else None
     sincos_name = "clik::sincos_fast" if os.environ.get("CLIK_FAST_SINCOS", "1") == "1" else "sincos"
@@ -895,6 +947,9 @@ def _emit_nlp(nlp, label, block_threads, tol):
     meta["duals"] = 0 < m <= DUALS_MAX_ROWS
     if meta["duals"]:
         out.append("  o[18] = 2;   // multiplier kernels (1 QP, 2 NLP)")
+    meta["vjp"] = bool(vjp) and meta["duals"]
+    if meta["vjp"]:
+        out.append(_VJP_MANIFEST % 2)
     out.append("}")
     if meta["duals"]:
         out += ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
@@ -904,6 +959,8 @@ def _emit_nlp(nlp, label, block_threads, tol):
                 "    const double* y, const double* sol, const int* status, const unsigned* active, double* lam) {",
                 "  clik::nlp_duals<Skill>(N, ld, t, t_stride, q, x, y, sol, status, active, lam);",
                 "}"]
+    if meta["vjp"]:
+        out += _emit_vjp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
     return "\n".join(out) + "\n", meta
 
 

@@ -4,8 +4,8 @@ import ctypes
 
 import numpy as np
 
+from .. import build, runtime
 from .. import sym as cs
-from .. import runtime
 
 
 class BaseController(object):
@@ -73,6 +73,108 @@ def multipliers_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, s
         runtime.check(getattr(lib, "clik_%s_duals_host" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp,
                                                                  b.yp, solp, stp, acp, lamp))
     return lam
+
+
+def vjp_image(ctrl, kind, device):
+    """The skill's VJP image (emit_skill(..., vjp=True): the default image plus clik_<kind>_vjp_kernel) loaded on
+    `device`.  Built and loaded on the first call, cached like every cubin, one handle per device: a controller
+    that never asks for derivatives compiles nothing more."""
+    if ctrl._vjp is None:
+        source, meta = ctrl._vjp_source()
+        cubin, path = build.compile_cubin(source, tag="%s_vjp_%s" % (kind, ctrl.skill_spec.label))
+        ctrl._vjp = {"source": source, "meta": meta, "cubin": cubin, "path": path, "skills": {}}
+    skills = ctrl._vjp["skills"]
+    if device not in skills:
+        skills[device] = runtime.CompiledSkill(ctrl._vjp["cubin"], ctrl._vjp["meta"],
+                                               n_slack=ctrl.skill_spec.n_slack_var, device=device)
+    return skills[device]
+
+
+def vjp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out):
+    """Shared body of ReactiveQPController / ReactiveNLPController.vjp_batch (`kind` "qp" or "nlp"): validates the
+    step's inputs, outputs and the cotangent like multipliers_batch and calls clik_<kind>_vjp on the current
+    stream.  -> (t_bar (N,), q_bar (n_robot, N), x_bar (n_virtual, N) | None, y_bar (n_input, N) | None)."""
+    if ctrl._cubin is None:
+        raise RuntimeError("call setup_problem_functions() / setup_solver() before vjp_batch()")
+    if not ctrl.kernel_meta.get("duals"):
+        raise ValueError("the VJP needs at most 32 constraint rows and at least one (the skill has %d)" % ctrl._qm)
+    if not (runtime._is_torch(robot_var) and robot_var.is_cuda):
+        raise ValueError("vjp_batch needs torch CUDA tensors (there is no host-array form)")
+    spec = ctrl.skill_spec
+    b = Batch(spec.n_robot_var, ctrl._nxv, ctrl._ny, time_var, robot_var, virtual_var,
+              input_var if ctrl._ny else None)
+    if sol is None or status is None or active is None or sol_bar is None:
+        raise ValueError("sol, status and active of the step and the cotangent sol_bar are required")
+    if not all(runtime._is_torch(a) for a in (sol, status, active, sol_bar)):
+        raise ValueError("sol, status, active and sol_bar must be CUDA tensors")
+    solp = runtime.dev_ptr(sol, "f64", ctrl._qn * b.N, "sol")
+    stp = runtime.dev_ptr(status, "i32", b.N, "status")
+    acp = runtime.dev_ptr(active, "u32", 2 * b.N, "active")
+    sbp = runtime.dev_ptr(sol_bar, "f64", ctrl._qn * b.N, "sol_bar")
+    if any(a.device != b.device for a in (sol, status, active, sol_bar)):
+        raise ValueError("sol, status, active and sol_bar must live on %s like robot_var" % b.device)
+    rows = (0, spec.n_robot_var, ctrl._nxv, ctrl._ny)
+    names = ("t_bar", "q_bar", "x_bar", "y_bar")
+    if out is None:
+        out = [b.empty(r) if (r or k == 0) else None for k, r in enumerate(rows)]
+    else:
+        out = list(out)
+        if len(out) != 4:
+            raise ValueError("out=(t_bar, q_bar, x_bar, y_bar)")
+        for k, r in enumerate(rows):
+            if (r or k == 0) and out[k] is None:
+                raise runtime.ClikError("out[%d] (%s) is required" % (k, names[k]))
+            if not (r or k == 0):
+                out[k] = None
+    ptrs = [b.out_ptr(a, r, "f64", "out[%d] (%s)" % (k, names[k])) if a is not None else None
+            for k, (a, r) in enumerate(zip(out, rows))]
+    skill = vjp_image(ctrl, kind, b.device_index)
+    lib = runtime.load_library()
+    runtime.check(getattr(lib, "clik_%s_vjp" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, solp, stp,
+                                                      acp, sbp, *ptrs, b.stream()))
+    return tuple(out)
+
+
+_STEP_FUNCTION = []
+
+
+def _step_function():
+    """torch.autograd.Function of a controller step: forward solve_batch, backward vjp_batch."""
+    if _STEP_FUNCTION:
+        return _STEP_FUNCTION[0]
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class ControllerStep(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, ctrl, t, q, x, y, warmstart, max_iter):
+            outs = ctrl.solve_batch(t, q, x, y, warmstart=warmstart, max_iter=max_iter)
+            ctx.ctrl, ctx.t = ctrl, t
+            ctx.save_for_backward(q, x, y, *outs[:3])
+            ctx.mark_non_differentiable(*outs[1:])
+            return outs
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, sol_bar, *unused):
+            q, x, y, sol, status, active = ctx.saved_tensors
+            ctrl, t = ctx.ctrl, ctx.t
+            t_bar, q_bar, x_bar, y_bar = ctrl.vjp_batch(t, q, x, y, sol, status, active, sol_bar.contiguous())
+            t_grad = None
+            if torch.is_tensor(t):
+                t_grad = (t_bar.sum() if t.numel() == 1 else t_bar).reshape(t.shape).to(t.dtype)
+            return (None, t_grad, q_bar, x_bar if x is not None else None, y_bar if y is not None else None,
+                    None, None)
+
+    _STEP_FUNCTION.append(ControllerStep)
+    return ControllerStep
+
+
+def solve_batch_differentiable(ctrl, time_var, robot_var, virtual_var, input_var, warmstart, max_iter):
+    """Shared body of the controllers' solve_batch_differentiable."""
+    if not (runtime._is_torch(robot_var) and robot_var.is_cuda):
+        raise ValueError("solve_batch_differentiable needs torch CUDA tensors")
+    return _step_function().apply(ctrl, time_var, robot_var, virtual_var, input_var, warmstart, max_iter)
 
 
 def skill_handle_array(skills):

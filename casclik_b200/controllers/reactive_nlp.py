@@ -22,7 +22,7 @@ from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
-                              skill_handle_array)
+                              skill_handle_array, solve_batch_differentiable, vjp_batch)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -55,6 +55,7 @@ class ReactiveNLPController(BaseController):
         self.options = options
         self._cubin = None
         self._compiled = None
+        self._vjp = None
         self._has_initial = False
         self.res = None
         self._prog = self._program()     # validates the cost and the problem size now
@@ -128,6 +129,7 @@ class ReactiveNLPController(BaseController):
         self.row_labels = prog.labels
         self._cubin = cubin
         self._compiled = None
+        self._vjp = None
         if load:
             self._skill()
 
@@ -218,6 +220,22 @@ class ReactiveNLPController(BaseController):
         ReactiveQPController.multipliers_batch: lam (m, N) float64 with grad F + A' lam = 0 on the last
         subproblem's working set; NaN for an instance whose status is not 0 (include/clik.h clik_nlp_duals)."""
         return multipliers_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
+
+    def _vjp_source(self):
+        """Source of the VJP image: the default image plus the VJP kernel."""
+        return emit_skill(nlp=self._prog, label=self.skill_spec.label, nlp_tol=float(self.options["tol"]), vjp=True)
+
+    def vjp_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out=None):
+        """Reverse-mode derivative of a solve_batch result, as ReactiveQPController.vjp_batch; the adjoint solve
+        uses the Hessian of the cost at sol, factored without a shift: an instance whose Hessian is not positive
+        definite there gets NaN (include/clik.h clik_nlp_vjp)."""
+        return vjp_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out)
+
+    def solve_batch_differentiable(self, time_var, robot_var, virtual_var=None, input_var=None, warmstart=None,
+                                   max_iter=None):
+        """solve_batch on torch CUDA tensors as a torch.autograd.Function (see
+        ReactiveQPController.solve_batch_differentiable): (sol, status, active, iterations), sol differentiable."""
+        return solve_batch_differentiable(self, time_var, robot_var, virtual_var, input_var, warmstart, max_iter)
 
     def rollout_batch(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
                       max_speed=None, max_virtual_speed=None, max_iter=None):

@@ -23,7 +23,7 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
-                              skill_handle_array)
+                              skill_handle_array, solve_batch_differentiable, vjp_batch)
 from .qp_solver import ConicSolver
 
 
@@ -69,6 +69,7 @@ class ReactiveQPController(BaseController):
         self.options = options
         self._compiled = None
         self._cubin = None
+        self._vjp = None
         self._has_initial = False
         self.res = None
 
@@ -200,6 +201,7 @@ class ReactiveQPController(BaseController):
         self._h_const = (np.array([n.val for n in prog.h]) if all(n.is_const for n in prog.h) else None)
         self._cubin = cubin
         self._compiled = None
+        self._vjp = None
         ins, names = self._input_list()
         H = cs.diag(cs.MX(cs.vertcat(*prog.h)))
         A = cs.MX(cs.vertcat(*[cs.horzcat(*row) for row in prog.A]))
@@ -337,6 +339,30 @@ class ReactiveQPController(BaseController):
         an instance that is not solved or whose working set is rank-deficient (include/clik.h clik_qp_duals).
         Skills with more than 32 constraint rows raise ValueError."""
         return multipliers_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
+
+    def _vjp_source(self):
+        """Source of the VJP image: the default image's emission (same fast-kernel register cap) plus the VJP kernel."""
+        return emit_skill(qp=self._program(), label=self.skill_spec.label, vjp=True,
+                          qp_fast_min_blocks=self.kernel_meta.get("qp_fast_min_blocks"))
+
+    def vjp_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out=None):
+        """Reverse-mode derivative (vector-Jacobian product) of a solve_batch result: the step's inputs and its
+        (sol, status, active) as torch CUDA tensors, and the cotangent sol_bar (nx, N) float64 of sol.  Runs on the
+        current stream.  Returns (t_bar (N,), q_bar (n_robot, N), x_bar (n_virtual, N) | None, y_bar (n_input, N) |
+        None): (d sol / d theta)' sol_bar for the face problem of the returned working set, the one-sided derivative
+        that keeps the working set where a held row has a zero multiplier (DESIGN.md §4.6).  t_bar is per instance
+        also for a shared t.  An all-zero cotangent column gives exactly 0; otherwise an unsolved instance or a
+        rank-deficient working set gives NaN (include/clik.h clik_qp_vjp).  out= (t_bar, q_bar, x_bar, y_bar)
+        buffers of those shapes.  The VJP image is compiled and loaded on the first call (one per device).
+        NumPy inputs and skills with more than 32 constraint rows raise ValueError."""
+        return vjp_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out)
+
+    def solve_batch_differentiable(self, time_var, robot_var, virtual_var=None, input_var=None, warmstart=None,
+                                   max_iter=None):
+        """solve_batch on torch CUDA tensors as a torch.autograd.Function: (sol, status, active) with sol attached
+        to the graph of time_var, robot_var, virtual_var and input_var (backward: vjp_batch); status and active are
+        not differentiable.  A 0-d / one-element tensor t gets the summed t_bar; a Python float t gets none."""
+        return solve_batch_differentiable(self, time_var, robot_var, virtual_var, input_var, warmstart, max_iter)
 
     def rollout_batch(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
                       max_speed=None, max_virtual_speed=None, max_iter=None):

@@ -92,6 +92,7 @@ struct clik_skill {
   KernelInfo pinv, pinv_tma, pinv_rollout, pinv_fast, pinv_group, qp, qp_fast, qp_tail, qp_tail_capped, qp_rollout;
   KernelInfo nlp, nlp_rollout;   // NLP images (manifest flag 256)
   KernelInfo qp_duals, nlp_duals;   // constraint multipliers (manifest o[18]: bit 0 QP, bit 1 NLP; at most 32 rows)
+  KernelInfo qp_vjp, nlp_vjp;       // reverse-mode derivative of the step (manifest o[19]: bit 0 QP, bit 1 NLP)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
@@ -429,6 +430,9 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
     } else {
       int* dsz = nullptr;
       cudaError_t le = cudaMalloc(&dsz, sizeof(hsz));
+      // slots an image does not write (o[18], o[19] of older or pinv-only images) must read 0, not whatever the
+      // allocation held before
+      if (le == cudaSuccess) le = cudaMemset(dsz, 0, sizeof(hsz));
       if (le == cudaSuccess) {
         void* args[] = {&dsz};
         le = cudaLaunchKernel((const void*)probe, dim3(1), dim3(1), args, 0, nullptr);
@@ -482,6 +486,9 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
   const int duals = hsz[18];   // multiplier kernels: bit 0 QP, bit 1 NLP
   if (st == CLIK_OK && (duals & 1)) st = setup_kernel(s, "clik_qp_duals_kernel", &s->qp_duals);
   if (st == CLIK_OK && (duals & 2)) st = setup_kernel(s, "clik_nlp_duals_kernel", &s->nlp_duals);
+  const int vjp = hsz[19];     // VJP kernels (images built with emit_skill(..., vjp=True)): bit 0 QP, bit 1 NLP
+  if (st == CLIK_OK && (vjp & 1)) st = setup_kernel(s, "clik_qp_vjp_kernel", &s->qp_vjp);
+  if (st == CLIK_OK && (vjp & 2)) st = setup_kernel(s, "clik_nlp_vjp_kernel", &s->nlp_vjp);
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
     delete s;
@@ -1309,6 +1316,52 @@ clik_status clik_nlp_duals_host(const clik_skill* s, int64_t N, const double* t,
                                 const double* x, const double* y, const double* sol, const int32_t* status,
                                 const uint32_t* active, double* lam) {
   return duals_host(const_cast<clik_skill*>(s), true, N, t, t_stride, q, x, y, sol, status, active, lam);
+}
+
+}  // extern "C"
+
+// ---- reverse-mode derivative of a step's output (clik_vjp.cuh) -------------------------------------------
+namespace {
+
+clik_status vjp_impl(const clik_skill* s, bool nlp, int64_t N, const double* t, int32_t t_stride, const double* q,
+                     const double* x, const double* y, const double* sol, const int32_t* status,
+                     const uint32_t* active, const double* sol_bar, double* t_bar, double* q_bar, double* x_bar,
+                     double* y_bar, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_vjp : s->qp_vjp;
+  if (!k.kernel)
+    return fail(CLIK_ERR_INVALID, "skill image has no %s VJP kernel (build it with emit_skill(..., vjp=True); at most "
+                "32 constraint rows)", nlp ? "NLP" : "QP");
+  clik_status st = check_common(s, N, t, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!sol || !status || !active || !sol_bar || !t_bar || !q_bar)
+    return fail(CLIK_ERR_INVALID, "sol, status, active, sol_bar, t_bar and q_bar are required");
+  if (s->desc.n_virtual > 0 && !x_bar) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x_bar is required");
+  if (s->desc.n_input > 0 && !y_bar) return fail(CLIK_ERR_INVALID, "skill reads input_var: y_bar is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0;
+  void* args[] = {&n, &l, &t, &ts, &q, &x, &y, &sol, &status, &active, &sol_bar, &t_bar, &q_bar, &x_bar, &y_bar};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_qp_vjp(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                        const double* x, const double* y, const double* sol, const int32_t* status,
+                        const uint32_t* active, const double* sol_bar, double* t_bar, double* q_bar, double* x_bar,
+                        double* y_bar, void* stream) {
+  return vjp_impl(s, false, N, t, t_stride, q, x, y, sol, status, active, sol_bar, t_bar, q_bar, x_bar, y_bar, stream);
+}
+
+clik_status clik_nlp_vjp(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                         const double* x, const double* y, const double* sol, const int32_t* status,
+                         const uint32_t* active, const double* sol_bar, double* t_bar, double* q_bar, double* x_bar,
+                         double* y_bar, void* stream) {
+  return vjp_impl(s, true, N, t, t_stride, q, x, y, sol, status, active, sol_bar, t_bar, q_bar, x_bar, y_bar, stream);
 }
 
 clik_status clik_measure_fp64_peak(int32_t device, int32_t iters, double* tflops) {

@@ -28,16 +28,12 @@
 
 namespace clik {
 
-// A: M x N row-major, s = D^1/2 (diagonal), g: gradient; up / lo: working-set masks.  Writes lam[0..M);
-// false (lam all NaN) when A_W is rank-deficient.
+// Working set of the masks up / lo: rows W[0..k) in ascending order, lam[r] = 0 for every row; false when more
+// rows are held than there are variables (dependent).
 template <int N, int M>
-__device__ __forceinline__ bool working_set_multipliers(const double* A, const double* s, const double* g,
-                                                        unsigned up, unsigned lo, double* lam) {
+__device__ __forceinline__ bool working_set_rows(unsigned up, unsigned lo, int (&W)[N], int& k, double* lam) {
   static_assert(M <= 32, "the working-set masks describe rows below 32 only");
-  int W[N];
-  double Q[N * N], R[N * N], c[N], b[N];
-  int k = 0;
-  bool ok = true;
+  k = 0;
   for (int r = 0; r < M; ++r) {
     lam[r] = 0.0;
     if (((up | lo) >> r) & 1u) {
@@ -45,18 +41,22 @@ __device__ __forceinline__ bool working_set_multipliers(const double* A, const d
       ++k;
     }
   }
-  if (k > N) ok = false;                 // more held rows than variables: dependent
+  return k <= N;
+}
+
+// QR step: Q holds k pre-scaled columns D^1/2 a_r (N entries each) on entry and their orthonormal basis on
+// return, R (N x N, upper) the factor.  Modified Gram-Schmidt, two orthogonalisation passes; false when a
+// pivot falls below 1e-12 max_r |D^1/2 a_r| (rank-deficient).
+template <int N>
+__device__ __forceinline__ bool working_set_qr(int k, double* Q, double* R) {
   double cmax = 0.0;
-  for (int a = 0; a < k && ok; ++a) {
-    double* col = &Q[a * N];
+  for (int a = 0; a < k; ++a) {
+    const double* col = &Q[a * N];
     double nrm = 0.0;
-    for (int j = 0; j < N; ++j) {
-      col[j] = s[j] * A[W[a] * N + j];
-      nrm = fma(col[j], col[j], nrm);
-    }
+    for (int j = 0; j < N; ++j) nrm = fma(col[j], col[j], nrm);
     cmax = fmax(cmax, sqrt(nrm));
   }
-  for (int a = 0; a < k && ok; ++a) {
+  for (int a = 0; a < k; ++a) {
     double* col = &Q[a * N];
     for (int pass = 0; pass < 2; ++pass) {
       for (int l = 0; l < a; ++l) {
@@ -69,17 +69,22 @@ __device__ __forceinline__ bool working_set_multipliers(const double* A, const d
     double nrm = 0.0;
     for (int j = 0; j < N; ++j) nrm = fma(col[j], col[j], nrm);
     nrm = sqrt(nrm);
-    if (!(nrm > 1e-12 * cmax)) { ok = false; break; }
+    if (!(nrm > 1e-12 * cmax)) return false;
     R[a * N + a] = nrm;
     const double inv = 1.0 / nrm;
     for (int j = 0; j < N; ++j) col[j] *= inv;
   }
-  if (!ok) {
-    for (int r = 0; r < M; ++r) lam[r] = NAN;
-    return false;
-  }
-  // c = Q' b with b = -D^1/2 g, projected out column by column (two passes, as above)
-  for (int j = 0; j < N; ++j) b[j] = -s[j] * g[j];
+  return true;
+}
+
+// Solve step: c = argmin |sg + (Q R) c| for the pre-scaled gradient sg = D^1/2 g, i.e. R c = -Q' sg
+// (c = Q' b with b = -sg projected out column by column, two passes, then back substitution).  Writes
+// lam[W[a]] = c[a].
+template <int N>
+__device__ __forceinline__ void working_set_solve(int k, const int* W, const double* Q, const double* R,
+                                                  const double* sg, double* lam) {
+  double c[N], b[N];
+  for (int j = 0; j < N; ++j) b[j] = -sg[j];
   for (int a = 0; a < k; ++a) c[a] = 0.0;
   for (int pass = 0; pass < 2; ++pass) {
     for (int a = 0; a < k; ++a) {
@@ -95,6 +100,28 @@ __device__ __forceinline__ bool working_set_multipliers(const double* A, const d
     c[a] = acc / R[a * N + a];
     lam[W[a]] = c[a];
   }
+}
+
+// A: M x N row-major, s = D^1/2 (diagonal), g: gradient; up / lo: working-set masks.  Writes lam[0..M);
+// false (lam all NaN) when A_W is rank-deficient.
+template <int N, int M>
+__device__ __forceinline__ bool working_set_multipliers(const double* A, const double* s, const double* g,
+                                                        unsigned up, unsigned lo, double* lam) {
+  int W[N];
+  double Q[N * N], R[N * N], sg[N];
+  int k;
+  bool ok = working_set_rows<N, M>(up, lo, W, k, lam);
+  if (ok) {
+    for (int a = 0; a < k; ++a)
+      for (int j = 0; j < N; ++j) Q[a * N + j] = s[j] * A[W[a] * N + j];
+    ok = working_set_qr<N>(k, Q, R);
+  }
+  if (!ok) {
+    for (int r = 0; r < M; ++r) lam[r] = NAN;
+    return false;
+  }
+  for (int j = 0; j < N; ++j) sg[j] = s[j] * g[j];
+  working_set_solve<N>(k, W, Q, R, sg, lam);
   return true;
 }
 

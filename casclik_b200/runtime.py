@@ -39,7 +39,7 @@ EXPORTS = (
     "clik_nlp_step", "clik_nlp_step_host", "clik_nlp_solve_one", "clik_nlp_rollout",
     "clik_nlp_step_ld", "clik_nlp_step_host_multi",
     "clik_qp_duals", "clik_nlp_duals", "clik_qp_duals_host", "clik_nlp_duals_host",
-    "clik_qp_solve_one_lam", "clik_nlp_solve_one_lam",
+    "clik_qp_solve_one_lam", "clik_nlp_solve_one_lam", "clik_qp_vjp", "clik_nlp_vjp",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -124,6 +124,9 @@ def load_library():
     for name in ("clik_qp_duals_host", "clik_nlp_duals_host"):
         getattr(lib, name).restype = i32
         getattr(lib, name).argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    for name in ("clik_qp_vjp", "clik_nlp_vjp"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.clik_qp_solve_one_lam.restype = i32
     lib.clik_qp_solve_one_lam.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.clik_nlp_solve_one_lam.restype = i32

@@ -268,6 +268,37 @@ clik_status clik_nlp_duals_host(const clik_skill* skill, int64_t N, const double
                                 const double* q, const double* x, const double* y, const double* sol,
                                 const int32_t* status, const uint32_t* active, double* lam);
 
+/* Reverse-mode derivative (vector-Jacobian product) of a step's output, for N instances.  theta = (t, q, x, y) of
+ * instance i; its step returned x* = sol and the working set W of `active`.  On W the step solves
+ *   r1 = g(x, theta) + A_W(theta)' lam_W = 0   (QP: g = H(theta) x;  NLP: g = grad F(x, theta))
+ *   r2 = A_W(theta) x - b_W(theta)       = 0   (b_r = ub_r for an upper bit, lb_r for a lower bit)
+ * For the cotangent xb = sol_bar[:, i] the adjoint system [[M, A_W'], [A_W, 0]] [u; v] = [xb; 0] (M = H, or
+ * grad^2 F(x*) for the NLP) gives theta_bar = -grad_theta (u'(g + A' lam) + v'(A_W x* - b_W)) with x*, lam, u, v
+ * held fixed: (d(x*)/d(theta))' xb for the face problem of W.  It is the derivative of the step where strict
+ * complementarity holds; where a row of W has lam = 0 it is the one-sided derivative that keeps W.  lam is
+ * computed inside the kernel as clik_qp_duals / clik_nlp_duals compute it.  Adjoint solve: QP v = argmin
+ * |D^1/2 (-xb + A_W' v)| with D = H^-1, u = D (xb - A_W' v); NLP grad^2 F(x*) = L L' (no shift), the same
+ * least-squares solve on the columns L^-1 a_r, u = L^-T L^-1 (xb - A_W' v).
+ *   inputs:  t, q, x, y as clik_qp_step / clik_nlp_step; sol [qp_n * N], status [N], active [2 * N] of the step;
+ *            sol_bar [qp_n * N] the cotangent of sol (all required)
+ *   outputs: t_bar [N] (per instance, also when t_stride = 0: the caller sums it for a shared t),
+ *            q_bar [n_robot * N], x_bar [n_virtual * N], y_bar [n_input * N] (x_bar / y_bar may be NULL when the
+ *            size is 0)
+ * Rules: an instance whose cotangent column is all zeros gets exactly 0, whatever its status; otherwise every
+ * output of the instance is NaN when status[i] is not 0, when A_W is rank-deficient (the tests of clik_qp_duals)
+ * or, for the NLP, when grad^2 F(x*) is not positive definite (the Cholesky factorisation fails).
+ * The kernel is in images built with emit_skill(..., vjp=True) (manifest o[19]) only, and only for skills with
+ * 1..32 constraint rows: other images, and a NULL skill, fail with CLIK_ERR_INVALID.  Device pointers only, row
+ * stride N, asynchronous on `stream`; one thread per instance. */
+clik_status clik_qp_vjp(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                        const double* q, const double* x, const double* y, const double* sol,
+                        const int32_t* status, const uint32_t* active, const double* sol_bar, double* t_bar,
+                        double* q_bar, double* x_bar, double* y_bar, void* stream);
+clik_status clik_nlp_vjp(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                         const double* q, const double* x, const double* y, const double* sol,
+                         const int32_t* status, const uint32_t* active, const double* sol_bar, double* t_bar,
+                         double* q_bar, double* x_bar, double* y_bar, void* stream);
+
 /* One host batch over several GPUs of the box: `skills[k]` is the same cubin loaded on device k
  * (clik_skill_load with desc.device = k); the batch is cut into n_skills contiguous shards (sizes differ
  * by at most one, shard k = [k*N/n .. )), each shard runs on its device from its own host thread (zero
