@@ -14,6 +14,77 @@ class BaseController(object):
     def __repr__(self):
         return "%s<%s>" % (self.controller_type, self.skill_spec.label)
 
+    def _skill(self, device=None):
+        """The cubin loaded on `device` (default: runtime.current_device()); one handle per device, created on first
+        use with the controller's overlap and staging switches, so a batch always runs on the device its tensors
+        live on."""
+        if getattr(self, "_cubin", None) is None:
+            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
+        dev = runtime.current_device() if device is None else int(device)
+        if dev not in self._compiled:
+            skill = runtime.CompiledSkill(self._cubin, self.kernel_meta, n_slack=self.skill_spec.n_slack_var,
+                                          device=dev)
+            if getattr(self, "_overlap", None) is not None:
+                skill.set_overlap(self._overlap)
+            if getattr(self, "_staging", None):
+                skill.set_staging(True)
+            self._compiled[dev] = skill
+        return self._compiled[dev]
+
+
+def set_overlap(ctrl, level):
+    """How successive solve_batch launches on one CUDA stream may overlap (include/clik.h,
+    clik_skill_set_overlap): 0 plain stream order, 1 (default) the two launches of one step overlap,
+    2 successive steps overlap as well — only for streams of independent batches (step k+1 must not
+    read what step k writes; closed loops belong in rollout_batch).
+
+    The set_overlap method of the controllers whose step has two launches (pinv and QP)."""
+    level = int(level)
+    if level not in (0, 1, 2):
+        raise ValueError("overlap level must be 0, 1 or 2")
+    ctrl._overlap = level
+    for skill in ctrl._compiled.values():
+        skill.set_overlap(level)
+
+
+def run_step(skill, kind, b, devices, *args):
+    """Shared dispatch of a controller step (`kind` "pinv", "qp" or "nlp") for the Batch `b`, `skill(device)` the
+    controller's handle on a device: CUDA tensors run clik_<kind>_step on their own device and the current stream;
+    host arrays run clik_<kind>_step_host_multi with one handle per device of `devices` (resolve_devices; None:
+    the default device).  `args`: the kind's arguments after (t, t_stride, q, x, y)."""
+    devs = resolve_devices(devices)
+    lib = runtime.load_library()
+    if b.on_device:
+        if devs is not None:
+            raise ValueError("devices= applies to host arrays; CUDA tensors run on the device they live on")
+        runtime.check(getattr(lib, "clik_%s_step" % kind)(skill(b.device_index).handle, b.N, b.tp, b.t_stride,
+                                                          b.qp, b.xp, b.yp, *args, b.stream()))
+        return
+    skills = [skill(d) for d in (devs or [b.device_index])]
+    runtime.check(getattr(lib, "clik_%s_step_host_multi" % kind)(skill_handle_array(skills), len(skills), b.N, b.tp,
+                                                                  b.t_stride, b.qp, b.xp, b.yp, *args))
+
+
+def one_instance(ctrl, robot_var, virtual_var, input_var):
+    """Validated (q, x, y) of a single-instance solve() as contiguous float64 vectors; x and y are None when the
+    skill has no such rows, and x defaults to zeros when the skill's expressions do not depend on it."""
+    if getattr(ctrl, "_cubin", None) is None:
+        raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
+    spec, n_virtual, n_input = ctrl.skill_spec, ctrl.kernel_meta["n_virtual"], ctrl.kernel_meta["n_input"]
+    q = np.ascontiguousarray(as_vector(robot_var, spec.n_robot_var, "robot_var"))
+    x = None
+    if n_virtual:
+        if spec._has_virtual and virtual_var is None:
+            raise ValueError("the skill depends on virtual_var: a value is required")
+        x = np.ascontiguousarray(as_vector(virtual_var, n_virtual, "virtual_var") if virtual_var is not None
+                                 else np.zeros(n_virtual))
+    y = None
+    if n_input:
+        if input_var is None:
+            raise ValueError("the skill depends on input_var: a value is required")
+        y = np.ascontiguousarray(as_vector(input_var, n_input, "input_var"))
+    return q, x, y
+
 
 def resolve_devices(devices):
     """`devices` argument of solve_batch -> list of CUDA ordinals, or None for "the default device".

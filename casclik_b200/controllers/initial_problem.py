@@ -118,7 +118,7 @@ class InitialProblem(object):
         dq0 (n_robot, N) | None (zeros), y0 (n_input, N): torch CUDA tensors (or NumPy arrays -> host path).
         Returns (virtual_vel (n_virtual, N) | None, slack (n_slack, N) | None, status (N,) int32)."""
         from .. import runtime
-        from .base_controller import Batch
+        from .base_controller import Batch, run_step
         b = self._batch or self._batch_setup()
         prog = b["prog"]
         on_dev = runtime._is_torch(q0)
@@ -133,20 +133,15 @@ class InitialProblem(object):
             dq = np.zeros_like(q0) if dq0 is None else np.ascontiguousarray(dq0, dtype=np.float64)
             y = dq if prog.n_y_user == 0 else np.ascontiguousarray(np.vstack([np.asarray(y0, dtype=np.float64), dq]))
         batch = Batch(prog.n_rob, prog.n_virt, prog.n_in, t0, q0, x0, y)
-        dev = batch.device_index
-        if dev not in b["skills"]:
-            b["skills"][dev] = runtime.CompiledSkill(b["cubin"], b["meta"], n_slack=self.nslack, device=dev)
-        skill = b["skills"][dev]
+
+        def skill(dev):
+            if dev not in b["skills"]:
+                b["skills"][dev] = runtime.CompiledSkill(b["cubin"], b["meta"], n_slack=self.nslack, device=dev)
+            return b["skills"][dev]
+
         sol, status, active = batch.empty(prog.nx), batch.empty(0, "i32"), batch.empty(2, "i32")
-        lib = runtime.load_library()
-        if on_dev:
-            runtime.check(lib.clik_qp_step(skill.handle, batch.N, batch.tp, batch.t_stride, batch.qp, batch.xp,
-                                           batch.yp, None, None, batch.ptr(sol), batch.ptr(status),
-                                           batch.ptr(active), int(max_iter), batch.stream()))
-        else:
-            runtime.check(lib.clik_qp_step_host(skill.handle, batch.N, batch.tp, batch.t_stride, batch.qp, batch.xp,
-                                                batch.yp, None, None, batch.ptr(sol), batch.ptr(status),
-                                                batch.ptr(active), int(max_iter)))
+        run_step(skill, "qp", batch, None, None, None, batch.ptr(sol), batch.ptr(status), batch.ptr(active),
+                 int(max_iter))
         virt = sol[:self.nvirt] if self.nvirt > 0 else None
         slack = sol[self.nvirt:self.nvirt + self.nslack] if self.nslack > 0 else None
         return virt, slack, status

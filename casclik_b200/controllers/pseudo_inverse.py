@@ -21,8 +21,7 @@ from .. import sym as cs
 from ..codegen import PinvProgram, emit_skill
 from ..constraints import SetConstraint
 from ._modes import activation_map
-from .base_controller import (BaseController, Batch, as_vector, dm_column, resolve_devices,
-                              skill_handle_array)
+from .base_controller import BaseController, Batch, dm_column, one_instance, run_step, set_overlap
 
 
 class PseudoInverseController(BaseController):
@@ -40,7 +39,7 @@ class PseudoInverseController(BaseController):
 
     def __init__(self, skill_spec, options=None):
         self.current_mode = None
-        self._compiled = None
+        self._compiled = {}
         self.skill_spec = skill_spec
         self.options = options
 
@@ -84,7 +83,7 @@ class PseudoInverseController(BaseController):
         self.cntrl_var = cntrl
         self.n_state_var = n_state
         self._skill_spec = spec
-        self._compiled = None
+        self._compiled = {}
         self.create_activation_map()
 
     def create_activation_map(self):
@@ -144,7 +143,7 @@ class PseudoInverseController(BaseController):
         self.kernel_source, self.kernel_meta, self.cubin_path = source, meta, path
         self._nx, self._ny = prog.n_virt, prog.n_in
         self._cubin = cubin
-        self._compiled = None
+        self._compiled = {}
         if load:
             self._skill()
 
@@ -163,24 +162,6 @@ class PseudoInverseController(BaseController):
     def setup_solver(self):
         self.setup_problem_functions()
 
-    def _skill(self, device=None):
-        """The cubin loaded on `device` (default: runtime.current_device()); one handle per device,
-        created on first use, so a batch always runs on the device its tensors live on."""
-        if getattr(self, "_cubin", None) is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
-        if not isinstance(self._compiled, dict):
-            first = self._compiled
-            self._compiled = {} if first is None else {first.device: first}
-        dev = runtime.current_device() if device is None else int(device)
-        if dev not in self._compiled:
-            self._compiled[dev] = runtime.CompiledSkill(self._cubin, self.kernel_meta,
-                                                        n_slack=self.skill_spec.n_slack_var, device=dev)
-            if getattr(self, "_overlap", None) is not None:
-                self._compiled[dev].set_overlap(self._overlap)
-            if getattr(self, "_staging", None):
-                self._compiled[dev].set_staging(True)
-        return self._compiled[dev]
-
     def set_input_staging(self, on):
         """Device-resident batches through the TMA-staged persistent kernel (inputs brought into shared memory
         by bulk async copies two tiles ahead of the arithmetic; include/clik.h clik_skill_set_staging).  Same
@@ -190,26 +171,10 @@ class PseudoInverseController(BaseController):
         if on and not self.kernel_meta.get("pinv_staged_kernel"):
             raise runtime.ClikError("this skill has no staged kernel (two-launch step or too many rows)")
         self._staging = bool(on)
-        if isinstance(self._compiled, dict):
-            for sk in self._compiled.values():
-                sk.set_staging(self._staging)
-        elif self._compiled is not None:
-            self._compiled.set_staging(self._staging)
+        for sk in self._compiled.values():
+            sk.set_staging(self._staging)
 
-    def set_overlap(self, level):
-        """How successive solve_batch launches on one CUDA stream may overlap (include/clik.h,
-        clik_skill_set_overlap): 0 plain stream order, 1 (default) the two launches of one step overlap,
-        2 successive steps overlap as well — only for streams of independent batches (step k+1 must not
-        read what step k writes; closed loops belong in rollout_batch)."""
-        level = int(level)
-        if level not in (0, 1, 2):
-            raise ValueError("overlap level must be 0, 1 or 2")
-        self._overlap = level
-        if isinstance(self._compiled, dict):
-            for sk in self._compiled.values():
-                sk.set_overlap(level)
-        elif self._compiled is not None:
-            self._compiled.set_overlap(level)
+    set_overlap = set_overlap
 
     # ---- step --------------------------------------------------------------------------------------
     def solve_batch(self, time_var, robot_var, virtual_var=None, input_var=None, out=None, devices=None):
@@ -229,10 +194,6 @@ class PseudoInverseController(BaseController):
         spec = self.skill_spec
         nq, nx, ny = spec.n_robot_var, self._nx, self._ny
         b = Batch(nq, nx, ny, time_var, robot_var, virtual_var, input_var if ny else None)
-        devs = resolve_devices(devices)
-        if devs is not None and b.on_device:
-            raise ValueError("devices= applies to host arrays; CUDA tensors run on the device they live on")
-        skill = self._skill(b.device_index if devs is None else devs[0])
         if out is None:
             qdot = b.empty(nq)
             xdot = b.empty(nx) if nx else None
@@ -244,17 +205,7 @@ class PseudoInverseController(BaseController):
         qdp, xdp = b.out_ptr(qdot, nq, "f64", "out[0] (robot_vel)"), \
             (b.out_ptr(xdot, nx, "f64", "out[1] (virtual_vel)") if nx else None)
         mdp = b.out_ptr(mode, 0, "i32", "out[2] (mode)")
-        lib = runtime.load_library()
-        if b.on_device:
-            runtime.check(lib.clik_pinv_step(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp,
-                                             qdp, xdp, mdp, b.stream()))
-        elif devs is not None and len(devs) > 1:
-            skills = [self._skill(d) for d in devs]
-            runtime.check(lib.clik_pinv_step_host_multi(skill_handle_array(skills), len(skills), b.N, b.tp,
-                                                        b.t_stride, b.qp, b.xp, b.yp, qdp, xdp, mdp))
-        else:
-            runtime.check(lib.clik_pinv_step_host(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp,
-                                                  b.yp, qdp, xdp, mdp))
+        run_step(self._skill, "pinv", b, devices, qdp, xdp, mdp)
         return qdot, xdot, mode
 
     def rollout_batch(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
@@ -288,22 +239,9 @@ class PseudoInverseController(BaseController):
               warmstart_slack_var=None):
         """One controller step -> (cntrl_rob, cntrl_virt | None, None); sets `current_mode`."""
         spec = self.skill_spec
-        if getattr(self, "_cubin", None) is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
+        q, x, y = one_instance(self, robot_var, virtual_var, input_var)
         nq = spec.n_robot_var
-        q = np.ascontiguousarray(as_vector(robot_var, nq, "robot_var"))
         use_virt = virtual_var is not None and spec._has_virtual
-        x = None
-        if self._nx:
-            if spec._has_virtual and virtual_var is None:
-                raise ValueError("the skill depends on virtual_var: a value is required")
-            x = np.ascontiguousarray(as_vector(virtual_var, self._nx, "virtual_var") if virtual_var is not None
-                                     else np.zeros(self._nx))
-        y = None
-        if self._ny:
-            if input_var is None:
-                raise ValueError("the skill depends on input_var: a value is required")
-            y = np.ascontiguousarray(as_vector(input_var, self._ny, "input_var"))
         # one instance: straight to the single-instance ABI entry (a page-locked mapped slot inside the
         # library; no batch plumbing, no allocation) — the call a notebook makes in its control loop
         one = getattr(self, "_one", None)

@@ -21,8 +21,8 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
-from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
-                              skill_handle_array, solve_batch_differentiable, vjp_batch)
+from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
+                              solve_batch_differentiable, vjp_batch)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -54,7 +54,7 @@ class ReactiveNLPController(BaseController):
         self.slack_var_weights = slack_var_weights
         self.options = options
         self._cubin = None
-        self._compiled = None
+        self._compiled = {}
         self._vjp = None
         self._has_initial = False
         self.res = None
@@ -128,7 +128,7 @@ class ReactiveNLPController(BaseController):
         self._nxv, self._ny, self._qn, self._qm = prog.n_virt, prog.n_in, prog.nx, prog.m
         self.row_labels = prog.labels
         self._cubin = cubin
-        self._compiled = None
+        self._compiled = {}
         self._vjp = None
         if load:
             self._skill()
@@ -137,17 +137,6 @@ class ReactiveNLPController(BaseController):
         """Compiles and loads the kernels if setup_problem_functions has not (either order works)."""
         if self._cubin is None:
             self.setup_problem_functions()
-
-    def _skill(self, device=None):
-        if self._cubin is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
-        if self._compiled is None:
-            self._compiled = {}
-        dev = runtime.current_device() if device is None else int(device)
-        if dev not in self._compiled:
-            self._compiled[dev] = runtime.CompiledSkill(self._cubin, self.kernel_meta,
-                                                        n_slack=self.skill_spec.n_slack_var, device=dev)
-        return self._compiled[dev]
 
     def _max_iter(self, max_iter):
         return int(max_iter if max_iter is not None else self.options["max_iter"])
@@ -181,10 +170,6 @@ class ReactiveNLPController(BaseController):
         spec = self.skill_spec
         b = Batch(spec.n_robot_var, self._nxv, self._ny, time_var, robot_var, virtual_var,
                   input_var if self._ny else None)
-        devs = resolve_devices(devices)
-        if devs is not None and b.on_device:
-            raise ValueError("devices= applies to host arrays; CUDA tensors run on the device they live on")
-        skill = self._skill(b.device_index if devs is None else devs[0])
         if out is None:
             sol, status, active, iters = b.empty(self._qn), b.empty(0, "i32"), b.empty(2, "i32"), b.empty(0, "i32")
         else:
@@ -201,18 +186,7 @@ class ReactiveNLPController(BaseController):
                 x0p = runtime.dev_ptr(warmstart, "f64", self._qn * b.N, "warmstart")
             else:
                 x0p, warmstart = runtime.host_ptr(warmstart, np.float64, self._qn * b.N, "warmstart")
-        mi = self._max_iter(max_iter)
-        lib = runtime.load_library()
-        if b.on_device:
-            runtime.check(lib.clik_nlp_step(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, x0p,
-                                            solp, stp, itp, acp, mi, b.stream()))
-        elif devs is not None and len(devs) > 1:
-            skills = [self._skill(d) for d in devs]
-            runtime.check(lib.clik_nlp_step_host_multi(skill_handle_array(skills), len(skills), b.N, b.tp,
-                                                       b.t_stride, b.qp, b.xp, b.yp, x0p, solp, stp, itp, acp, mi))
-        else:
-            runtime.check(lib.clik_nlp_step_host(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, x0p,
-                                                 solp, stp, itp, acp, mi))
+        run_step(self._skill, "nlp", b, devices, x0p, solp, stp, itp, acp, self._max_iter(max_iter))
         return sol, status, active, iters
 
     def multipliers_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
@@ -267,22 +241,9 @@ class ReactiveNLPController(BaseController):
         raise.  lam_g (m x 1): the constraint multipliers (multipliers_batch; NaN when not solved, None for skills
         with more than 32 rows); lam_x (n x 1): zeros (no simple bounds)."""
         spec = self.skill_spec
-        if self._cubin is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
+        q, x, y = one_instance(self, robot_var, virtual_var, input_var)
         nrob, nvirt, nslack = spec.n_robot_var, spec.n_virtual_var, spec.n_slack_var
         has_virtual = spec._has_virtual
-        q = np.ascontiguousarray(as_vector(robot_var, nrob, "robot_var"))
-        x = None
-        if self._nxv:
-            if has_virtual and virtual_var is None:
-                raise ValueError("the skill depends on virtual_var: a value is required")
-            x = np.ascontiguousarray(as_vector(virtual_var, self._nxv, "virtual_var") if virtual_var is not None
-                                     else np.zeros(self._nxv))
-        y = None
-        if self._ny:
-            if input_var is None:
-                raise ValueError("the skill depends on input_var: a value is required")
-            y = np.ascontiguousarray(as_vector(input_var, self._ny, "input_var"))
         warm = None
         if warmstart_robot_vel_var is not None or warmstart_virtual_vel_var is not None or \
                 warmstart_slack_var is not None:

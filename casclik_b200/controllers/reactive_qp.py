@@ -22,8 +22,8 @@ import numpy as np
 from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
-from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, resolve_devices,
-                              skill_handle_array, solve_batch_differentiable, vjp_batch)
+from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
+                              set_overlap, solve_batch_differentiable, vjp_batch)
 from .qp_solver import ConicSolver
 
 
@@ -67,7 +67,7 @@ class ReactiveQPController(BaseController):
         self.virtual_var_weights = virtual_var_weights
         self.slack_var_weights = slack_var_weights
         self.options = options
-        self._compiled = None
+        self._compiled = {}
         self._cubin = None
         self._vjp = None
         self._has_initial = False
@@ -200,7 +200,7 @@ class ReactiveQPController(BaseController):
         # evaluate H_func through the expression interpreter at every call
         self._h_const = (np.array([n.val for n in prog.h]) if all(n.is_const for n in prog.h) else None)
         self._cubin = cubin
-        self._compiled = None
+        self._compiled = {}
         self._vjp = None
         ins, names = self._input_list()
         H = cs.diag(cs.MX(cs.vertcat(*prog.h)))
@@ -220,35 +220,7 @@ class ReactiveQPController(BaseController):
         if self._cubin is None:
             self.setup_problem_functions()
 
-    def _skill(self, device=None):
-        """The cubin loaded on `device` (default: runtime.current_device()); one handle per device."""
-        if self._cubin is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
-        if not isinstance(self._compiled, dict):
-            first = self._compiled
-            self._compiled = {} if first is None else {first.device: first}
-        dev = runtime.current_device() if device is None else int(device)
-        if dev not in self._compiled:
-            self._compiled[dev] = runtime.CompiledSkill(self._cubin, self.kernel_meta,
-                                                        n_slack=self.skill_spec.n_slack_var, device=dev)
-            if getattr(self, "_overlap", None) is not None:
-                self._compiled[dev].set_overlap(self._overlap)
-        return self._compiled[dev]
-
-    def set_overlap(self, level):
-        """How successive solve_batch launches on one CUDA stream may overlap (include/clik.h,
-        clik_skill_set_overlap): 0 plain stream order, 1 (default) the two launches of one step overlap,
-        2 successive steps overlap as well — only for streams of independent batches (step k+1 must not
-        read what step k writes; closed loops belong in rollout_batch)."""
-        level = int(level)
-        if level not in (0, 1, 2):
-            raise ValueError("overlap level must be 0, 1 or 2")
-        self._overlap = level
-        if isinstance(self._compiled, dict):
-            for sk in self._compiled.values():
-                sk.set_overlap(level)
-        elif self._compiled is not None:
-            self._compiled.set_overlap(level)
+    set_overlap = set_overlap
 
     # ---- initial problem (virtual + slack with robot velocity fixed), reference :300-459 ---------------
     def setup_initial_problem_solver(self):
@@ -290,10 +262,6 @@ class ReactiveQPController(BaseController):
         spec = self.skill_spec
         b = Batch(spec.n_robot_var, self._nxv, self._ny, time_var, robot_var, virtual_var,
                   input_var if self._ny else None)
-        devs = resolve_devices(devices)
-        if devs is not None and b.on_device:
-            raise ValueError("devices= applies to host arrays; CUDA tensors run on the device they live on")
-        skill = self._skill(b.device_index if devs is None else devs[0])
         if out is None:
             sol = b.empty(self._qn)
             status = b.empty(0, "i32")
@@ -318,17 +286,7 @@ class ReactiveQPController(BaseController):
             else:
                 a0p, warm_active = runtime.host_ptr(warm_active, np.int32, 2 * b.N, "warm_active")
         mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
-        lib = runtime.load_library()
-        if b.on_device:
-            runtime.check(lib.clik_qp_step(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp,
-                                           x0p, a0p, solp, stp, acp, mi, b.stream()))
-        elif devs is not None and len(devs) > 1:
-            skills = [self._skill(d) for d in devs]
-            runtime.check(lib.clik_qp_step_host_multi(skill_handle_array(skills), len(skills), b.N, b.tp,
-                                                      b.t_stride, b.qp, b.xp, b.yp, x0p, a0p, solp, stp, acp, mi))
-        else:
-            runtime.check(lib.clik_qp_step_host(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp,
-                                                b.yp, x0p, a0p, solp, stp, acp, mi))
+        run_step(self._skill, "qp", b, devices, x0p, a0p, solp, stp, acp, mi)
         return sol, status, active
 
     def multipliers_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
@@ -395,22 +353,10 @@ class ReactiveQPController(BaseController):
         "active_upper", "active_lower", "cost", "lam_a", "lam_x"}: lam_a (m x 1) are the constraint multipliers
         (multipliers_batch; None for skills with more than 32 rows), lam_x (n x 1) zeros (no simple bounds)."""
         spec = self.skill_spec
-        if self._cubin is None:
-            raise RuntimeError("call setup_problem_functions() / setup_solver() before solve()")
+        q, x, y = (None if a is None else a.reshape(-1, 1)
+                   for a in one_instance(self, robot_var, virtual_var, input_var))
         nrob, nvirt, nslack = spec.n_robot_var, spec.n_virtual_var, spec.n_slack_var
         has_virtual = spec._has_virtual
-        q = np.ascontiguousarray(as_vector(robot_var, nrob, "robot_var")).reshape(nrob, 1)
-        x = None
-        if self._nxv:
-            if has_virtual and virtual_var is None:
-                raise ValueError("the skill depends on virtual_var: a value is required")
-            x = np.ascontiguousarray(as_vector(virtual_var, self._nxv, "virtual_var") if virtual_var is not None
-                                     else np.zeros(self._nxv)).reshape(self._nxv, 1)
-        y = None
-        if self._ny:
-            if input_var is None:
-                raise ValueError("the skill depends on input_var: a value is required")
-            y = np.ascontiguousarray(as_vector(input_var, self._ny, "input_var")).reshape(self._ny, 1)
         ws_rob = warmstart_robot_vel_var is not None
         ws_virt = warmstart_virtual_vel_var is not None and has_virtual
         ws_slack = warmstart_slack_var is not None and nslack > 0

@@ -10,6 +10,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -246,15 +247,22 @@ std::mutex g_flush_mu;
 double* g_flush_buf[64] = {nullptr};
 constexpr size_t FLUSH_BYTES = (size_t)256 << 20;  // 256 MiB > 126 MB L2
 
-// ---- host-buffer pipeline ----------------------------------------------------------------------------
-struct Field {
-  const void* src;   // host source (input) or nullptr
-  void* dst;         // host destination (output) or nullptr
-  int rows;          // SoA rows
-  int elem;          // bytes per element
-  int stride;        // 1 = per instance, 0 = broadcast scalar row (only for t)
-  size_t dev_off;    // byte offset inside the slot buffer
+// ---- host-buffer calls ---------------------------------------------------------------------------------
+// One array of a host call: the caller's pointer and how it reaches the device.
+enum Dir { IN, OUT };
+struct HostField {
+  const void* host;                // caller's array (rows N apart); nullptr or rows == 0: absent
+  Dir dir;                         // IN: read by the kernel; OUT: written by it
+  int rows;                        // SoA rows
+  int elem;                        // bytes per element
+  bool broadcast = false;          // one value for every instance (t with t_stride 0)
   unsigned rowmask = 0xffffffffu;  // input rows the kernel reads (unread rows are not copied)
+};
+
+// A device pointer that converts to whatever pointer type the *_impl parameter it is passed to has.
+struct DevPtr {
+  void* p = nullptr;
+  template <class T> operator T*() const { return static_cast<T*>(p); }
 };
 
 clik_status ensure_scratch(clik_skill* s, int slot, size_t bytes) {
@@ -336,17 +344,40 @@ clik_status for_row_runs(int rows, unsigned mask, Copy copy) {
   return CLIK_OK;
 }
 
-// Instances [lo, lo + cnt) of a host batch whose rows are N apart (lo = 0, cnt = N: the whole batch).
-template <class Launch>
-clik_status run_host_pipeline(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, std::vector<Field>& f,
-                              Launch launch) {
+// Instances [lo, lo + cnt) of a host batch whose rows are N apart (lo = 0, cnt = N: the whole batch), one
+// HostField per array.  If every present array is page-locked memory mapped into the device, one launch runs on it
+// directly (zero copy); otherwise the instances go through the chunked copy pipeline on the skill's scratch slots.
+// `launch(p, n, ld, stream, zero_copy)` launches the step on n instances whose rows are ld apart, p[k] the device
+// pointer of field k (nullptr exactly when the field is absent).  Returns once the results are in the host arrays.
+template <size_t NF, class Launch>
+clik_status run_host_batch(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, const std::array<HostField, NF>& f,
+                           Launch launch) {
+  if (cnt <= 0) return CLIK_OK;
   std::lock_guard<std::mutex> lock(s->mu);
   ON_DEVICE(s->desc.device);
+  std::array<DevPtr, NF> p;
+  auto present = [&](size_t k) { return f[k].host != nullptr && f[k].rows > 0; };
+  bool zero_copy = zero_copy_enabled();
+  for (size_t k = 0; k < NF && zero_copy; ++k) {
+    const void* dev = nullptr;
+    zero_copy = device_alias(present(k) ? f[k].host : nullptr, &dev);
+    if (dev && !f[k].broadcast) dev = (const char*)dev + lo * f[k].elem;
+    p[k].p = const_cast<void*>(dev);
+  }
+  if (zero_copy) {
+    clik_status st = ensure_scratch(s, 0, 256);
+    if (st != CLIK_OK) return st;
+    GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
+    st = launch(p, cnt, N, s->scratch.stream[0], true);
+    if (st != CLIK_OK) return st;
+    CK(cudaStreamSynchronize(s->scratch.stream[0]));
+    return CLIK_OK;
+  }
   const int64_t chunk = std::min<int64_t>(cnt, host_chunk());
-  size_t bytes = 0;
-  for (auto& fl : f) {
-    fl.dev_off = bytes;
-    bytes += (((size_t)fl.rows * chunk * fl.elem) + 255) & ~(size_t)255;
+  size_t off[NF], bytes = 0;
+  for (size_t k = 0; k < NF; ++k) {
+    off[k] = bytes;
+    bytes += (((size_t)f[k].rows * chunk * f[k].elem) + 255) & ~(size_t)255;
   }
   const int nslots = (int)std::min<int64_t>(NSLOTS, (cnt + chunk - 1) / chunk);
   for (int slot = 0; slot < nslots; ++slot) {
@@ -358,27 +389,29 @@ clik_status run_host_pipeline(clik_skill* s, int64_t N, int64_t lo, int64_t cnt,
     const int64_t c = std::min<int64_t>(chunk, lo + cnt - i0);
     cudaStream_t st = s->scratch.stream[slot];
     char* base = (char*)s->scratch.dev[slot];
-    for (auto& fl : f) {
-      if (!fl.src) continue;
-      if (fl.stride == 0) {
-        if (fl.rowmask & 1u) CK(cudaMemcpyAsync(base + fl.dev_off, fl.src, fl.elem, cudaMemcpyHostToDevice, st));
+    for (size_t k = 0; k < NF; ++k) {
+      const HostField& fl = f[k];
+      p[k].p = present(k) ? base + off[k] : nullptr;
+      if (!present(k) || fl.dir != IN) continue;
+      if (fl.broadcast) {
+        if (fl.rowmask & 1u) CK(cudaMemcpyAsync(p[k].p, fl.host, fl.elem, cudaMemcpyHostToDevice, st));
         continue;
       }
       clik_status cs = for_row_runs(fl.rows, fl.rowmask, [&](int r0, int nr) -> clik_status {
-        CK(cudaMemcpy2DAsync(base + fl.dev_off + (size_t)r0 * c * fl.elem, (size_t)c * fl.elem,
-                             (const char*)fl.src + ((size_t)r0 * N + (size_t)i0) * fl.elem,
+        CK(cudaMemcpy2DAsync(base + off[k] + (size_t)r0 * c * fl.elem, (size_t)c * fl.elem,
+                             (const char*)fl.host + ((size_t)r0 * N + (size_t)i0) * fl.elem,
                              (size_t)N * fl.elem, (size_t)c * fl.elem, nr, cudaMemcpyHostToDevice, st));
         return CLIK_OK;
       });
       if (cs != CLIK_OK) return cs;
     }
-    clik_status ls = launch(base, c, st);
+    clik_status ls = launch(p, c, c, st, false);
     if (ls != CLIK_OK) return ls;
-    for (auto& fl : f) {
-      if (!fl.dst) continue;
-      CK(cudaMemcpy2DAsync((char*)fl.dst + (size_t)i0 * fl.elem, (size_t)N * fl.elem,
-                           base + fl.dev_off, (size_t)c * fl.elem, (size_t)c * fl.elem, fl.rows,
-                           cudaMemcpyDeviceToHost, st));
+    for (size_t k = 0; k < NF; ++k) {
+      const HostField& fl = f[k];
+      if (!present(k) || fl.dir != OUT) continue;
+      CK(cudaMemcpy2DAsync((char*)fl.host + (size_t)i0 * fl.elem, (size_t)N * fl.elem, base + off[k],
+                           (size_t)c * fl.elem, (size_t)c * fl.elem, fl.rows, cudaMemcpyDeviceToHost, st));
     }
   }
   for (int k = 0; k < nslots; ++k) CK(cudaStreamSynchronize(s->scratch.stream[k]));
@@ -735,113 +768,6 @@ clik_status clik_qp_dense(int32_t device, int64_t N, int32_t nx, int32_t m, cons
 
 namespace {
 
-// ---- host-buffer entry points: instances [lo, lo + cnt) of a host batch of N ------------------------
-clik_status pinv_host_range(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, const double* t,
-                            int32_t t_stride, const double* q, const double* x, const double* y,
-                            double* qdot, double* xdot, int32_t* mode) {
-  const clik_skill_desc& d = s->desc;
-  if (cnt <= 0) return CLIK_OK;
-  if (zero_copy_enabled()) {
-    const void *dt, *dq, *dx, *dy, *dqd, *dxd, *dm;
-    ON_DEVICE(d.device);
-    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
-        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(qdot, &dqd) &&
-        device_alias(d.n_virtual ? xdot : nullptr, &dxd) && device_alias(mode, &dm)) {
-      std::lock_guard<std::mutex> lock(s->mu);
-      clik_status zs = ensure_scratch(s, 0, 256);
-      if (zs != CLIK_OK) return zs;
-      auto off = [lo](const void* p) { return p ? (const double*)p + lo : nullptr; };
-      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
-      zs = pinv_step_impl(s, cnt, N, t_stride ? off(dt) : (const double*)dt, t_stride, off(dq), off(dx),
-                          off(dy), (double*)off(dqd), (double*)off(dxd),
-                          dm ? (int32_t*)dm + lo : nullptr, s->scratch.stream[0], std::min(s->overlap, 1),
-                          /*staged_ok=*/zero_copy_staged(),    // the inputs are mapped host memory:
-                          /*split_ok=*/false);                 // no hand-over through mode[] over PCIe either
-      if (zs != CLIK_OK) return zs;
-      CK(cudaStreamSynchronize(s->scratch.stream[0]));
-      return CLIK_OK;
-    }
-  }
-  std::vector<Field> f;
-  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
-  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
-  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
-  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
-  f[0].rowmask = s->pinv_reads.t;
-  f[1].rowmask = s->pinv_reads.q;
-  f[2].rowmask = s->pinv_reads.x;
-  f[3].rowmask = s->pinv_reads.y;
-  f.push_back({nullptr, qdot, d.n_robot, 8, 1, 0});
-  f.push_back({nullptr, d.n_virtual ? xdot : nullptr, d.n_virtual, 8, 1, 0});
-  f.push_back({nullptr, mode, 1, 4, 1, 0});
-  return run_host_pipeline(s, N, lo, cnt, f, [&](char* base, int64_t c, cudaStream_t stream) {
-    return pinv_step_impl(s, c, c, (const double*)(base + f[0].dev_off), t_stride,
-                          (const double*)(base + f[1].dev_off),
-                          d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
-                          d.n_input ? (const double*)(base + f[3].dev_off) : nullptr,
-                          (double*)(base + f[4].dev_off),
-                          d.n_virtual ? (double*)(base + f[5].dev_off) : nullptr,
-                          mode ? (int32_t*)(base + f[6].dev_off) : nullptr, stream, std::min(s->overlap, 1));
-  });
-}
-
-clik_status qp_host_range(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, const double* t, int32_t t_stride,
-                          const double* q, const double* x, const double* y, const double* x0,
-                          const uint32_t* active0, double* sol, int32_t* status, uint32_t* active,
-                          int32_t max_iter) {
-  const clik_skill_desc& d = s->desc;
-  if (cnt <= 0) return CLIK_OK;
-  if (zero_copy_enabled()) {
-    const void *dt, *dq, *dx, *dy, *dx0, *da0, *dsol, *dst, *dact;
-    ON_DEVICE(d.device);
-    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
-        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(x0, &dx0) && device_alias(active0, &da0) &&
-        device_alias(sol, &dsol) && device_alias(status, &dst) && device_alias(active, &dact)) {
-      std::lock_guard<std::mutex> lock(s->mu);
-      clik_status zs = ensure_scratch(s, 0, 256);
-      if (zs != CLIK_OK) return zs;
-      auto off = [lo](const void* p) { return p ? (const double*)p + lo : nullptr; };
-      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
-      zs = qp_step_impl(s, cnt, N, t_stride ? off(dt) : (const double*)dt, t_stride, off(dq), off(dx), off(dy),
-                        off(dx0), da0 ? (const uint32_t*)da0 + lo : nullptr, (double*)off(dsol),
-                        dst ? (int32_t*)dst + lo : nullptr, dact ? (uint32_t*)dact + lo : nullptr, max_iter,
-                        s->scratch.stream[0], std::min(s->overlap, 1),
-                        // one kernel: a tail pass would scan status[] and re-read the inputs of the pending
-                        // instances over PCIe (1.7e8 vs 4.4-4.8e8 steps/s for the UR5 problem, profiles/r2_ab19.txt)
-                        /*split_ok=*/false);
-      if (zs != CLIK_OK) return zs;
-      CK(cudaStreamSynchronize(s->scratch.stream[0]));
-      return CLIK_OK;
-    }
-  }
-  std::vector<Field> f;
-  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
-  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
-  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
-  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
-  f[0].rowmask = s->qp_reads.t;
-  f[1].rowmask = s->qp_reads.q;
-  f[2].rowmask = s->qp_reads.x;
-  f[3].rowmask = s->qp_reads.y;
-  f.push_back({x0, nullptr, d.qp_n, 8, 1, 0});
-  f.push_back({nullptr, sol, d.qp_n, 8, 1, 0});
-  f.push_back({nullptr, status, 1, 4, 1, 0});
-  f.push_back({nullptr, active, 2, 4, 1, 0});
-  f.push_back({active0, nullptr, 2, 4, 1, 0});
-  return run_host_pipeline(s, N, lo, cnt, f, [&](char* base, int64_t c, cudaStream_t stream) {
-    return qp_step_impl(s, c, c, (const double*)(base + f[0].dev_off), t_stride,
-                        (const double*)(base + f[1].dev_off),
-                        d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
-                        d.n_input ? (const double*)(base + f[3].dev_off) : nullptr,
-                        x0 ? (const double*)(base + f[4].dev_off) : nullptr,
-                        active0 ? (const uint32_t*)(base + f[8].dev_off) : nullptr,
-                        (double*)(base + f[5].dev_off),
-                        status ? (int32_t*)(base + f[6].dev_off) : nullptr,
-                        active ? (uint32_t*)(base + f[7].dev_off) : nullptr, max_iter, stream,
-                        std::min(s->overlap, 1));
-  });
-}
-
 // Contiguous shards of one host batch, one per skill handle (= per device), each on its own host
 // thread; no exchange between devices (instances are independent), results land in the caller's arrays.
 template <class Run>
@@ -885,7 +811,19 @@ clik_status clik_pinv_step_host_multi(const clik_skill* const* skills, int32_t n
   if (st != CLIK_OK || N == 0) return st;
   if (!qdot) return fail(CLIK_ERR_INVALID, "qdot is required");
   return run_sharded(skills, n_skills, N, [&](clik_skill* s, int64_t lo, int64_t cnt) {
-    return pinv_host_range(s, N, lo, cnt, t, t_stride, q, x, y, qdot, xdot, mode);
+    const clik_skill_desc& d = s->desc;
+    const ReadMask& r = s->pinv_reads;
+    const std::array<HostField, 7> f = {{{t, IN, 1, 8, t_stride == 0, r.t}, {q, IN, d.n_robot, 8, false, r.q},
+                                         {x, IN, d.n_virtual, 8, false, r.x}, {y, IN, d.n_input, 8, false, r.y},
+                                         {qdot, OUT, d.n_robot, 8}, {xdot, OUT, d.n_virtual, 8}, {mode, OUT, 1, 4}}};
+    return run_host_batch(s, N, lo, cnt, f, [&](const std::array<DevPtr, 7>& p, int64_t n, int64_t ld,
+                                                cudaStream_t stream, bool zero_copy) {
+      auto [dt, dq, dx, dy, dqdot, dxdot, dmode] = p;
+      // on mapped host memory: the staged kernel only on request (CLIK_ZC_STAGED), and no hand-over through
+      // mode[] over PCIe
+      return pinv_step_impl(s, n, ld, dt, t_stride, dq, dx, dy, dqdot, dxdot, dmode, stream, std::min(s->overlap, 1),
+                            /*staged_ok=*/!zero_copy || zero_copy_staged(), /*split_ok=*/!zero_copy);
+    });
   });
 }
 
@@ -905,7 +843,20 @@ clik_status clik_qp_step_host_multi(const clik_skill* const* skills, int32_t n_s
   if (st != CLIK_OK || N == 0) return st;
   if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
   return run_sharded(skills, n_skills, N, [&](clik_skill* s, int64_t lo, int64_t cnt) {
-    return qp_host_range(s, N, lo, cnt, t, t_stride, q, x, y, x0, active0, sol, status, active, max_iter);
+    const clik_skill_desc& d = s->desc;
+    const ReadMask& r = s->qp_reads;
+    const std::array<HostField, 9> f = {{{t, IN, 1, 8, t_stride == 0, r.t}, {q, IN, d.n_robot, 8, false, r.q},
+                                         {x, IN, d.n_virtual, 8, false, r.x}, {y, IN, d.n_input, 8, false, r.y},
+                                         {x0, IN, d.qp_n, 8}, {active0, IN, 2, 4}, {sol, OUT, d.qp_n, 8},
+                                         {status, OUT, 1, 4}, {active, OUT, 2, 4}}};
+    return run_host_batch(s, N, lo, cnt, f, [&](const std::array<DevPtr, 9>& p, int64_t n, int64_t ld,
+                                                cudaStream_t stream, bool zero_copy) {
+      auto [dt, dq, dx, dy, dx0, dactive0, dsol, dstatus, dactive] = p;
+      // on mapped host memory one kernel: a tail pass would scan status[] and re-read the inputs of the pending
+      // instances over PCIe (1.7e8 vs 4.4-4.8e8 steps/s for the UR5 problem, profiles/r2_ab19.txt)
+      return qp_step_impl(s, n, ld, dt, t_stride, dq, dx, dy, dx0, dactive0, dsol, dstatus, dactive, max_iter, stream,
+                          std::min(s->overlap, 1), /*split_ok=*/!zero_copy);
+    });
   });
 }
 
@@ -926,6 +877,37 @@ static clik_status one_slot(clik_skill* s, size_t doubles) {
   return CLIK_OK;
 }
 
+// The single-instance slot of `s`, locked (until the OneSlot goes out of scope) and sized for t | q | x | y followed
+// by `own_cells` doubles of the caller's own cells, with the four inputs written.
+struct OneSlot {
+  std::unique_lock<std::mutex> lock;
+  double* host = nullptr;   // the slot: host view ...
+  double* dev = nullptr;    // ... and device view
+  const double *t = nullptr, *q = nullptr, *x = nullptr, *y = nullptr;   // device pointers of the inputs
+  size_t own = 0;           // first cell after the inputs: the caller's own cells start here
+};
+
+static clik_status fill_one_slot(clik_skill* s, size_t own_cells, double t, const double* q, const double* x,
+                                 const double* y, OneSlot* o) {
+  const int nq = s->desc.n_robot, nx = s->desc.n_virtual, ny = s->desc.n_input;
+  o->lock = std::unique_lock<std::mutex>(s->mu);
+  o->own = 1 + nq + nx + ny;
+  clik_status st = one_slot(s, o->own + own_cells);
+  if (st != CLIK_OK) return st;
+  double *h = s->one_host, *dv = s->one_dev;
+  h[0] = t;
+  std::memcpy(h + 1, q, sizeof(double) * nq);
+  if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
+  if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
+  o->host = h;
+  o->dev = dv;
+  o->t = dv;
+  o->q = dv + 1;
+  o->x = nx ? dv + 1 + nq : nullptr;
+  o->y = ny ? dv + 1 + nq + nx : nullptr;
+  return CLIK_OK;
+}
+
 clik_status clik_pinv_solve_one(const clik_skill* cs, double t, const double* q, const double* x, const double* y,
                                 double* qdot, double* xdot, int32_t* mode) {
   clik_skill* s = const_cast<clik_skill*>(cs);
@@ -935,29 +917,22 @@ clik_status clik_pinv_solve_one(const clik_skill* cs, double t, const double* q,
   if (d.n_virtual > 0 && (!x || !xdot)) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x and xdot are required");
   if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
   ON_DEVICE(d.device);
-  std::lock_guard<std::mutex> lock(s->mu);
-  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input;
-  clik_status st = one_slot(s, (size_t)(2 + 2 * nq + 2 * nx + ny + 2));
-  if (st != CLIK_OK) return st;
-  double* h = s->one_host;
+  const int nq = d.n_robot, nx = d.n_virtual;
+  OneSlot o;
   // slot: t | q | x | y | qdot | xdot | mode (as one double-sized cell)
-  h[0] = t;
-  std::memcpy(h + 1, q, sizeof(double) * nq);
-  if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
-  if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
-  const size_t o_in = 1 + nq + nx + ny;
-  double* dv = s->one_dev;
+  clik_status st = fill_one_slot(s, nq + nx + 1, t, q, x, y, &o);
+  if (st != CLIK_OK) return st;
   long long n = 1, l = 1;
   int ts = 0;
-  const double *dt = dv, *dq = dv + 1, *dx = nx ? dv + 1 + nq : nullptr, *dy = ny ? dv + 1 + nq + nx : nullptr;
-  double *dqd = dv + o_in, *dxd = nx ? dv + o_in + nq : nullptr;
-  int* dm = (int*)(dv + o_in + nq + nx);
-  void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dqd, &dxd, &dm};
+  double *dqd = o.dev + o.own, *dxd = nx ? o.dev + o.own + nq : nullptr;
+  int* dm = (int*)(o.dev + o.own + nq + nx);
+  void* args[] = {&n, &l, &o.t, &ts, &o.q, &o.x, &o.y, &dqd, &dxd, &dm};
   CK(cudaLaunchKernel((const void*)s->pinv.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
   CK(cudaStreamSynchronize(s->one_stream));
-  std::memcpy(qdot, h + o_in, sizeof(double) * nq);
-  if (nx) std::memcpy(xdot, h + o_in + nq, sizeof(double) * nx);
-  if (mode) *mode = *(const int*)(h + o_in + nq + nx);
+  const double* h = o.host + o.own;
+  std::memcpy(qdot, h, sizeof(double) * nq);
+  if (nx) std::memcpy(xdot, h + nq, sizeof(double) * nx);
+  if (mode) *mode = *(const int*)(h + nq + nx);
   return CLIK_OK;
 }
 
@@ -978,35 +953,29 @@ clik_status clik_qp_solve_one_lam(const clik_skill* cs, double t, const double* 
   if (d.n_virtual > 0 && !x) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x is required");
   if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
   ON_DEVICE(d.device);
-  std::lock_guard<std::mutex> lock(s->mu);
-  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n, qm = lam ? d.qp_m : 0;
-  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3 + qm));
-  if (st != CLIK_OK) return st;
-  double* h = s->one_host;
+  const int qn = d.qp_n, qm = lam ? d.qp_m : 0;
+  OneSlot o;
   // slot: t | q | x | y | x0 | sol | status, active_up, active_lo (three int cells in two doubles) | lam
-  h[0] = t;
-  std::memcpy(h + 1, q, sizeof(double) * nq);
-  if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
-  if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
-  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
+  clik_status st = fill_one_slot(s, 2 * qn + 2 + qm, t, q, x, y, &o);
+  if (st != CLIK_OK) return st;
+  const size_t o_x0 = o.own, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
+  double *h = o.host, *dv = o.dev;
   if (x0) std::memcpy(h + o_x0, x0, sizeof(double) * qn);
-  double* dv = s->one_dev;
   long long n = 1, l = 1;
   int ts = 0;
   int mi = max_iter > 0 ? max_iter : 10 * (d.qp_n + d.qp_m);
-  const double *dt = dv, *dq = dv + 1, *dx = nx ? dv + 1 + nq : nullptr, *dy = ny ? dv + 1 + nq + nx : nullptr;
   const double* dx0 = x0 ? dv + o_x0 : nullptr;
   const unsigned* da0 = nullptr;
   double* dsol = dv + o_sol;
   int* dst = (int*)(dv + o_int);
   unsigned* dact = (unsigned*)(dv + o_int) + 1;      // active[0], active[ld = 1]
-  void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dx0, &da0, &dsol, &dst, &dact, &mi};
+  void* args[] = {&n, &l, &o.t, &ts, &o.q, &o.x, &o.y, &dx0, &da0, &dsol, &dst, &dact, &mi};
   // one instance: the single full kernel (prediction + iteration in one launch)
   CK(cudaLaunchKernel((const void*)s->qp.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
   if (lam) {
     // the multipliers at the step's output, same stream: one wait for both launches
     double* dlam = dv + o_lam;
-    void* largs[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dsol, &dst, &dact, &dlam};
+    void* largs[] = {&n, &l, &o.t, &ts, &o.q, &o.x, &o.y, &dsol, &dst, &dact, &dlam};
     CK(cudaLaunchKernel((const void*)s->qp_duals.kernel, dim3(1), dim3(32), largs, 0, s->one_stream));
   }
   CK(cudaStreamSynchronize(s->one_stream));
@@ -1042,58 +1011,6 @@ clik_status nlp_step_impl(const clik_skill* s, int64_t N, int64_t ld, const doub
   return CLIK_OK;
 }
 
-// Instances [lo, lo + cnt) of a host batch of N (as qp_host_range).
-clik_status nlp_host_range(clik_skill* s, int64_t N, int64_t lo, int64_t cnt, const double* t, int32_t t_stride,
-                           const double* q, const double* x, const double* y, const double* x0, double* sol,
-                           int32_t* status, int32_t* iters, uint32_t* active, int32_t max_iter) {
-  const clik_skill_desc& d = s->desc;
-  if (cnt <= 0) return CLIK_OK;
-  if (zero_copy_enabled()) {
-    const void *dt, *dq, *dx, *dy, *dx0, *dsol, *dst, *dit, *dact;
-    ON_DEVICE(d.device);
-    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
-        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(x0, &dx0) && device_alias(sol, &dsol) &&
-        device_alias(status, &dst) && device_alias(iters, &dit) && device_alias(active, &dact)) {
-      std::lock_guard<std::mutex> lock(s->mu);
-      clik_status zs = ensure_scratch(s, 0, 256);
-      if (zs != CLIK_OK) return zs;
-      auto off = [lo](const void* p) { return p ? (const double*)p + lo : nullptr; };
-      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
-      zs = nlp_step_impl(s, cnt, N, t_stride ? off(dt) : (const double*)dt, t_stride, off(dq), off(dx), off(dy),
-                         off(dx0), (double*)off(dsol), dst ? (int32_t*)dst + lo : nullptr,
-                         dit ? (int32_t*)dit + lo : nullptr, dact ? (uint32_t*)dact + lo : nullptr, max_iter,
-                         s->scratch.stream[0]);
-      if (zs != CLIK_OK) return zs;
-      CK(cudaStreamSynchronize(s->scratch.stream[0]));
-      return CLIK_OK;
-    }
-  }
-  std::vector<Field> f;
-  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
-  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
-  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
-  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
-  f[0].rowmask = s->qp_reads.t;
-  f[1].rowmask = s->qp_reads.q;
-  f[2].rowmask = s->qp_reads.x;
-  f[3].rowmask = s->qp_reads.y;
-  f.push_back({x0, nullptr, d.qp_n, 8, 1, 0});
-  f.push_back({nullptr, sol, d.qp_n, 8, 1, 0});
-  f.push_back({nullptr, status, 1, 4, 1, 0});
-  f.push_back({nullptr, iters, 1, 4, 1, 0});
-  f.push_back({nullptr, active, 2, 4, 1, 0});
-  return run_host_pipeline(s, N, lo, cnt, f, [&](char* base, int64_t c, cudaStream_t stream) {
-    return nlp_step_impl(s, c, c, (const double*)(base + f[0].dev_off), t_stride,
-                         (const double*)(base + f[1].dev_off),
-                         d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
-                         d.n_input ? (const double*)(base + f[3].dev_off) : nullptr,
-                         x0 ? (const double*)(base + f[4].dev_off) : nullptr, (double*)(base + f[5].dev_off),
-                         status ? (int32_t*)(base + f[6].dev_off) : nullptr,
-                         iters ? (int32_t*)(base + f[7].dev_off) : nullptr,
-                         active ? (uint32_t*)(base + f[8].dev_off) : nullptr, max_iter, stream);
-  });
-}
-
 }  // namespace
 
 extern "C" {
@@ -1126,7 +1043,17 @@ clik_status clik_nlp_step_host_multi(const clik_skill* const* skills, int32_t n_
   if (!skills[0]->nlp.kernel) return fail(CLIK_ERR_INVALID, "skill was built without the NLP kernel");
   if (!sol) return fail(CLIK_ERR_INVALID, "sol is required");
   return run_sharded(skills, n_skills, N, [&](clik_skill* s, int64_t lo, int64_t cnt) {
-    return nlp_host_range(s, N, lo, cnt, t, t_stride, q, x, y, x0, sol, status, iters, active, max_iter);
+    const clik_skill_desc& d = s->desc;
+    const ReadMask& r = s->qp_reads;
+    const std::array<HostField, 9> f = {{{t, IN, 1, 8, t_stride == 0, r.t}, {q, IN, d.n_robot, 8, false, r.q},
+                                         {x, IN, d.n_virtual, 8, false, r.x}, {y, IN, d.n_input, 8, false, r.y},
+                                         {x0, IN, d.qp_n, 8}, {sol, OUT, d.qp_n, 8}, {status, OUT, 1, 4},
+                                         {iters, OUT, 1, 4}, {active, OUT, 2, 4}}};
+    return run_host_batch(s, N, lo, cnt, f, [&](const std::array<DevPtr, 9>& p, int64_t n, int64_t ld,
+                                                cudaStream_t stream, bool) {
+      auto [dt, dq, dx, dy, dx0, dsol, dstatus, diters, dactive] = p;
+      return nlp_step_impl(s, n, ld, dt, t_stride, dq, dx, dy, dx0, dsol, dstatus, diters, dactive, max_iter, stream);
+    });
   });
 }
 
@@ -1148,33 +1075,27 @@ clik_status clik_nlp_solve_one_lam(const clik_skill* cs, double t, const double*
   if (d.n_virtual > 0 && !x) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x is required");
   if (d.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
   ON_DEVICE(d.device);
-  std::lock_guard<std::mutex> lock(s->mu);
-  const int nq = d.n_robot, nx = d.n_virtual, ny = d.n_input, qn = d.qp_n, qm = lam ? d.qp_m : 0;
-  clik_status st = one_slot(s, (size_t)(1 + nq + nx + ny + 2 * qn + 3 + qm));
-  if (st != CLIK_OK) return st;
-  double* h = s->one_host;
+  const int qn = d.qp_n, qm = lam ? d.qp_m : 0;
+  OneSlot o;
   // slot: t | q | x | y | x0 | sol | status, iters, active_up, active_lo (four int cells in two doubles) | lam
-  h[0] = t;
-  std::memcpy(h + 1, q, sizeof(double) * nq);
-  if (nx) std::memcpy(h + 1 + nq, x, sizeof(double) * nx);
-  if (ny) std::memcpy(h + 1 + nq + nx, y, sizeof(double) * ny);
-  const size_t o_x0 = 1 + nq + nx + ny, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
+  clik_status st = fill_one_slot(s, 2 * qn + 2 + qm, t, q, x, y, &o);
+  if (st != CLIK_OK) return st;
+  const size_t o_x0 = o.own, o_sol = o_x0 + qn, o_int = o_sol + qn, o_lam = o_int + 2;
+  double *h = o.host, *dv = o.dev;
   if (x0) std::memcpy(h + o_x0, x0, sizeof(double) * qn);
-  double* dv = s->one_dev;
   long long n = 1, l = 1;
   int ts = 0;
   int mi = max_iter > 0 ? max_iter : NLP_DEFAULT_MAX_ITER;
-  const double *dt = dv, *dq = dv + 1, *dx = nx ? dv + 1 + nq : nullptr, *dy = ny ? dv + 1 + nq + nx : nullptr;
   const double* dx0 = x0 ? dv + o_x0 : nullptr;
   double* dsol = dv + o_sol;
   int* dst = (int*)(dv + o_int);
   int* dit = dst + 1;
   unsigned* dact = (unsigned*)(dst + 2);      // active[0], active[ld = 1]
-  void* args[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dx0, &dsol, &dst, &dit, &dact, &mi};
+  void* args[] = {&n, &l, &o.t, &ts, &o.q, &o.x, &o.y, &dx0, &dsol, &dst, &dit, &dact, &mi};
   CK(cudaLaunchKernel((const void*)s->nlp.kernel, dim3(1), dim3(32), args, 0, s->one_stream));
   if (lam) {
     double* dlam = dv + o_lam;
-    void* largs[] = {&n, &l, &dt, &ts, &dq, &dx, &dy, &dsol, &dst, &dact, &dlam};
+    void* largs[] = {&n, &l, &o.t, &ts, &o.q, &o.x, &o.y, &dsol, &dst, &dact, &dlam};
     CK(cudaLaunchKernel((const void*)s->nlp_duals.kernel, dim3(1), dim3(32), largs, 0, s->one_stream));
   }
   CK(cudaStreamSynchronize(s->one_stream));
@@ -1241,52 +1162,22 @@ clik_status duals_impl(const clik_skill* s, bool nlp, int64_t N, int64_t ld, con
   return CLIK_OK;
 }
 
-// Host arrays (as nlp_host_range): the kernel on mapped memory when every buffer is page-locked, else the
-// chunked copy pipeline.
+// Host arrays: the kernel on mapped memory when every buffer is page-locked, else the chunked copy pipeline.
 clik_status duals_host(clik_skill* s, bool nlp, int64_t N, const double* t, int32_t t_stride, const double* q,
                        const double* x, const double* y, const double* sol, const int32_t* status,
                        const uint32_t* active, double* lam) {
   clik_status st = duals_check(s, nlp, N, t, q, x, y, sol, status, active, lam);
   if (st != CLIK_OK || N == 0) return st;
   const clik_skill_desc& d = s->desc;
-  if (zero_copy_enabled()) {
-    const void *dt, *dq, *dx, *dy, *dsol, *dst, *dact, *dlam;
-    ON_DEVICE(d.device);
-    if (device_alias(t, &dt) && device_alias(q, &dq) && device_alias(d.n_virtual ? x : nullptr, &dx) &&
-        device_alias(d.n_input ? y : nullptr, &dy) && device_alias(sol, &dsol) && device_alias(status, &dst) &&
-        device_alias(active, &dact) && device_alias(lam, &dlam)) {
-      std::lock_guard<std::mutex> lock(s->mu);
-      clik_status zs = ensure_scratch(s, 0, 256);
-      if (zs != CLIK_OK) return zs;
-      GridCapScope cap(zero_copy_ctas_per_sm(), s->sm_count);
-      zs = duals_impl(s, nlp, N, N, (const double*)dt, t_stride, (const double*)dq, (const double*)dx,
-                      (const double*)dy, (const double*)dsol, (const int32_t*)dst, (const uint32_t*)dact,
-                      (double*)dlam, s->scratch.stream[0]);
-      if (zs != CLIK_OK) return zs;
-      CK(cudaStreamSynchronize(s->scratch.stream[0]));
-      return CLIK_OK;
-    }
-  }
-  std::vector<Field> f;
-  f.push_back({t, nullptr, 1, 8, t_stride ? 1 : 0, 0});
-  f.push_back({q, nullptr, d.n_robot, 8, 1, 0});
-  f.push_back({d.n_virtual ? x : nullptr, nullptr, d.n_virtual, 8, 1, 0});
-  f.push_back({d.n_input ? y : nullptr, nullptr, d.n_input, 8, 1, 0});
-  f[0].rowmask = s->qp_reads.t;
-  f[1].rowmask = s->qp_reads.q;
-  f[2].rowmask = s->qp_reads.x;
-  f[3].rowmask = s->qp_reads.y;
-  f.push_back({sol, nullptr, d.qp_n, 8, 1, 0});
-  f.push_back({status, nullptr, 1, 4, 1, 0});
-  f.push_back({active, nullptr, 2, 4, 1, 0});
-  f.push_back({nullptr, lam, d.qp_m, 8, 1, 0});
-  return run_host_pipeline(s, N, 0, N, f, [&](char* base, int64_t c, cudaStream_t stream) {
-    return duals_impl(s, nlp, c, c, (const double*)(base + f[0].dev_off), t_stride,
-                      (const double*)(base + f[1].dev_off),
-                      d.n_virtual ? (const double*)(base + f[2].dev_off) : nullptr,
-                      d.n_input ? (const double*)(base + f[3].dev_off) : nullptr, (const double*)(base + f[4].dev_off),
-                      (const int32_t*)(base + f[5].dev_off), (const uint32_t*)(base + f[6].dev_off),
-                      (double*)(base + f[7].dev_off), stream);
+  const ReadMask& r = s->qp_reads;
+  const std::array<HostField, 8> f = {{{t, IN, 1, 8, t_stride == 0, r.t}, {q, IN, d.n_robot, 8, false, r.q},
+                                       {x, IN, d.n_virtual, 8, false, r.x}, {y, IN, d.n_input, 8, false, r.y},
+                                       {sol, IN, d.qp_n, 8}, {status, IN, 1, 4}, {active, IN, 2, 4},
+                                       {lam, OUT, d.qp_m, 8}}};
+  return run_host_batch(s, N, 0, N, f, [&](const std::array<DevPtr, 8>& p, int64_t n, int64_t ld,
+                                           cudaStream_t stream, bool) {
+    auto [dt, dq, dx, dy, dsol, dstatus, dactive, dlam] = p;
+    return duals_impl(s, nlp, n, ld, dt, t_stride, dq, dx, dy, dsol, dstatus, dactive, dlam, stream);
   });
 }
 

@@ -46,6 +46,40 @@ def test_argument_validation_needs_no_device():
     assert b"nx <= 32, m <= 64" in lib.clik_last_error()
 
 
+# Host-array and single-instance entry points with a NULL skill or an empty handle array: (name, arguments after
+# the handle(s) with N = 4 and every array NULL, message).  The *_multi forms are called with no array, with a
+# count of 0 and with one NULL handle.
+_HOST_ENTRY_POINTS = [
+    ("clik_pinv_step_host", (4, None, 0) + (None,) * 6, b"no skill handles"),
+    ("clik_qp_step_host", (4, None, 0) + (None,) * 8 + (0,), b"no skill handles"),
+    ("clik_nlp_step_host", (4, None, 0) + (None,) * 8 + (0,), b"no skill handles"),
+    ("clik_pinv_step_host_multi", (4, None, 0) + (None,) * 6, b"no skill handles"),
+    ("clik_qp_step_host_multi", (4, None, 0) + (None,) * 8 + (0,), b"no skill handles"),
+    ("clik_nlp_step_host_multi", (4, None, 0) + (None,) * 8 + (0,), b"no skill handles"),
+    ("clik_qp_duals_host", (4, None, 0) + (None,) * 7, b"skill is NULL"),
+    ("clik_nlp_duals_host", (4, None, 0) + (None,) * 7, b"skill is NULL"),
+    ("clik_pinv_solve_one", (0.0,) + (None,) * 6, b"NULL argument"),
+    ("clik_qp_solve_one", (0.0,) + (None,) * 7 + (0,), b"NULL argument"),
+    ("clik_qp_solve_one_lam", (0.0,) + (None,) * 7 + (0, None), b"NULL argument"),
+    ("clik_nlp_solve_one", (0.0,) + (None,) * 8 + (0,), b"NULL argument"),
+    ("clik_nlp_solve_one_lam", (0.0,) + (None,) * 8 + (0, None), b"NULL argument"),
+]
+
+
+@pytest.mark.parametrize("name,args,message", _HOST_ENTRY_POINTS, ids=[e[0] for e in _HOST_ENTRY_POINTS])
+def test_host_entry_points_reject_a_missing_skill_without_a_device(name, args, message):
+    lib = runtime.load_library()
+    fn = getattr(lib, name)
+    if name.endswith("_multi"):
+        one_null = (ctypes.c_void_p * 1)(None)
+        calls = [(None, 1), (one_null, 0), (one_null, 1)]
+    else:
+        calls = [(None,)]
+    for handles in calls:
+        assert fn(*handles, *args) == 1, (name, handles)      # CLIK_ERR_INVALID
+        assert message in lib.clik_last_error(), (name, handles, lib.clik_last_error())
+
+
 def test_no_cpu_fallback_without_a_device():
     if runtime.device_count() > 0:
         pytest.skip("a CUDA device is present")
