@@ -20,7 +20,8 @@
 //   NLP: grad^2 F(x*) = L L' (no shift), columns L^-1 a_r, pre-scaled gradient -L^-1 xb, u = L^-T L^-1 (xb - A_W' v).
 // lam is the multipliers routine's own output.  Rules: an all-zero cotangent column gives theta_bar = 0 exactly
 // (whatever the status); otherwise theta_bar is NaN when the status is not 0, when A_W is rank-deficient (the
-// tests of clik_duals.cuh) or, for the NLP, when grad^2 F(x*) is not positive definite.
+// tests of clik_duals.cuh) or, for the NLP, when a Cholesky pivot of grad^2 F(x*) is at or below
+// 1e-12 max(1, max_j |H_jj|), the step's own threshold (singular or indefinite to working precision).
 //
 // The generated skill provides (codegen/emit.py, emit_skill(..., vjp=True)) S::eval_vjp — the gradient program
 // of Phi over the skill's expression graph — and the read masks VJP_READ_* (rows eval_vjp and the row evaluation
@@ -164,7 +165,11 @@ __device__ __forceinline__ void nlp_vjp(long long N, long long ld, const double*
         }
         S::eval_nlp_fgH(d.P, xs, g, H);
         ok = working_set_multipliers<NN, M>(d.A, one, g, up, lo, lam);
-        if (ok) ok = nlp_cholesky<NN>(H, 0.0, 0.0, L);
+        // the step's pivot threshold (clik_nlp.cuh): on a singular Hessian the trailing pivots are rounding noise of
+        // either sign, and a positive one would give a finite theta_bar of that noise
+        double hmax = 1.0;
+        for (int j = 0; j < NN; ++j) hmax = fmax(hmax, fabs(H[j * (j + 1) / 2 + j]));
+        if (ok) ok = nlp_cholesky<NN>(H, 0.0, 1e-12 * hmax, L);
         int W[NN], k;
         double v[M], Q[NN * NN], R[NN * NN];
         if (ok) ok = working_set_rows<NN, M>(up, lo, W, k, v);

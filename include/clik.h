@@ -286,7 +286,8 @@ clik_status clik_nlp_duals_host(const clik_skill* skill, int64_t N, const double
  *            size is 0)
  * Rules: an instance whose cotangent column is all zeros gets exactly 0, whatever its status; otherwise every
  * output of the instance is NaN when status[i] is not 0, when A_W is rank-deficient (the tests of clik_qp_duals)
- * or, for the NLP, when grad^2 F(x*) is not positive definite (the Cholesky factorisation fails).
+ * or, for the NLP, when a Cholesky pivot of grad^2 F(x*) is at or below 1e-12 max(1, max_j |H_jj|), the pivot threshold
+ * of the step itself (a Hessian that is singular or indefinite to working precision).
  * The kernel is in images built with emit_skill(..., vjp=True) (manifest o[19]) only, and only for skills with
  * 1..32 constraint rows: other images, and a NULL skill, fail with CLIK_ERR_INVALID.  Device pointers only, row
  * stride N, asynchronous on `stream`; one thread per instance. */

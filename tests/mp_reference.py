@@ -472,3 +472,451 @@ def family_kappa(blocks, row_block=-1):
             ev = mp.eigsy(G, eigvals_only=True)
             out[i] = math.inf if min(ev) <= 0 else float(max(ev) / min(ev))
     return out
+
+
+# ----------------------------------------------------------------------------------------------
+# faces of the QP and NLP steps: solution, certificate and derivative at 50 (80) digits
+# ----------------------------------------------------------------------------------------------
+#
+# The face problem of a working set W (masks up / lo; b_r = ub_r on an upper bit, lb_r on a lower bit):
+#
+#     r1 = g(x, theta) + A_W(theta)' lam_W = 0,    r2 = A_W(theta) x - b_W(theta) = 0,
+#
+# g = H x (QP, H = diag(h)) or grad F (NLP).  K = [[M, A_W'], [A_W, 0]] with M = H or grad^2 F(x*).
+#
+# Criteria of tests/test_face_reference_on_host.py and tests/test_gpu_face_reference.py, derived here.
+#
+# Metric and kappa.  Both kernels work in the metric of a factor L of M (QP: L = H^1/2, exact to one rounding per
+# entry; NLP: the Cholesky factor of grad^2 F, whose backward error u|M| is a forward error of up to u kappa(M)
+# relative), on the rows B = A_W L^-T: the scaled face matrix K' = [[I, B'], [B, 0]] has the eigenvalues 1,
+# (1 +- sqrt(1 + 4 mu)) / 2 for the eigenvalues mu of B B' (as in qp_face_reference).  kappa = kappa(K') for the
+# QP and kappa(K') kappa(M) for the NLP; the accuracy claim is made where kappa u < CLAIM, as for the other steps.
+#
+# NLP step.  x is compared in the L metric, |L'(x - x_ref)| <= C u kappa s + |L'| E_stop, s = |(L'x_ref, lam_ref)|.
+# E_stop is what the two stopping rules of clik_nlp.cuh leave.  Rule 1 accepts the full step p of the subproblem
+# at v with |p|_inf max(1, delta) <= tol (1 + |v|_inf); rule 2 a line-search step alpha p (alpha <= 1) with
+# |p|_inf <= 100 tol (1 + |v|_inf).  Without a shift (delta = 0) p is the Newton step of the face, so the error of
+# the returned point is at most |p| (alpha < 1) plus a term of second order; with a shift the iteration contracts
+# by delta / (lambda + delta) per step and the error is at most |p| (1 + delta / lambda_min(M)).  Both rules
+# together (where a rule runs): E_stop = 100 tol (1 + |x|_inf) sqrt(nx) (1 + delta_hat / lambda_min(M)).  delta_hat is the largest
+# shift the step can have used: 0 where lambda_min(M) > 2e-12 max(1, max_j M_jj) (every Cholesky pivot is at least
+# lambda_min minus (n + 1) u of the diagonal, above the step's pivot threshold 1e-12 max(1, max_j M_jj)), else the
+# first shift 1e-8 max(1, max_j M_jj), which makes a positive semi-definite M factorisable.
+#
+# NLP backward error (every status-0 instance, whatever kappa): the stationarity residual |g(x) + A' lam|_j at the
+# returned x and its multipliers.  Rule 1 leaves (H~ - H - delta) p with H~ the mean Hessian on [v, x]: at most
+# tol (1 + |v|_inf) plus a term of second order; rule 2 leaves (alpha H~ - H - delta) p, at most
+# (|M|_inf + delta_hat) 100 tol (1 + |x|_inf).  The rounding of the subproblem, solved in the metric of L (M = L L'),
+# adds (k + 1) C u of the sizes of the terms (as qp_residuals) and (k + 1) C u |L|_2 s_L, s_L = |L'x| + |L^-1 c| +
+# |L^-1 A' lam| (c = g - M x), mapped to x through L (on a row: |L^-1 a_r| s_L).
+#
+# Where no stopping rule runs, E_stop and both stopping terms are 0 (exact_step): the QP, and a cost quadratic in
+# the decision variables without a possible shift, which the step solves by its first subproblem.  Its error is then
+# arithmetic alone.  Rule 2's bound is first order in |p| (it must allow a line-search step alpha < 1), so a widened
+# rule 2 can stay inside it; test_face_reference_on_host.py checks the claim of include/clik.h on the last step itself.
+#
+# Multipliers (NLP, metric D = I): |lam - lam_ref| <= C u kappa s + |A_W^+|_2 |g(x) - g(x_ref)|_2, the second term
+# the 50-digit sensitivity of the least-squares multipliers to the kernel's own x.
+#
+# VJP.  theta_bar = -[u; v]' dr/dtheta with K [u; v] = [xb; 0].  The adjoint solve in the scaled metric has
+# the error C u kappa |w'| (w' = [L'u; v]), which reaches u through L^-T: per theta entry k the bound is
+# C u kappa (|dr1/dtheta_k|_2 |L^-1|_2 + |dr2/dtheta_k|_2) |w'|_2 + ATOL.  What the kernel's fp64 x* and lam carry
+# into Phi is evaluated at 50 digits along the kernel's own point: |theta_bar_50(x_kernel, lam_50(x_kernel)) -
+# theta_bar_ref|_inf is added to the bound.
+#
+# NaN bands (as the multipliers' rank rule): theta_bar may be NaN only where the face's sigma_min / sigma_max (in
+# the kernel's metric) is below 1e-9 or, NLP only, lambda_min / max(1, lambda_max) of grad^2 F(x*) is below 1e-9
+# (the kernels' 1e-12 thresholds widened by RANK_BAND), and must be NaN where either is below 1e-15.
+
+TOL_NLP = 1e-10        # ReactiveNLPController's default options["tol"]
+
+
+def exact_step(P, delta_hat):
+    """True where no stopping rule runs: the QP, and an NLP whose cost is quadratic in the decision variables
+    (S::NLP_QUADRATIC) with no shift possible, which clik_nlp.cuh solves by its first subproblem (`exact`).  Its
+    error is then arithmetic alone, and E_stop = 0."""
+    return P.qp or (P.prog.quadratic and delta_hat == 0)
+
+
+class MpProblem(object):
+    """One instance of a lowered program (codegen.lower.QpProgram or NlpProgram) at `dps` digits.  `vals`: symbol
+    id -> float or mpf for t, q, x, y.  A (m rows of nx mpf), lb, ub; fgH(x) -> (F, g, H as an mp.matrix) of the
+    cost (QP: 1/2 x' diag(h) x)."""
+
+    def __init__(self, prog, vals, dps=DPS):
+        self.prog, self.vals, self.dps = prog, dict(vals), dps
+        self.qp = not hasattr(prog, "F")
+        self.nx, self.m = nx, m = prog.nx, prog.m
+        flat = [n for r in prog.A for n in r] + list(prog.lb) + list(prog.ub) + (list(prog.h) if self.qp else [])
+        with mp.workdps(dps):
+            out = _eval_order(dag.topo(flat), flat, self.vals)
+        k = m * nx
+        self.A = [out[r * nx:(r + 1) * nx] for r in range(m)]
+        self.lb, self.ub = out[k:k + m], out[k + m:k + 2 * m]
+        if self.qp:
+            self.h = out[k + 2 * m:]
+        else:
+            self._nodes = [prog.F] + list(prog.g) + list(prog.H)
+            self._order = dag.topo(self._nodes)
+
+    def fgH(self, x):
+        nx = self.nx
+        with mp.workdps(self.dps):
+            if self.qp:
+                g = [self.h[j] * x[j] for j in range(nx)]
+                return sum(g[j] * x[j] for j in range(nx)) / 2, g, mp.diag(self.h)
+            vals = dict(self.vals)
+            vals.update({n.id: x[j] for j, n in enumerate(self.prog.dec)})
+            out = _eval_order(self._order, self._nodes, vals)
+            H = mp.matrix(nx, nx)
+            for i in range(nx):
+                for j in range(i + 1):
+                    H[i, j] = H[j, i] = out[1 + nx + i * (i + 1) // 2 + j]
+            return out[0], out[1:1 + nx], H
+
+    def rows(self, up, lo):
+        """W and b_W of the masks (an upper bit selects ub, as the kernels' vjp_split_v)."""
+        W = [r for r in range(self.m) if ((up | lo) >> r) & 1]
+        return W, [self.ub[r] if (up >> r) & 1 else self.lb[r] for r in W]
+
+
+def mp_problem(prog, inp, i, dps=DPS, theta=None):
+    """MpProblem of instance i of the batch `inp` (the layout of sc.sample); theta: {symbol id: offset} added to
+    the inputs at `dps` digits."""
+    from nlp_oracle import _inputs_map
+    vals = {k: mp.mpf(v) for k, v in _inputs_map(prog, inp, i).items()}
+    with mp.workdps(dps):
+        for k, d in (theta or {}).items():
+            vals[k] = vals[k] + d
+    return MpProblem(prog, vals, dps)
+
+
+def theta_symbols(prog, rows):
+    """The symbol id of each (key, row) of test_vjp_on_host.theta_rows (None where the program does not read it)."""
+    syms = {"t": prog.syms.t, "q": prog.syms.q, "x": prog.syms.x, "y": prog.syms.y}
+    out = []
+    for key, row in rows:
+        nodes = syms[key]
+        j = 0 if row is None else row
+        out.append(nodes[j].id if j < len(nodes) else None)
+    return out
+
+
+def check_derivatives(P, x, dps=120):
+    """Largest |prog.g - d F| and |prog.H - d2 F| (mp.diff of prog.F, central differences with h = 1e-30 on a
+    `dps`-digit evaluation: truncation ~1e-60, rounding ~1e-60) at x, relative to 1 + the largest entry: the only
+    place where the NLP referee relies on the product's automatic differentiation."""
+    nx = P.nx
+    Q = MpProblem(P.prog, P.vals, dps)
+    with mp.workdps(dps):
+        step = mp.mpf(10) ** -30
+        xm = [mp.mpf(v) for v in x]
+        _, g, H = Q.fgH(xm)
+
+        def F(*v):
+            return Q.fgH(list(v))[0]
+        worst = mp.mpf(0)
+        for j in range(nx):
+            d = [0] * nx
+            d[j] = 1
+            worst = max(worst, abs(mp.diff(F, xm, tuple(d), h=step) - g[j]) / (1 + max(abs(a) for a in g)))
+            for i in range(j + 1):
+                d2 = [0] * nx
+                d2[i] += 1
+                d2[j] += 1
+                hmax = 1 + max(abs(H[a, b]) for a in range(nx) for b in range(nx))
+                worst = max(worst, abs(mp.diff(F, xm, tuple(d2), h=step) - H[i, j]) / hmax)
+    return float(worst)
+
+
+def _face_newton(P, up, lo, x0):
+    """Newton on [r1; r2] = 0 of the face from x0 until the residual is below 10^(10 - dps) (1e-40 at 50 digits).
+    -> (x, lam_W, W) as mpf lists, or None where K is singular at this precision or Newton does not converge."""
+    W, b = P.rows(up, lo)
+    nx, k = P.nx, len(W)
+    with mp.workdps(P.dps):
+        tol = mp.mpf(10) ** (10 - P.dps)
+        x = [mp.mpf(v) for v in x0]
+        lam = [mp.mpf(0)] * k
+        for _ in range(40):
+            _, g, H = P.fgH(x)
+            r = [g[j] + sum(P.A[W[a]][j] * lam[a] for a in range(k)) for j in range(nx)]
+            r += [sum(P.A[W[a]][j] * x[j] for j in range(nx)) - b[a] for a in range(k)]
+            if max(abs(v) for v in r) < tol:
+                return x, lam, W
+            K = mp.zeros(nx + k, nx + k)
+            for i in range(nx):
+                for j in range(nx):
+                    K[i, j] = H[i, j]
+            for a in range(k):
+                for j in range(nx):
+                    K[nx + a, j] = K[j, nx + a] = P.A[W[a]][j]
+            try:
+                d = mp.lu_solve(K, mp.matrix([-v for v in r]))
+            except ZeroDivisionError:
+                return None
+            x = [x[j] + d[j] for j in range(nx)]
+            lam = [lam[a] + d[nx + a] for a in range(k)]
+    return None
+
+
+def _eigs(S):
+    ev = mp.eigsy(S, eigvals_only=True)
+    return min(ev), max(ev)
+
+
+def face_solve(P, up, lo, x0, tol=TOL_NLP):
+    """The face of the working set (up, lo) at P's precision, from the kernel's x0.  -> dict of
+      x, lam (m,) float64 (CasADi's signs, 0 off W), xm / lamW (mpf), W;
+      kappa (the criterion's kappa), kappa_K (of K' in the kernel's metric), kappa_M (of M), rank_ratio
+      (sigma_min / sigma_max of B = A_W L^-T), hess_ratio (lambda_min / max(1, lambda_max) of M), lam_min (of M);
+      ratio (smallest decision margin over its bound), cert (feasible, stationary, signs right, reduced Hessian
+      positive definite: for a convex F a proof of global optimality), scale s, bound (C u kappa s + ATOL), e_stop
+      (the NLP's stopping error in the L metric), Lnorm / Linv (|L'|_2, |L^-1|_2)."""
+    nx, m = P.nx, P.m
+    W, _ = P.rows(up, lo)
+    k = len(W)
+    bad = {"x": np.full(nx, np.nan), "lam": np.full(m, np.nan), "cert": False, "kappa": math.inf, "kappa_K": math.inf,
+           "kappa_M": math.inf, "rank_ratio": 0.0, "hess_ratio": 0.0, "ratio": 0.0, "W": W, "xm": None}
+    sol = _face_newton(P, up, lo, x0)
+    with mp.workdps(P.dps):
+        _, _, H = P.fgH(sol[0] if sol else [mp.mpf(v) for v in x0])
+        ev_lo, ev_hi = _eigs(H)
+        hmax = max([mp.mpf(1)] + [abs(H[j, j]) for j in range(nx)])
+        bad["hess_ratio"] = float(ev_lo / max(1, ev_hi))
+        bad["lam_min"] = float(ev_lo)
+        if k:
+            Aw = mp.matrix([P.A[r] for r in W])
+            mu0 = _eigs(Aw * Aw.T)
+            bad["rank_ratio_plain"] = float(mp.sqrt(max(mu0[0], 0) / mu0[1])) if mu0[1] > 0 else 0.0
+        try:                     # singular to 50 digits (an eigenvalue of rounding size) counts as singular
+            L = mp.cholesky(H) if ev_lo > 0 else None
+        except ValueError:
+            L = None
+        if L is not None:
+            Bt = [mp.lu_solve(L, mp.matrix(P.A[r])) for r in W]          # rows of B = A_W L^-T
+            if k:
+                B = mp.matrix([[Bt[a][j] for j in range(nx)] for a in range(k)])
+                mu_lo, mu_hi = _eigs(B * B.T)
+            else:
+                mu_lo = mu_hi = mp.mpf(1)
+            bad["rank_ratio"] = rank_ratio = float(mp.sqrt(mu_lo / mu_hi)) if mu_lo > 0 else 0.0
+        if sol is None or L is None:
+            return bad
+        x, lamW, _ = sol
+        eigs = [mp.mpf(1)] + [(1 + mp.sqrt(1 + 4 * u_)) / 2 for u_ in (mu_lo, mu_hi)] + \
+               [(mp.sqrt(1 + 4 * u_) - 1) / 2 for u_ in (mu_lo, mu_hi)]
+        kappa_K = float(max(eigs) / min(eigs)) if mu_lo > 0 else math.inf
+        kappa_M = 1.0 if P.qp else float(ev_hi / ev_lo)
+        kappa = kappa_K * kappa_M
+        z = L.T * mp.matrix(x)
+        sn = math.sqrt(sum(float(v) ** 2 for v in list(z) + lamW))
+        bnd = C * U * kappa * sn + ATOL
+        delta_hat = 0.0 if ev_lo > 2e-12 * hmax else 1e-8 * float(hmax)
+        xinf = max(float(abs(v)) for v in x)
+        e_stop = 0.0 if exact_step(P, delta_hat) else \
+            100 * tol * (1 + xinf) * math.sqrt(nx) * (1 + delta_hat / float(ev_lo))
+        lam = [mp.mpf(0)] * m
+        for a, r in enumerate(W):
+            lam[r] = lamW[a]
+        tau = mp.mpf(10) ** (-30)
+        _, g, _ = P.fgH(x)
+        cert = max([abs(g[j] + sum(P.A[r][j] * lam[r] for r in W)) for j in range(nx)]) < tau
+        ratio = math.inf
+        for r in range(m):
+            row = sum(P.A[r][j] * x[j] for j in range(nx))
+            lo_r, hi_r = P.lb[r], P.ub[r]
+            cert &= (row >= lo_r - tau * (1 + abs(lo_r))) and (row <= hi_r + tau * (1 + abs(hi_r)))
+            if r in W:
+                if lo_r != hi_r:      # an equality row's multiplier may have either sign: no decision
+                    cert &= (lam[r] >= 0) if (up >> r) & 1 else (lam[r] <= 0)
+                    ratio = min(ratio, float(abs(lam[r])) / bnd)
+            else:
+                rn = float(mp.norm(mp.lu_solve(L, mp.matrix(P.A[r]))))
+                slack = min(row - lo_r, hi_r - row)
+                ratio = min(ratio, float(slack) / (rn * (bnd + float(mp.sqrt(ev_hi)) * e_stop)
+                                                   + C * U * (1 + float(max(abs(lo_r), abs(hi_r))))))
+        # reduced Hessian: M is positive definite here, hence also on the null space of A_W
+    return {"x": np.array([float(v) for v in x]), "lam": np.array([float(v) for v in lam]), "xm": x, "lamW": lamW,
+            "W": W, "cert": bool(cert), "kappa": kappa, "kappa_K": kappa_K, "kappa_M": kappa_M,
+            "rank_ratio": rank_ratio, "rank_ratio_plain": bad.get("rank_ratio_plain", 1.0),
+            "hess_ratio": float(ev_lo / max(1, ev_hi)), "lam_min": float(ev_lo), "ratio": ratio, "scale": sn,
+            "bound": bnd, "e_stop": e_stop, "Lnorm": float(mp.sqrt(ev_hi)), "Linv": float(1 / mp.sqrt(ev_lo)),
+            "LT": _f(L.T.tolist())}
+
+
+DDPS = 80              # digits of the derivative routes
+DH = mp.mpf(10) ** -25  # their central-difference step (relative to max(1, |theta_k|))
+
+
+def _theta_step(P, sid):
+    with mp.workdps(DDPS):
+        return DH * max(1, abs(mp.mpf(P.vals[sid])))
+
+
+def _shifted(P, sid, d):
+    vals = dict(P.vals)
+    with mp.workdps(DDPS):
+        vals[sid] = mp.mpf(vals[sid]) + d
+    return MpProblem(P.prog, vals, DDPS)
+
+
+def face_derivative(P, up, lo, x, sids):
+    """dx*/dtheta (nx, n_theta) of the face of (up, lo), W held fixed, by a central difference of the 80-digit face
+    solution (h = 1e-25): from the definition, sharing nothing with codegen/vjp.py's Phi, dag.jacobian over theta
+    or the adjoint solve.  x: a point near the face's solution (the Newton start).  Columns of unread symbols are 0."""
+    out = np.zeros((P.nx, len(sids)), dtype=object)
+    with mp.workdps(DDPS):
+        for c, sid in enumerate(sids):
+            if sid is None:
+                out[:, c] = mp.mpf(0)
+                continue
+            h = _theta_step(P, sid)
+            xp = _face_newton(_shifted(P, sid, h), up, lo, x)[0]
+            xq = _face_newton(_shifted(P, sid, -h), up, lo, x)[0]
+            out[:, c] = [(a - b) / (2 * h) for a, b in zip(xp, xq)]
+    return out
+
+
+def _face_residual(P, W, b, x, lamW):
+    nx, k = P.nx, len(W)
+    _, g, _ = P.fgH(x)
+    r = [g[j] + sum(P.A[W[a]][j] * lamW[a] for a in range(k)) for j in range(nx)]
+    return r + [sum(P.A[W[a]][j] * x[j] for j in range(nx)) - b[a] for a in range(k)]
+
+
+def vjp_adjoint(P, up, lo, x, lamW, xb, sids):
+    """The adjoint formula of include/clik.h at 50 digits: K [u; v] = [xb; 0] with K = d(r1, r2)/d(x, lam) at x,
+    theta_bar = -[u; v]' dr/dtheta with x, lam_W held fixed (dr/dx and dr/dtheta by 80-digit central differences,
+    h = 1e-25).  -> (theta_bar
+    (n_theta,) mpf, per-theta error scale (n_theta,) float: (|dr1/dtheta_k| |L^-1| + |dr2/dtheta_k|) |[L'u; v]|)."""
+    nx = P.nx
+    W, b = P.rows(up, lo)
+    k = len(W)
+    P80 = MpProblem(P.prog, P.vals, DDPS)
+    with mp.workdps(DDPS):
+        # M = dg/dx of the residual itself (prog.H may differ from it by the rounding of constants the automatic
+        # differentiation folds, e.g. 2/0.3^2 of the quartic cost)
+        xm, lm = [mp.mpf(v) for v in x], [mp.mpf(v) for v in lamW]
+        Mcol = []
+        for j in range(nx):
+            h = DH * max(1, abs(xm[j]))
+            xp, xq = list(xm), list(xm)
+            xp[j] += h
+            xq[j] -= h
+            Mcol.append([(a - b) / (2 * h) for a, b in zip(P80.fgH(xp)[1], P80.fgH(xq)[1])])
+    with mp.workdps(P.dps):
+        _, _, H = P.fgH(xm)
+        K = mp.zeros(nx + k, nx + k)
+        for i in range(nx):
+            for j in range(nx):
+                K[i, j] = Mcol[j][i]
+        for a in range(k):
+            for j in range(nx):
+                K[nx + a, j] = K[j, nx + a] = P.A[W[a]][j]
+        w = mp.lu_solve(K, mp.matrix([mp.mpf(float(v)) for v in xb] + [0] * k))
+        ev_lo = _eigs(H)[0]
+        Linv = float(1 / mp.sqrt(ev_lo)) if ev_lo > 0 else math.inf
+        wn = float(mp.sqrt(sum((mp.cholesky(H).T * mp.matrix([w[j] for j in range(nx)]))[j] ** 2 for j in range(nx))
+                           + sum(w[nx + a] ** 2 for a in range(k)))) if ev_lo > 0 else math.inf
+    tb, scale = [], []
+    with mp.workdps(DDPS):
+        for sid in sids:
+            if sid is None:
+                tb.append(mp.mpf(0))
+                scale.append(0.0)
+                continue
+            h = _theta_step(P, sid)
+            rp = _face_residual(_shifted(P, sid, h), W, _shifted(P, sid, h).rows(up, lo)[1], xm, lm)
+            Pm = _shifted(P, sid, -h)
+            rm = _face_residual(Pm, W, Pm.rows(up, lo)[1], xm, lm)
+            d = [(a - c) / (2 * h) for a, c in zip(rp, rm)]
+            tb.append(-sum(w[i] * d[i] for i in range(nx + k)))
+            n1 = math.sqrt(sum(float(v) ** 2 for v in d[:nx]))
+            n2 = math.sqrt(sum(float(v) ** 2 for v in d[nx:]))
+            scale.append((n1 * Linv + n2) * wn)
+    return tb, np.array(scale)
+
+
+def vjp_bound(kappa, scale):
+    return C * U * kappa * scale + ATOL
+
+
+def ls_multipliers(P, up, lo, x):
+    """lam_W = argmin |D^1/2 (g(x) + A_W' lam)| at 50 digits at the point x, in the metric of clik_duals.cuh (QP
+    D = H^-1, NLP D = I) -> (lam (m,) float64, lam_W (mpf), |(D^1/2 A_W')^+|_2 (inf where rank deficient),
+    g(x) (mpf))."""
+    W, _ = P.rows(up, lo)
+    k = len(W)
+    with mp.workdps(P.dps):
+        xm = [mp.mpf(float(v)) for v in x]
+        _, g, _ = P.fgH(xm)
+        lam = np.zeros(P.m)
+        if not k:
+            return lam, [], 0.0, g
+        d = [1 / mp.sqrt(h) for h in P.h] if P.qp else [mp.mpf(1)] * P.nx
+        Aw = mp.matrix([[P.A[r][j] * d[j] for j in range(P.nx)] for r in W])
+        G = Aw * Aw.T
+        lo_ev = _eigs(G)[0]
+        if lo_ev <= 0:
+            return np.full(P.m, np.nan), None, math.inf, g
+        sol = mp.lu_solve(G, -(Aw * mp.matrix([g[j] * d[j] for j in range(P.nx)])))
+        for a, r in enumerate(W):
+            lam[r] = float(sol[a])
+        return lam, [sol[a] for a in range(k)], float(1 / mp.sqrt(lo_ev)), g
+
+
+def nlp_residuals(P, x, up, lo, lam, tol=TOL_NLP):
+    """Backward error of a returned NLP point x (float64) with its multipliers lam on its own working set, at 50
+    digits, as the ratio to its bound (module comment above the face section): the stationarity residual
+    |g(x) + A' lam|_j over (k + 1) C u (|g_j| + sum_r |a_rj lam_r|) + (|M|_inf + delta_hat) 100 tol (1 + |x|_inf),
+    and the held-row residual / bound violation over (k + 1) C u (sum_j |a_rj x_j| + |b_r|) + |a_r|_1 100 tol
+    (1 + |x|_inf) (a line-search step of rule 2 stops short of the face by at most |p|)."""
+    nx, m = P.nx, P.m
+    W, b = P.rows(up, lo)
+    k1 = len(W) + 1
+    with mp.workdps(P.dps):
+        xm = [mp.mpf(float(v)) for v in x]
+        lm = [mp.mpf(float(v)) for v in lam]
+        _, g, H = P.fgH(xm)
+        xinf = max(abs(v) for v in xm)
+        hmax = max([mp.mpf(1)] + [abs(H[j, j]) for j in range(nx)])
+        dhat = 0 if _eigs(H)[0] > 2e-12 * hmax else 1e-8 * hmax
+        Minf = max(sum(abs(H[i, j]) for j in range(nx)) for i in range(nx))
+        exact = exact_step(P, dhat)
+        stop_g = 0 if exact else (Minf + dhat) * 100 * tol * (1 + xinf)
+        stop_r = 0 if exact else 100 * tol * (1 + xinf)
+        # the subproblem is solved in the metric of L (M = L L'): its backward error reaches x through L, so the
+        # rounding of its terms s_L = |L'x| + |L^-1 c| + |L^-1 A' lam| (c = g - M x) counts with |L|_2 there
+        ev_lo, ev_hi = _eigs(H)
+        Linv_rows = [mp.mpf(0)] * m
+        round_g = mp.mpf(0)
+        try:
+            L = mp.cholesky(H) if ev_lo > 0 else None
+        except ValueError:       # positive definite below mpmath's tolerance: a shifted step, the stop terms cover it
+            L = None
+        if L is not None:
+            xv = mp.matrix(xm)
+            at_lam = mp.matrix([sum(P.A[r][j] * lm[r] for r in range(m)) for j in range(nx)])
+            sL = mp.norm(L.T * xv) + mp.norm(mp.lu_solve(L, mp.matrix(g) - H * xv)) + mp.norm(mp.lu_solve(L, at_lam))
+            round_g = k1 * C * U * mp.sqrt(ev_hi) * sL
+            Linv_rows = [mp.norm(mp.lu_solve(L, mp.matrix(P.A[r]))) * k1 * C * U * sL for r in range(m)]
+        worst = mp.mpf(0)
+        for j in range(nx):
+            at = [P.A[r][j] * lm[r] for r in range(m)]
+            res = abs(g[j] + sum(at))
+            worst = max(worst, res / (k1 * C * U * (abs(g[j]) + sum(abs(t) for t in at)) + round_g + stop_g
+                                      + mp.mpf(10) ** -300))
+        for r in range(m):
+            terms = [P.A[r][j] * xm[j] for j in range(nx)]
+            row = sum(terms)
+            a1 = sum(abs(a) for a in P.A[r])
+            if r in W:
+                br = b[W.index(r)]
+                dev = abs(row - br)
+            else:
+                br = mp.mpf(0)
+                dev = max(P.lb[r] - row, row - P.ub[r], 0)
+            worst = max(worst, dev / (k1 * C * U * (sum(abs(t) for t in terms) + abs(br)) + Linv_rows[r] + a1 * stop_r
+                                      + mp.mpf(10) ** -300))
+    return float(worst)
