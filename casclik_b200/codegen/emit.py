@@ -339,11 +339,12 @@ def _switch(name, values, ret="int"):
 
 
 def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None,
-               nlp=None, nlp_tol=1e-10, vjp=False):
+               nlp=None, nlp_tol=1e-10, vjp=False, jvp=False):
     """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None; or `nlp`:
     NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).  `vjp`: also append the reverse-mode
     derivative kernel of the QP / NLP step (clik_vjp.cuh) after the multiplier kernel, for skills that have
-    one; everything emitted before it is the same text as with vjp=False.
+    one; everything emitted before it is the same text as with vjp=False.  `jvp`: likewise append the
+    forward-mode derivative and Jacobian kernels (clik_jvp.cuh), after the VJP kernel when both are asked for.
     Tuning knobs (also settable through the environment for experiments): CLIK_BLOCK,
     CLIK_MINBLOCKS, CLIK_CONSTBANK (1), CLIK_FAST_SINCOS (1)."""
     if block_threads is None:
@@ -351,7 +352,7 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     if nlp is not None:
         if pinv is not None or qp is not None:
             raise ValueError("an NLP image holds the NLP kernels only")
-        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp)
+        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp, jvp)
     env_min_blocks = int(os.environ.get("CLIK_MINBLOCKS", "0"))
     if min_blocks is None:
         min_blocks = env_min_blocks
@@ -737,11 +738,17 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     meta["vjp"] = bool(vjp) and meta["duals"]
     if meta["vjp"]:
         out.append(_VJP_MANIFEST % 1)
+    meta["jvp"] = bool(jvp) and meta["duals"]
+    if meta["jvp"]:
+        out.append(_JVP_MANIFEST % 1)
     out.append("}")
     if meta["duals"]:
         out += _emit_qp_duals(qp, sig, sincos_name, block_threads, meta["qp_structured"])
     if meta["vjp"]:
         out += _emit_vjp(qp, "qp", sig, sincos_name, block_threads,
+                         "SkillDuals" if meta["qp_structured"] else "Skill", meta["qp_read_masks"], meta)
+    if meta["jvp"]:
+        out += _emit_jvp(qp, "qp", sig, sincos_name, block_threads,
                          "SkillDuals" if meta["qp_structured"] else "Skill", meta["qp_read_masks"], meta)
     return "\n".join(out) + "\n", meta
 
@@ -824,6 +831,68 @@ def _emit_vjp(prog, kind, sig, sincos_name, block_threads, base, base_masks, met
     return out
 
 
+_JVP_MANIFEST = "  o[20] = %d;   // JVP and Jacobian kernels (1 QP, 2 NLP)"
+
+
+def _emit_jvp(prog, kind, sig, sincos_name, block_threads, base, base_masks, meta):
+    """clik_<kind>_jvp_kernel and clik_<kind>_jacobian_kernel (clik_jvp.cuh), appended last: a struct derived from
+    `base` adds eval_jvp and eval_jac, the tangent programs of codegen/jvp.py, and the rows the kernels load (those
+    of `base_masks` and those the two programs read).  Its constants are literals, so the constant bank of the step
+    kernels stays as it is."""
+    from .jvp import JacProgram, JvpProgram
+    n, m = prog.nx, prog.m
+    jp = JvpProgram(prog, kind)
+    em = Emitter(jp.names, None, sincos_name)
+    for arr, nodes in (("r1", jp.r1), ("r2u", jp.r2u), ("r2l", jp.r2l)):
+        for j, node in enumerate(nodes):
+            em.assign("%s[%d]" % (arr, j), node)
+    jc = JacProgram(prog, kind)
+    nt = jc.n_theta
+    emj = Emitter(jc.names, None, sincos_name)
+    for arr, rows in (("r1", jc.r1), ("r2u", jc.r2u), ("r2l", jc.r2l)):
+        for j, row in enumerate(rows):
+            for c, node in enumerate(row):
+                emj.assign("%s[%d]" % (arr, j * nt + c), node)
+    masks = tuple(a | b | c for a, b, c in zip(base_masks, em.read_masks(prog.syms), emj.read_masks(prog.syms)))
+    meta["jvp_eval"] = em.counts()
+    meta["jac_eval"] = emj.counts()
+    meta["jvp_read_masks"] = masks
+    nq, nxv, ny = max(prog.n_rob, 1), max(prog.n_virt, 1), max(prog.n_in, 1)
+    out = ["", "// ---- forward-mode derivative of the step's output (clik_jvp.cuh) ----",
+           '#include "clik_jvp.cuh"',
+           "struct SkillJvp : %s {" % base,
+           "  using Base = %s;   // the struct whose row evaluation the kernels call" % base,
+           "  static constexpr unsigned JVP_READ_T = %du, JVP_READ_Q = 0x%xu, JVP_READ_X = 0x%xu, JVP_READ_Y = 0x%xu;"
+           % masks,
+           "  __device__ static __forceinline__ void eval_jvp(%s," % sig,
+           "      const double (&xs_)[%d], const double (&lam_)[%d], const double td, const double (&qd_)[%d],"
+           % (n, m, nq),
+           "      const double (&xd_)[%d], const double (&yd_)[%d], double (&r1)[%d], double (&r2u)[%d],"
+           " double (&r2l)[%d]) {" % (nxv, ny, n, m, m)]
+    out += ["    " + ln for ln in em.finish()]
+    out += ["  }",
+            "  __device__ static __forceinline__ void eval_jac(%s," % sig,
+            "      const double (&xs_)[%d], const double (&lam_)[%d], double (&r1)[%d], double (&r2u)[%d],"
+            " double (&r2l)[%d]) {" % (n, m, n * nt, m * nt, m * nt)]
+    out += ["    " + ln for ln in emj.finish()]
+    out += ["  }",
+            "};",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_jvp_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,",
+            "    const double* y, const double* sol, const int* status, const unsigned* active, const double* t_dot,",
+            "    const double* q_dot, const double* x_dot, const double* y_dot, double* sol_dot) {",
+            "  clik::%s_jvp<SkillJvp>(N, ld, t, t_stride, q, x, y, sol, status, active, t_dot, q_dot, x_dot, y_dot,"
+            % kind,
+            "                         sol_dot);",
+            "}",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_jacobian_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, const double* t, int t_stride, const double* q, const double* x,",
+            "    const double* y, const double* sol, const int* status, const unsigned* active, double* jac) {",
+            "  clik::%s_jacobian<SkillJvp>(N, ld, t, t_stride, q, x, y, sol, status, active, jac);" % kind,
+            "}"]
+    return out
+
+
 def nlp_hoisted(nlp):
     """The maximal decision-free subexpressions the cost graph (F, g, H) consumes: every non-constant
     argument without a decision symbol below it of a node that has one, and every output without one.
@@ -848,7 +917,7 @@ def nlp_hoisted(nlp):
     return P
 
 
-def _emit_nlp(nlp, label, block_threads, tol, vjp=False):
+def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False):
     """Translation unit of the reactive-NLP controller (csrc/clik_nlp.cuh instantiated on the skill)."""
     const_table = [] if os.environ.get("CLIK_CONSTBANK", "1") == "1" else None
     sincos_name = "clik::sincos_fast" if os.environ.get("CLIK_FAST_SINCOS", "1") == "1" else "sincos"
@@ -950,6 +1019,9 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False):
     meta["vjp"] = bool(vjp) and meta["duals"]
     if meta["vjp"]:
         out.append(_VJP_MANIFEST % 2)
+    meta["jvp"] = bool(jvp) and meta["duals"]
+    if meta["jvp"]:
+        out.append(_JVP_MANIFEST % 2)
     out.append("}")
     if meta["duals"]:
         out += ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
@@ -961,6 +1033,8 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False):
                 "}"]
     if meta["vjp"]:
         out += _emit_vjp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
+    if meta["jvp"]:
+        out += _emit_jvp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
     return "\n".join(out) + "\n", meta
 
 

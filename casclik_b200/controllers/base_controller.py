@@ -146,17 +146,20 @@ def multipliers_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, s
     return lam
 
 
-def vjp_image(ctrl, kind, device):
-    """The skill's VJP image (emit_skill(..., vjp=True): the default image plus clik_<kind>_vjp_kernel) loaded on
-    `device`.  Built and loaded on the first call, cached like every cubin, one handle per device: a controller
-    that never asks for derivatives compiles nothing more."""
-    if ctrl._vjp is None:
-        source, meta = ctrl._vjp_source()
-        cubin, path = build.compile_cubin(source, tag="%s_vjp_%s" % (kind, ctrl.skill_spec.label))
-        ctrl._vjp = {"source": source, "meta": meta, "cubin": cubin, "path": path, "skills": {}}
-    skills = ctrl._vjp["skills"]
+def vjp_image(ctrl, kind, device, which="vjp"):
+    """The skill's derivative image `which` loaded on `device`: "vjp" (emit_skill(..., vjp=True): the default image
+    plus clik_<kind>_vjp_kernel, source ctrl._vjp_source()) or "jvp" (emit_skill(..., jvp=True): the default image
+    plus clik_<kind>_jvp_kernel and clik_<kind>_jacobian_kernel, source ctrl._jvp_source()).  Built and loaded on
+    the first call, cached like every cubin, one handle per device: a controller that never asks for derivatives
+    compiles nothing more."""
+    attr = "_" + which
+    if getattr(ctrl, attr) is None:
+        source, meta = getattr(ctrl, "_%s_source" % which)()
+        cubin, path = build.compile_cubin(source, tag="%s_%s_%s" % (kind, which, ctrl.skill_spec.label))
+        setattr(ctrl, attr, {"source": source, "meta": meta, "cubin": cubin, "path": path, "skills": {}})
+    skills = getattr(ctrl, attr)["skills"]
     if device not in skills:
-        skills[device] = runtime.CompiledSkill(ctrl._vjp["cubin"], ctrl._vjp["meta"],
+        skills[device] = runtime.CompiledSkill(getattr(ctrl, attr)["cubin"], getattr(ctrl, attr)["meta"],
                                                n_slack=ctrl.skill_spec.n_slack_var, device=device)
     return skills[device]
 
@@ -206,11 +209,90 @@ def vjp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, stat
     return tuple(out)
 
 
+def _step_outputs(ctrl, what, time_var, robot_var, virtual_var, input_var, sol, status, active):
+    """Validated Batch and device pointers of a step's inputs and (sol, status, active), as vjp_batch checks them."""
+    if ctrl._cubin is None:
+        raise RuntimeError("call setup_problem_functions() / setup_solver() before %s()" % what)
+    if not ctrl.kernel_meta.get("duals"):
+        raise ValueError("the %s needs at most 32 constraint rows and at least one (the skill has %d)"
+                         % ("Jacobian" if what == "jacobian_batch" else "JVP", ctrl._qm))
+    if not (runtime._is_torch(robot_var) and robot_var.is_cuda):
+        raise ValueError("%s needs torch CUDA tensors (there is no host-array form)" % what)
+    b = Batch(ctrl.skill_spec.n_robot_var, ctrl._nxv, ctrl._ny, time_var, robot_var, virtual_var,
+              input_var if ctrl._ny else None)
+    if sol is None or status is None or active is None:
+        raise ValueError("sol, status and active of the step are required")
+    if not all(runtime._is_torch(a) for a in (sol, status, active)):
+        raise ValueError("sol, status and active must be CUDA tensors")
+    ptrs = (runtime.dev_ptr(sol, "f64", ctrl._qn * b.N, "sol"), runtime.dev_ptr(status, "i32", b.N, "status"),
+            runtime.dev_ptr(active, "u32", 2 * b.N, "active"))
+    if any(a.device != b.device for a in (sol, status, active)):
+        raise ValueError("sol, status and active must live on %s like robot_var" % b.device)
+    return b, ptrs
+
+
+def jvp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot, q_dot, x_dot,
+              y_dot, out):
+    """Shared body of ReactiveQPController / ReactiveNLPController.jvp_batch (`kind` "qp" or "nlp"): validates the
+    step's inputs and outputs like vjp_batch and the tangent (None: zero; t_dot of N entries, or one broadcast to
+    every instance), and calls clik_<kind>_jvp on the current stream.  -> sol_dot (nx, N)."""
+    b, (solp, stp, acp) = _step_outputs(ctrl, "jvp_batch", time_var, robot_var, virtual_var, input_var, sol, status,
+                                        active)
+    tangents = []
+    for a, rows, name in ((t_dot, 0, "t_dot"), (q_dot, ctrl.skill_spec.n_robot_var, "q_dot"),
+                          (x_dot, ctrl._nxv, "x_dot"), (y_dot, ctrl._ny, "y_dot")):
+        if a is None or (rows == 0 and name != "t_dot"):
+            tangents.append(None)
+            continue
+        if not runtime._is_torch(a) or a.device != b.device:
+            raise ValueError("%s must be a CUDA tensor on %s like robot_var" % (name, b.device))
+        if name == "t_dot" and a.numel() == 1:
+            a = a.reshape(1).expand(b.N).contiguous()
+        elif a.dim() != (1 if rows == 0 else 2) or tuple(a.shape) != ((b.N,) if rows == 0 else (rows, b.N)):
+            raise ValueError("%s must have shape %s" % (name, (b.N,) if rows == 0 else (rows, b.N)))
+        tangents.append(a)
+    tptrs = [runtime.dev_ptr(a, "f64", (r or 1) * b.N, n) if a is not None else None
+             for a, r, n in zip(tangents, (0, ctrl.skill_spec.n_robot_var, ctrl._nxv, ctrl._ny),
+                                ("t_dot", "q_dot", "x_dot", "y_dot"))]
+    sd = b.empty(ctrl._qn) if out is None else out
+    sdp = b.out_ptr(sd, ctrl._qn, "f64", "out (sol_dot)")
+    skill = vjp_image(ctrl, kind, b.device_index, "jvp")
+    lib = runtime.load_library()
+    runtime.check(getattr(lib, "clik_%s_jvp" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp, solp, stp,
+                                                      acp, *tptrs, sdp, b.stream()))
+    return sd
+
+
+def n_theta(ctrl):
+    """Entries of theta = (t, q, x, y) of one instance: the columns of jacobian_batch."""
+    return 1 + ctrl.skill_spec.n_robot_var + ctrl._nxv + ctrl._ny
+
+
+def jacobian_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, out):
+    """Shared body of ReactiveQPController / ReactiveNLPController.jacobian_batch: validates like jvp_batch and
+    calls clik_<kind>_jacobian on the current stream.  -> jac (nx, n_theta, N), theta ordered (t, q, x, y)."""
+    b, (solp, stp, acp) = _step_outputs(ctrl, "jacobian_batch", time_var, robot_var, virtual_var, input_var, sol,
+                                        status, active)
+    nt = n_theta(ctrl)
+    if out is None:
+        jac = b.torch.empty((ctrl._qn, nt, b.N), dtype=b.torch.float64, device=b.device)
+    else:
+        jac = out
+        if not runtime._is_torch(jac) or tuple(jac.shape) != (ctrl._qn, nt, b.N):
+            raise runtime.ClikError("out (jac) must be a CUDA tensor of shape %s" % ((ctrl._qn, nt, b.N),))
+    jp = b.out_ptr(jac, ctrl._qn * nt, "f64", "out (jac)")
+    skill = vjp_image(ctrl, kind, b.device_index, "jvp")
+    lib = runtime.load_library()
+    runtime.check(getattr(lib, "clik_%s_jacobian" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp,
+                                                           solp, stp, acp, jp, b.stream()))
+    return jac
+
+
 _STEP_FUNCTION = []
 
 
 def _step_function():
-    """torch.autograd.Function of a controller step: forward solve_batch, backward vjp_batch."""
+    """torch.autograd.Function of a controller step: forward solve_batch, backward vjp_batch, jvp jvp_batch."""
     if _STEP_FUNCTION:
         return _STEP_FUNCTION[0]
     import torch
@@ -220,10 +302,24 @@ def _step_function():
         @staticmethod
         def forward(ctx, ctrl, t, q, x, y, warmstart, max_iter):
             outs = ctrl.solve_batch(t, q, x, y, warmstart=warmstart, max_iter=max_iter)
-            ctx.ctrl, ctx.t = ctrl, t
+            ctx.ctrl, ctx.t, ctx.n_outs = ctrl, t, len(outs)
             ctx.save_for_backward(q, x, y, *outs[:3])
+            ctx.save_for_forward(q, x, y, *outs[:3])
             ctx.mark_non_differentiable(*outs[1:])
             return outs
+
+        @staticmethod
+        def jvp(ctx, _ctrl, t_dot, q_dot, x_dot, y_dot, *unused):
+            # the warm start and max_iter carry no tangent; status / active / iterations get none
+            q, x, y, sol, status, active = ctx.saved_tensors
+            ctrl, t = ctx.ctrl, ctx.t
+            c = lambda a: None if a is None else a.contiguous()  # noqa: E731
+            if not torch.is_tensor(t):
+                t_dot = None
+            sol_dot = ctrl.jvp_batch(t, q, x, y, sol, status, active, t_dot=c(t_dot), q_dot=c(q_dot),
+                                     x_dot=c(x_dot) if x is not None else None,
+                                     y_dot=c(y_dot) if y is not None else None)
+            return (sol_dot,) + (None,) * (ctx.n_outs - 1)
 
         @staticmethod
         @once_differentiable

@@ -22,7 +22,7 @@ from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, solve_batch_differentiable, vjp_batch)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -56,6 +56,7 @@ class ReactiveNLPController(BaseController):
         self._cubin = None
         self._compiled = {}
         self._vjp = None
+        self._jvp = None
         self._has_initial = False
         self.res = None
         self._prog = self._program()     # validates the cost and the problem size now
@@ -130,6 +131,7 @@ class ReactiveNLPController(BaseController):
         self._cubin = cubin
         self._compiled = {}
         self._vjp = None
+        self._jvp = None
         if load:
             self._skill()
 
@@ -204,6 +206,21 @@ class ReactiveNLPController(BaseController):
         uses the Hessian of the cost at sol, factored without a shift: an instance whose Hessian is not positive
         definite there gets NaN (include/clik.h clik_nlp_vjp)."""
         return vjp_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out)
+
+    def _jvp_source(self):
+        """Source of the JVP image: the default image plus the JVP and Jacobian kernels."""
+        return emit_skill(nlp=self._prog, label=self.skill_spec.label, nlp_tol=float(self.options["tol"]), jvp=True)
+
+    def jvp_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot=None, q_dot=None,
+                  x_dot=None, y_dot=None, out=None):
+        """Forward-mode derivative of a solve_batch result, as ReactiveQPController.jvp_batch; the solve uses the
+        Hessian of the cost at sol, factored without a shift (include/clik.h clik_nlp_jvp)."""
+        return jvp_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot, q_dot,
+                         x_dot, y_dot, out)
+
+    def jacobian_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
+        """The full step Jacobian (nx, n_theta, N) of a solve_batch result, as ReactiveQPController.jacobian_batch."""
+        return jacobian_batch(self, "nlp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
 
     def solve_batch_differentiable(self, time_var, robot_var, virtual_var=None, input_var=None, warmstart=None,
                                    max_iter=None):

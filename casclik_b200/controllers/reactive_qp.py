@@ -23,7 +23,7 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              set_overlap, solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, set_overlap, solve_batch_differentiable, vjp_batch)
 from .qp_solver import ConicSolver
 
 
@@ -70,6 +70,7 @@ class ReactiveQPController(BaseController):
         self._compiled = {}
         self._cubin = None
         self._vjp = None
+        self._jvp = None
         self._has_initial = False
         self.res = None
 
@@ -202,6 +203,7 @@ class ReactiveQPController(BaseController):
         self._cubin = cubin
         self._compiled = {}
         self._vjp = None
+        self._jvp = None
         ins, names = self._input_list()
         H = cs.diag(cs.MX(cs.vertcat(*prog.h)))
         A = cs.MX(cs.vertcat(*[cs.horzcat(*row) for row in prog.A]))
@@ -314,6 +316,32 @@ class ReactiveQPController(BaseController):
         buffers of those shapes.  The VJP image is compiled and loaded on the first call (one per device).
         NumPy inputs and skills with more than 32 constraint rows raise ValueError."""
         return vjp_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, sol_bar, out)
+
+    def _jvp_source(self):
+        """Source of the JVP image: the default image's emission (same fast-kernel register cap) plus the JVP and
+        Jacobian kernels."""
+        return emit_skill(qp=self._program(), label=self.skill_spec.label, jvp=True,
+                          qp_fast_min_blocks=self.kernel_meta.get("qp_fast_min_blocks"))
+
+    def jvp_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot=None, q_dot=None,
+                  x_dot=None, y_dot=None, out=None):
+        """Forward-mode derivative (Jacobian-vector product) of a solve_batch result: the step's inputs and its
+        (sol, status, active) as torch CUDA tensors, and the tangent (t_dot (N,) or one entry for every instance,
+        q_dot (n_robot, N), x_dot (n_virtual, N), y_dot (n_input, N); None is a zero tangent), float64.  Runs on the
+        current stream and returns sol_dot (nx, N) = (d sol / d theta) theta_dot for the face problem of the
+        returned working set, the exact adjoint of vjp_batch (DESIGN.md §4.7).  An all-zero tangent gives exactly 0;
+        otherwise an unsolved instance or a rank-deficient working set gives NaN (include/clik.h clik_qp_jvp).
+        out= a (nx, N) buffer.  The JVP image is compiled and loaded on the first call (one per device).  NumPy
+        inputs and skills with more than 32 constraint rows raise ValueError."""
+        return jvp_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot, q_dot,
+                         x_dot, y_dot, out)
+
+    def jacobian_batch(self, time_var, robot_var, virtual_var, input_var, sol, status, active, out=None):
+        """The full step Jacobian of a solve_batch result: (nx, n_theta, N) float64 on the inputs' device, column c
+        the derivative along entry c of theta = (t, q, x, y) (n_theta = 1 + n_robot + n_virtual + n_input), one
+        factorisation per instance.  The rules of jvp_batch per column: an unsolved or rejected instance gets NaN
+        everywhere (include/clik.h clik_qp_jacobian).  out= a buffer of that shape."""
+        return jacobian_batch(self, "qp", time_var, robot_var, virtual_var, input_var, sol, status, active, out)
 
     def solve_batch_differentiable(self, time_var, robot_var, virtual_var=None, input_var=None, warmstart=None,
                                    max_iter=None):

@@ -94,6 +94,7 @@ struct clik_skill {
   KernelInfo nlp, nlp_rollout;   // NLP images (manifest flag 256)
   KernelInfo qp_duals, nlp_duals;   // constraint multipliers (manifest o[18]: bit 0 QP, bit 1 NLP; at most 32 rows)
   KernelInfo qp_vjp, nlp_vjp;       // reverse-mode derivative of the step (manifest o[19]: bit 0 QP, bit 1 NLP)
+  KernelInfo qp_jvp, nlp_jvp, qp_jac, nlp_jac;   // forward-mode derivative and Jacobian (o[20]: bit 0 QP, bit 1 NLP)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
@@ -522,6 +523,11 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
   const int vjp = hsz[19];     // VJP kernels (images built with emit_skill(..., vjp=True)): bit 0 QP, bit 1 NLP
   if (st == CLIK_OK && (vjp & 1)) st = setup_kernel(s, "clik_qp_vjp_kernel", &s->qp_vjp);
   if (st == CLIK_OK && (vjp & 2)) st = setup_kernel(s, "clik_nlp_vjp_kernel", &s->nlp_vjp);
+  const int jvp = hsz[20];     // JVP + Jacobian kernels (emit_skill(..., jvp=True)): bit 0 QP, bit 1 NLP
+  if (st == CLIK_OK && (jvp & 1)) st = setup_kernel(s, "clik_qp_jvp_kernel", &s->qp_jvp);
+  if (st == CLIK_OK && (jvp & 1)) st = setup_kernel(s, "clik_qp_jacobian_kernel", &s->qp_jac);
+  if (st == CLIK_OK && (jvp & 2)) st = setup_kernel(s, "clik_nlp_jvp_kernel", &s->nlp_jvp);
+  if (st == CLIK_OK && (jvp & 2)) st = setup_kernel(s, "clik_nlp_jacobian_kernel", &s->nlp_jac);
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
     delete s;
@@ -1253,6 +1259,86 @@ clik_status clik_nlp_vjp(const clik_skill* s, int64_t N, const double* t, int32_
                          const uint32_t* active, const double* sol_bar, double* t_bar, double* q_bar, double* x_bar,
                          double* y_bar, void* stream) {
   return vjp_impl(s, true, N, t, t_stride, q, x, y, sol, status, active, sol_bar, t_bar, q_bar, x_bar, y_bar, stream);
+}
+
+}  // extern "C"
+
+// ---- forward-mode derivative and Jacobian of a step's output (clik_jvp.cuh) --------------------------------
+namespace {
+
+clik_status jvp_check(const clik_skill* s, const KernelInfo& k, const char* what, bool nlp, int64_t N,
+                      const double* t, const double* q, const double* x, const double* y, const double* sol,
+                      const int32_t* status, const uint32_t* active) {
+  if (!k.kernel)
+    return fail(CLIK_ERR_INVALID, "skill image has no %s %s kernel (build it with emit_skill(..., jvp=True); at most "
+                "32 constraint rows)", nlp ? "NLP" : "QP", what);
+  clik_status st = check_common(s, N, t, q, x, y);
+  if (st != CLIK_OK) return st;
+  if (N > 0 && (!sol || !status || !active)) return fail(CLIK_ERR_INVALID, "sol, status and active are required");
+  return CLIK_OK;
+}
+
+clik_status jvp_impl(const clik_skill* s, bool nlp, int64_t N, const double* t, int32_t t_stride, const double* q,
+                     const double* x, const double* y, const double* sol, const int32_t* status,
+                     const uint32_t* active, const double* t_dot, const double* q_dot, const double* x_dot,
+                     const double* y_dot, double* sol_dot, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_jvp : s->qp_jvp;
+  clik_status st = jvp_check(s, k, "JVP", nlp, N, t, q, x, y, sol, status, active);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!sol_dot) return fail(CLIK_ERR_INVALID, "sol_dot is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0;
+  void* args[] = {&n, &l, &t, &ts, &q, &x, &y, &sol, &status, &active, &t_dot, &q_dot, &x_dot, &y_dot, &sol_dot};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+clik_status jacobian_impl(const clik_skill* s, bool nlp, int64_t N, const double* t, int32_t t_stride,
+                          const double* q, const double* x, const double* y, const double* sol,
+                          const int32_t* status, const uint32_t* active, double* jac, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_jac : s->qp_jac;
+  clik_status st = jvp_check(s, k, "Jacobian", nlp, N, t, q, x, y, sol, status, active);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!jac) return fail(CLIK_ERR_INVALID, "jac is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0;
+  void* args[] = {&n, &l, &t, &ts, &q, &x, &y, &sol, &status, &active, &jac};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_qp_jvp(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                        const double* x, const double* y, const double* sol, const int32_t* status,
+                        const uint32_t* active, const double* t_dot, const double* q_dot, const double* x_dot,
+                        const double* y_dot, double* sol_dot, void* stream) {
+  return jvp_impl(s, false, N, t, t_stride, q, x, y, sol, status, active, t_dot, q_dot, x_dot, y_dot, sol_dot, stream);
+}
+
+clik_status clik_nlp_jvp(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                         const double* x, const double* y, const double* sol, const int32_t* status,
+                         const uint32_t* active, const double* t_dot, const double* q_dot, const double* x_dot,
+                         const double* y_dot, double* sol_dot, void* stream) {
+  return jvp_impl(s, true, N, t, t_stride, q, x, y, sol, status, active, t_dot, q_dot, x_dot, y_dot, sol_dot, stream);
+}
+
+clik_status clik_qp_jacobian(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                             const double* x, const double* y, const double* sol, const int32_t* status,
+                             const uint32_t* active, double* jac, void* stream) {
+  return jacobian_impl(s, false, N, t, t_stride, q, x, y, sol, status, active, jac, stream);
+}
+
+clik_status clik_nlp_jacobian(const clik_skill* s, int64_t N, const double* t, int32_t t_stride, const double* q,
+                              const double* x, const double* y, const double* sol, const int32_t* status,
+                              const uint32_t* active, double* jac, void* stream) {
+  return jacobian_impl(s, true, N, t, t_stride, q, x, y, sol, status, active, jac, stream);
 }
 
 clik_status clik_measure_fp64_peak(int32_t device, int32_t iters, double* tflops) {

@@ -300,6 +300,47 @@ clik_status clik_nlp_vjp(const clik_skill* skill, int64_t N, const double* t, in
                          const int32_t* status, const uint32_t* active, const double* sol_bar, double* t_bar,
                          double* q_bar, double* x_bar, double* y_bar, void* stream);
 
+/* Forward-mode derivative (Jacobian-vector product) of a step's output, for N instances: the same face problem as
+ * clik_qp_vjp / clik_nlp_vjp, read forwards.  For the tangent theta_dot of instance i, with x* and lam fixed,
+ *   rho1 = d_theta (g(x*, theta) + A(theta)' lam) . theta_dot,   rho2_r = d_theta (A_r x* - b_r) . theta_dot (r in W)
+ * (b_r = ub_r for an upper bit, lb_r for a lower bit; an equality row has both bits and uses ub_r), and
+ *   [[M, A_W'], [A_W, 0]] [x_dot; lam_dot_W] = -[rho1; rho2_W]
+ * gives sol_dot[:, i] = x_dot = (d(x*)/d(theta)) theta_dot, the exact adjoint of the VJP (one-sided where a row
+ * of W has lam = 0).  The solve reuses the VJP's factorisation B = D^1/2 A_W' = Q R (QP D = H^-1; NLP
+ * grad^2 F(x*) = L L', no shift, B = L^-1 A_W'): w = -R^-T rho2_W, z = (I - Q Q') c + Q w with c = -D^1/2 rho1
+ * (NLP -L^-1 rho1), x_dot = D^1/2 z (NLP L^-T z).
+ *   inputs:  t, q, x, y, sol, status, active as clik_qp_vjp; the tangent t_dot [N] (per instance, also when
+ *            t_stride = 0), q_dot [n_robot * N], x_dot [n_virtual * N], y_dot [n_input * N]; a NULL tangent
+ *            array is a zero tangent
+ *   output:  sol_dot [qp_n * N]
+ * Rules, as the VJP's: an instance whose tangent is all zeros gets exactly 0, whatever its status; otherwise
+ * every output of the instance is NaN when status[i] is not 0, when A_W is rank-deficient or, for the NLP, when a
+ * Cholesky pivot of grad^2 F(x*) is at or below 1e-12 max(1, max_j |H_jj|).
+ * The kernels are in images built with emit_skill(..., jvp=True) (manifest o[20]) only, and only for skills with
+ * 1..32 constraint rows: other images, and a NULL skill, fail with CLIK_ERR_INVALID.  Device pointers only, row
+ * stride N, asynchronous on `stream`; one thread per instance. */
+clik_status clik_qp_jvp(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                        const double* q, const double* x, const double* y, const double* sol,
+                        const int32_t* status, const uint32_t* active, const double* t_dot, const double* q_dot,
+                        const double* x_dot, const double* y_dot, double* sol_dot, void* stream);
+clik_status clik_nlp_jvp(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                         const double* q, const double* x, const double* y, const double* sol,
+                         const int32_t* status, const uint32_t* active, const double* t_dot, const double* q_dot,
+                         const double* x_dot, const double* y_dot, double* sol_dot, void* stream);
+
+/* The full step Jacobian d(x*)/d(theta) of N instances, theta ordered (t, q, x, y) as the VJP's outputs are
+ * stacked, n_theta = 1 + n_robot + n_virtual + n_input: entry (j, c) of instance i at jac[(j * n_theta + c) * N + i]
+ * (qp_n * n_theta * N doubles).  One factorisation per instance and n_theta right-hand sides of the JVP's solve;
+ * the JVP's rules per column: an unsolved or rejected instance gets a block that is NaN everywhere, a solved one
+ * exact zeros in the columns of theta entries its program does not read.  Same images, errors and launch rules as
+ * clik_qp_jvp / clik_nlp_jvp. */
+clik_status clik_qp_jacobian(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                             const double* q, const double* x, const double* y, const double* sol,
+                             const int32_t* status, const uint32_t* active, double* jac, void* stream);
+clik_status clik_nlp_jacobian(const clik_skill* skill, int64_t N, const double* t, int32_t t_stride,
+                              const double* q, const double* x, const double* y, const double* sol,
+                              const int32_t* status, const uint32_t* active, double* jac, void* stream);
+
 /* One host batch over several GPUs of the box: `skills[k]` is the same cubin loaded on device k
  * (clik_skill_load with desc.device = k); the batch is cut into n_skills contiguous shards (sizes differ
  * by at most one, shard k = [k*N/n .. )), each shard runs on its device from its own host thread (zero
