@@ -339,12 +339,14 @@ def _switch(name, values, ret="int"):
 
 
 def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None,
-               nlp=None, nlp_tol=1e-10, vjp=False, jvp=False):
+               nlp=None, nlp_tol=1e-10, vjp=False, jvp=False, rollout_jvp=False):
     """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None; or `nlp`:
     NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).  `vjp`: also append the reverse-mode
     derivative kernel of the QP / NLP step (clik_vjp.cuh) after the multiplier kernel, for skills that have
     one; everything emitted before it is the same text as with vjp=False.  `jvp`: likewise append the
     forward-mode derivative and Jacobian kernels (clik_jvp.cuh), after the VJP kernel when both are asked for.
+    `rollout_jvp` (with `jvp`): then also the tangent and Jacobian rollouts (clik_jvp.cuh), for skills with a
+    rollout kernel.
     Tuning knobs (also settable through the environment for experiments): CLIK_BLOCK,
     CLIK_MINBLOCKS, CLIK_CONSTBANK (1), CLIK_FAST_SINCOS (1)."""
     if block_threads is None:
@@ -352,7 +354,7 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     if nlp is not None:
         if pinv is not None or qp is not None:
             raise ValueError("an NLP image holds the NLP kernels only")
-        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp, jvp)
+        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp, jvp, rollout_jvp)
     env_min_blocks = int(os.environ.get("CLIK_MINBLOCKS", "0"))
     if min_blocks is None:
         min_blocks = env_min_blocks
@@ -741,6 +743,9 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     meta["jvp"] = bool(jvp) and meta["duals"]
     if meta["jvp"]:
         out.append(_JVP_MANIFEST % 1)
+    meta["rollout_jvp"] = bool(rollout_jvp) and meta["jvp"] and qp_rollout
+    if meta["rollout_jvp"]:
+        out.append(_ROLLOUT_JVP_MANIFEST % 1)
     out.append("}")
     if meta["duals"]:
         out += _emit_qp_duals(qp, sig, sincos_name, block_threads, meta["qp_structured"])
@@ -750,6 +755,8 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     if meta["jvp"]:
         out += _emit_jvp(qp, "qp", sig, sincos_name, block_threads,
                          "SkillDuals" if meta["qp_structured"] else "Skill", meta["qp_read_masks"], meta)
+    if meta["rollout_jvp"]:
+        out += _emit_rollout_jvp("qp", block_threads)
     return "\n".join(out) + "\n", meta
 
 
@@ -893,6 +900,33 @@ def _emit_jvp(prog, kind, sig, sincos_name, block_threads, base, base_masks, met
     return out
 
 
+_ROLLOUT_JVP_MANIFEST = "  o[21] = %d;   // tangent and Jacobian rollout kernels (1 QP, 2 NLP)"
+
+
+def _emit_rollout_jvp(kind, block_threads):
+    """clik_<kind>_rollout_jvp_kernel and clik_<kind>_rollout_jacobian_kernel (clik_jvp.cuh), appended after the JVP
+    section: the rollout of clik_<kind>_rollout_kernel on the step skill `Skill`, differentiated with the face solve
+    of `SkillJvp`."""
+    return ["", "// ---- forward-mode derivative of the closed-loop rollout ----",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_rollout_jvp_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, int steps, double dt, const double* t0, int t_stride, double* q, double* x,",
+            "    const double* y, double vmax_q, double vmax_x, double* sol_last, int* n_failed, int max_iter,",
+            "    const double* t_dot, const double* q_dot, const double* x_dot, const double* y_dot, double* q_dot_out,",
+            "    double* x_dot_out, double* sol_dot) {",
+            "  clik::%s_rollout_jvp<SkillJvp, Skill>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,"
+            % kind,
+            "      n_failed, max_iter, t_dot, q_dot, x_dot, y_dot, q_dot_out, x_dot_out, sol_dot);",
+            "}",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_rollout_jacobian_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, int steps, double dt, const double* t0, int t_stride, double* q, double* x,",
+            "    const double* y, double vmax_q, double vmax_x, double* sol_last, int* n_failed, int max_iter,",
+            "    double* jac) {",
+            "  clik::%s_rollout_jacobian<SkillJvp, Skill>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x,"
+            % kind,
+            "      sol_last, n_failed, max_iter, jac);",
+            "}"]
+
+
 def nlp_hoisted(nlp):
     """The maximal decision-free subexpressions the cost graph (F, g, H) consumes: every non-constant
     argument without a decision symbol below it of a node that has one, and every output without one.
@@ -917,7 +951,7 @@ def nlp_hoisted(nlp):
     return P
 
 
-def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False):
+def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False, rollout_jvp=False):
     """Translation unit of the reactive-NLP controller (csrc/clik_nlp.cuh instantiated on the skill)."""
     const_table = [] if os.environ.get("CLIK_CONSTBANK", "1") == "1" else None
     sincos_name = "clik::sincos_fast" if os.environ.get("CLIK_FAST_SINCOS", "1") == "1" else "sincos"
@@ -1022,6 +1056,9 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False):
     meta["jvp"] = bool(jvp) and meta["duals"]
     if meta["jvp"]:
         out.append(_JVP_MANIFEST % 2)
+    meta["rollout_jvp"] = bool(rollout_jvp) and meta["jvp"]
+    if meta["rollout_jvp"]:
+        out.append(_ROLLOUT_JVP_MANIFEST % 2)
     out.append("}")
     if meta["duals"]:
         out += ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
@@ -1035,6 +1072,8 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False):
         out += _emit_vjp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
     if meta["jvp"]:
         out += _emit_jvp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
+    if meta["rollout_jvp"]:
+        out += _emit_rollout_jvp("nlp", block_threads)
     return "\n".join(out) + "\n", meta
 
 

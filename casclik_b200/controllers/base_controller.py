@@ -148,8 +148,10 @@ def multipliers_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, s
 
 def vjp_image(ctrl, kind, device, which="vjp"):
     """The skill's derivative image `which` loaded on `device`: "vjp" (emit_skill(..., vjp=True): the default image
-    plus clik_<kind>_vjp_kernel, source ctrl._vjp_source()) or "jvp" (emit_skill(..., jvp=True): the default image
-    plus clik_<kind>_jvp_kernel and clik_<kind>_jacobian_kernel, source ctrl._jvp_source()).  Built and loaded on
+    plus clik_<kind>_vjp_kernel, source ctrl._vjp_source()), "jvp" (emit_skill(..., jvp=True): the default image
+    plus clik_<kind>_jvp_kernel and clik_<kind>_jacobian_kernel, source ctrl._jvp_source()) or "rollout_jvp"
+    (emit_skill(..., jvp=True, rollout_jvp=True): the JVP image plus clik_<kind>_rollout_jvp_kernel and
+    clik_<kind>_rollout_jacobian_kernel, source ctrl._rollout_jvp_source()).  Built and loaded on
     the first call, cached like every cubin, one handle per device: a controller that never asks for derivatives
     compiles nothing more."""
     attr = "_" + which
@@ -231,13 +233,9 @@ def _step_outputs(ctrl, what, time_var, robot_var, virtual_var, input_var, sol, 
     return b, ptrs
 
 
-def jvp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot, q_dot, x_dot,
-              y_dot, out):
-    """Shared body of ReactiveQPController / ReactiveNLPController.jvp_batch (`kind` "qp" or "nlp"): validates the
-    step's inputs and outputs like vjp_batch and the tangent (None: zero; t_dot of N entries, or one broadcast to
-    every instance), and calls clik_<kind>_jvp on the current stream.  -> sol_dot (nx, N)."""
-    b, (solp, stp, acp) = _step_outputs(ctrl, "jvp_batch", time_var, robot_var, virtual_var, input_var, sol, status,
-                                        active)
+def _tangent_ptrs(ctrl, b, t_dot, q_dot, x_dot, y_dot):
+    """Validated device pointers of a tangent (t_dot, q_dot, x_dot, y_dot) of the Batch `b`: None is a zero tangent,
+    t_dot has N entries or one broadcast to every instance."""
     tangents = []
     for a, rows, name in ((t_dot, 0, "t_dot"), (q_dot, ctrl.skill_spec.n_robot_var, "q_dot"),
                           (x_dot, ctrl._nxv, "x_dot"), (y_dot, ctrl._ny, "y_dot")):
@@ -251,9 +249,20 @@ def jvp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, stat
         elif a.dim() != (1 if rows == 0 else 2) or tuple(a.shape) != ((b.N,) if rows == 0 else (rows, b.N)):
             raise ValueError("%s must have shape %s" % (name, (b.N,) if rows == 0 else (rows, b.N)))
         tangents.append(a)
-    tptrs = [runtime.dev_ptr(a, "f64", (r or 1) * b.N, n) if a is not None else None
-             for a, r, n in zip(tangents, (0, ctrl.skill_spec.n_robot_var, ctrl._nxv, ctrl._ny),
-                                ("t_dot", "q_dot", "x_dot", "y_dot"))]
+    b.keep = b.keep + tuple(tangents)      # (a broadcast t_dot lives until the launch)
+    return [runtime.dev_ptr(a, "f64", (r or 1) * b.N, n) if a is not None else None
+            for a, r, n in zip(tangents, (0, ctrl.skill_spec.n_robot_var, ctrl._nxv, ctrl._ny),
+                               ("t_dot", "q_dot", "x_dot", "y_dot"))]
+
+
+def jvp_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol, status, active, t_dot, q_dot, x_dot,
+              y_dot, out):
+    """Shared body of ReactiveQPController / ReactiveNLPController.jvp_batch (`kind` "qp" or "nlp"): validates the
+    step's inputs and outputs like vjp_batch and the tangent (None: zero; t_dot of N entries, or one broadcast to
+    every instance), and calls clik_<kind>_jvp on the current stream.  -> sol_dot (nx, N)."""
+    b, (solp, stp, acp) = _step_outputs(ctrl, "jvp_batch", time_var, robot_var, virtual_var, input_var, sol, status,
+                                        active)
+    tptrs = _tangent_ptrs(ctrl, b, t_dot, q_dot, x_dot, y_dot)
     sd = b.empty(ctrl._qn) if out is None else out
     sdp = b.out_ptr(sd, ctrl._qn, "f64", "out (sol_dot)")
     skill = vjp_image(ctrl, kind, b.device_index, "jvp")
@@ -286,6 +295,61 @@ def jacobian_batch(ctrl, kind, time_var, robot_var, virtual_var, input_var, sol,
     runtime.check(getattr(lib, "clik_%s_jacobian" % kind)(skill.handle, b.N, b.tp, b.t_stride, b.qp, b.xp, b.yp,
                                                            solp, stp, acp, jp, b.stream()))
     return jac
+
+
+def _rollout_batch(ctrl, what, time_var0, robot_var, virtual_var, input_var):
+    """Validated Batch of a tangent / Jacobian rollout: the checks of rollout_batch and of jvp_batch, all before any
+    image is built."""
+    if ctrl._cubin is None:
+        raise RuntimeError("call setup_problem_functions() / setup_solver() before %s()" % what)
+    if not ctrl.kernel_meta.get("duals"):
+        raise ValueError("the %s needs at most 32 constraint rows and at least one (the skill has %d)" % (what, ctrl._qm))
+    if not (runtime._is_torch(robot_var) and robot_var.is_cuda):
+        raise ValueError("%s needs torch CUDA tensors (state is updated in place on the device)" % what)
+    if ctrl._nxv and virtual_var is None:
+        raise ValueError("the skill has a virtual_var: pass its initial value")
+    return Batch(ctrl.skill_spec.n_robot_var, ctrl._nxv, ctrl._ny, time_var0, robot_var, virtual_var,
+                 input_var if ctrl._ny else None)
+
+
+def _speeds(max_speed, max_virtual_speed):
+    inf = float("inf")
+    return (ctypes.c_double(inf if max_speed is None else float(max_speed)),
+            ctypes.c_double(inf if max_virtual_speed is None else float(max_virtual_speed)))
+
+
+def rollout_jvp(ctrl, kind, time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed, max_virtual_speed,
+                max_iter, t_dot, q_dot, x_dot, y_dot):
+    """Shared body of ReactiveQPController / ReactiveNLPController.rollout_jvp: the rollout of rollout_batch (state
+    updated in place) with the tangent of its state carried along, clik_<kind>_rollout_jvp on the current stream.
+    -> {"sol", "n_failed", "q_dot", "x_dot", "sol_dot"}."""
+    b = _rollout_batch(ctrl, "rollout_jvp", time_var0, robot_var, virtual_var, input_var)
+    tptrs = _tangent_ptrs(ctrl, b, t_dot, q_dot, x_dot, y_dot)
+    sol, failed, sd = b.empty(ctrl._qn), b.empty(0, "i32"), b.empty(ctrl._qn)
+    qd = b.empty(ctrl.skill_spec.n_robot_var)
+    xd = b.empty(ctrl._nxv) if ctrl._nxv else None
+    skill = vjp_image(ctrl, kind, b.device_index, "rollout_jvp")
+    runtime.check(getattr(runtime.load_library(), "clik_%s_rollout_jvp" % kind)(
+        skill.handle, b.N, int(steps), ctypes.c_double(float(dt)), b.tp, b.t_stride, b.qp, b.xp, b.yp,
+        *_speeds(max_speed, max_virtual_speed), b.ptr(sol), b.ptr(failed), max_iter, *tptrs, b.ptr(qd), b.ptr(xd),
+        b.ptr(sd), b.stream()))
+    return {"sol": sol, "n_failed": failed, "q_dot": qd, "x_dot": xd, "sol_dot": sd}
+
+
+def rollout_jacobian(ctrl, kind, time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                     max_virtual_speed, max_iter):
+    """Shared body of ReactiveQPController / ReactiveNLPController.rollout_jacobian: the rollout of rollout_batch
+    with d(q_K, x_K)/d(t0, q0, x0, y) carried along, clik_<kind>_rollout_jacobian on the current stream.
+    -> {"sol", "n_failed", "jac" (n_robot + n_virtual, n_theta, N)}."""
+    b = _rollout_batch(ctrl, "rollout_jacobian", time_var0, robot_var, virtual_var, input_var)
+    sol, failed = b.empty(ctrl._qn), b.empty(0, "i32")
+    jac = b.torch.empty((ctrl.skill_spec.n_robot_var + ctrl._nxv, n_theta(ctrl), b.N), dtype=b.torch.float64,
+                        device=b.device)
+    skill = vjp_image(ctrl, kind, b.device_index, "rollout_jvp")
+    runtime.check(getattr(runtime.load_library(), "clik_%s_rollout_jacobian" % kind)(
+        skill.handle, b.N, int(steps), ctypes.c_double(float(dt)), b.tp, b.t_stride, b.qp, b.xp, b.yp,
+        *_speeds(max_speed, max_virtual_speed), b.ptr(sol), b.ptr(failed), max_iter, b.ptr(jac), b.stream()))
+    return {"sol": sol, "n_failed": failed, "jac": jac}
 
 
 _STEP_FUNCTION = []

@@ -22,7 +22,7 @@ from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              jacobian_batch, jvp_batch, solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, rollout_jacobian, rollout_jvp, solve_batch_differentiable, vjp_batch)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -57,6 +57,7 @@ class ReactiveNLPController(BaseController):
         self._compiled = {}
         self._vjp = None
         self._jvp = None
+        self._rollout_jvp = None
         self._has_initial = False
         self.res = None
         self._prog = self._program()     # validates the cost and the problem size now
@@ -132,6 +133,7 @@ class ReactiveNLPController(BaseController):
         self._compiled = {}
         self._vjp = None
         self._jvp = None
+        self._rollout_jvp = None
         if load:
             self._skill()
 
@@ -250,6 +252,25 @@ class ReactiveNLPController(BaseController):
             ctypes.c_double(inf if max_virtual_speed is None else float(max_virtual_speed)),
             b.ptr(sol), b.ptr(failed), self._max_iter(max_iter), b.stream()))
         return {"sol": sol, "n_failed": failed}
+
+    def _rollout_jvp_source(self):
+        """Source of the rollout-JVP image: the JVP image plus the tangent and Jacobian rollout kernels."""
+        return emit_skill(nlp=self._prog, label=self.skill_spec.label, nlp_tol=float(self.options["tol"]), jvp=True,
+                          rollout_jvp=True)
+
+    def rollout_jvp(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                    max_virtual_speed=None, max_iter=None, t_dot=None, q_dot=None, x_dot=None, y_dot=None):
+        """rollout_batch with the tangent of the closed loop, as ReactiveQPController.rollout_jvp; each step's
+        tangent is the jvp_batch tangent of its solution (Hessian at sol, no shift: NaN where it is not positive
+        definite).  The dependence of a step on its warm start (below tol) is not differentiated."""
+        return rollout_jvp(self, "nlp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                           max_virtual_speed, self._max_iter(max_iter), t_dot, q_dot, x_dot, y_dot)
+
+    def rollout_jacobian(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                         max_virtual_speed=None, max_iter=None):
+        """rollout_batch with d(q_K, x_K)/d(t0, q0, x0, y), as ReactiveQPController.rollout_jacobian."""
+        return rollout_jacobian(self, "nlp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                                max_virtual_speed, self._max_iter(max_iter))
 
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None, warmstart_slack_var=None):

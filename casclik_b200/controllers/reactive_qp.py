@@ -23,7 +23,7 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              jacobian_batch, jvp_batch, set_overlap, solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, rollout_jacobian, rollout_jvp, set_overlap, solve_batch_differentiable, vjp_batch)
 from .qp_solver import ConicSolver
 
 
@@ -71,6 +71,7 @@ class ReactiveQPController(BaseController):
         self._cubin = None
         self._vjp = None
         self._jvp = None
+        self._rollout_jvp = None
         self._has_initial = False
         self.res = None
 
@@ -204,6 +205,7 @@ class ReactiveQPController(BaseController):
         self._compiled = {}
         self._vjp = None
         self._jvp = None
+        self._rollout_jvp = None
         ins, names = self._input_list()
         H = cs.diag(cs.MX(cs.vertcat(*prog.h)))
         A = cs.MX(cs.vertcat(*[cs.horzcat(*row) for row in prog.A]))
@@ -373,6 +375,37 @@ class ReactiveQPController(BaseController):
             ctypes.c_double(inf if max_virtual_speed is None else float(max_virtual_speed)),
             b.ptr(sol), b.ptr(failed), mi, b.stream()))
         return {"sol": sol, "n_failed": failed}
+
+    def _rollout_jvp_source(self):
+        """Source of the rollout-JVP image: the JVP image plus the tangent and Jacobian rollout kernels."""
+        return emit_skill(qp=self._program(), label=self.skill_spec.label, jvp=True, rollout_jvp=True,
+                          qp_fast_min_blocks=self.kernel_meta.get("qp_fast_min_blocks"))
+
+    def rollout_jvp(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                    max_virtual_speed=None, max_iter=None, t_dot=None, q_dot=None, x_dot=None, y_dot=None):
+        """rollout_batch (robot_var / virtual_var UPDATED IN PLACE, bit for bit the same states, `sol` and `n_failed`)
+        with the tangent of the closed loop carried along in one kernel: the inputs p = (t0, q0, x0, y) move along
+        (t_dot (N,) or one entry for every instance, q_dot (n_robot, N), x_dot (n_virtual, N), y_dot (n_input, N);
+        None is a zero tangent; none is modified).  Every step takes the jvp_batch tangent of its solution on its
+        own working set, keeps the entries the clip max_speed / max_virtual_speed does not hold (|sol_j| < max) and
+        integrates them like the state (DESIGN.md §4.8).  Returns {"sol", "n_failed", "q_dot" (n_robot, N), "x_dot"
+        (n_virtual, N) | None, "sol_dot" (nx, N)}: the tangents of the final state and of `sol`.  An instance whose
+        tangent hits a step with status != 0, a rank-deficient working set gets NaN from that step on; an all-zero
+        tangent stays exactly 0.  The image is compiled and loaded on the first call (one per device).  NumPy
+        inputs and skills with more than 32 constraint rows raise ValueError."""
+        mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
+        return rollout_jvp(self, "qp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                           max_virtual_speed, mi, t_dot, q_dot, x_dot, y_dot)
+
+    def rollout_jacobian(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                         max_virtual_speed=None, max_iter=None):
+        """rollout_batch (state UPDATED IN PLACE, the same bits) with the Jacobian of the final state carried along:
+        {"sol", "n_failed", "jac"}, jac (n_robot + n_virtual, n_theta, N) = d(q_K, x_K)/d(t0, q0, x0, y), column c
+        the rollout_jvp tangent along the unit tangent e_c, computed with one factorisation per step; the rules of
+        rollout_jvp per instance (a NaN block)."""
+        mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
+        return rollout_jacobian(self, "qp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                                max_virtual_speed, mi)
 
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None,

@@ -95,6 +95,7 @@ struct clik_skill {
   KernelInfo qp_duals, nlp_duals;   // constraint multipliers (manifest o[18]: bit 0 QP, bit 1 NLP; at most 32 rows)
   KernelInfo qp_vjp, nlp_vjp;       // reverse-mode derivative of the step (manifest o[19]: bit 0 QP, bit 1 NLP)
   KernelInfo qp_jvp, nlp_jvp, qp_jac, nlp_jac;   // forward-mode derivative and Jacobian (o[20]: bit 0 QP, bit 1 NLP)
+  KernelInfo qp_rjvp, nlp_rjvp, qp_rjac, nlp_rjac;   // tangent and Jacobian rollouts (o[21]: bit 0 QP, bit 1 NLP)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
@@ -528,6 +529,11 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
   if (st == CLIK_OK && (jvp & 1)) st = setup_kernel(s, "clik_qp_jacobian_kernel", &s->qp_jac);
   if (st == CLIK_OK && (jvp & 2)) st = setup_kernel(s, "clik_nlp_jvp_kernel", &s->nlp_jvp);
   if (st == CLIK_OK && (jvp & 2)) st = setup_kernel(s, "clik_nlp_jacobian_kernel", &s->nlp_jac);
+  const int rjvp = hsz[21];    // tangent + Jacobian rollouts (emit_skill(..., jvp=True, rollout_jvp=True))
+  if (st == CLIK_OK && (rjvp & 1)) st = setup_kernel(s, "clik_qp_rollout_jvp_kernel", &s->qp_rjvp);
+  if (st == CLIK_OK && (rjvp & 1)) st = setup_kernel(s, "clik_qp_rollout_jacobian_kernel", &s->qp_rjac);
+  if (st == CLIK_OK && (rjvp & 2)) st = setup_kernel(s, "clik_nlp_rollout_jvp_kernel", &s->nlp_rjvp);
+  if (st == CLIK_OK && (rjvp & 2)) st = setup_kernel(s, "clik_nlp_rollout_jacobian_kernel", &s->nlp_rjac);
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
     delete s;
@@ -1339,6 +1345,103 @@ clik_status clik_nlp_jacobian(const clik_skill* s, int64_t N, const double* t, i
                               const double* x, const double* y, const double* sol, const int32_t* status,
                               const uint32_t* active, double* jac, void* stream) {
   return jacobian_impl(s, true, N, t, t_stride, q, x, y, sol, status, active, jac, stream);
+}
+
+}  // extern "C"
+
+// ---- forward-mode derivative of the closed-loop rollouts (clik_jvp.cuh) --------------------------------------
+namespace {
+
+clik_status rollout_tangent_check(const clik_skill* s, const KernelInfo& k, const char* what, bool nlp, int64_t N,
+                                  int32_t steps, const double* t0, const double* q, const double* x,
+                                  const double* y) {
+  if (!k.kernel)
+    return fail(CLIK_ERR_INVALID, "skill image has no %s %s rollout kernel (build it with emit_skill(..., jvp=True, "
+                "rollout_jvp=True); at most 32 constraint rows)", nlp ? "NLP" : "QP", what);
+  clik_status st = check_common(s, N, t0, q, x, y);
+  if (st != CLIK_OK) return st;
+  if (steps < 0) return fail(CLIK_ERR_INVALID, "steps < 0");
+  return CLIK_OK;
+}
+
+int rollout_max_iter(const clik_skill* s, bool nlp, int32_t max_iter) {
+  if (max_iter > 0) return max_iter;
+  return nlp ? NLP_DEFAULT_MAX_ITER : 10 * (s->desc.qp_n + s->desc.qp_m);
+}
+
+clik_status rollout_jvp_impl(const clik_skill* s, bool nlp, int64_t N, int32_t steps, double dt, const double* t0,
+                             int32_t t_stride, double* q, double* x, const double* y, double vmax_q, double vmax_x,
+                             double* sol_last, int32_t* n_failed, int32_t max_iter, const double* t0_dot,
+                             const double* q_dot, const double* x_dot, const double* y_dot, double* q_dot_out,
+                             double* x_dot_out, double* sol_dot, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_rjvp : s->qp_rjvp;
+  clik_status st = rollout_tangent_check(s, k, "tangent", nlp, N, steps, t0, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!q_dot_out) return fail(CLIK_ERR_INVALID, "q_dot_out is required");
+  if (s->desc.n_virtual > 0 && !x_dot_out) return fail(CLIK_ERR_INVALID, "x_dot_out is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0, ks = steps, mi = rollout_max_iter(s, nlp, max_iter);
+  void* args[] = {&n, &l, &ks, &dt, &t0, &ts, &q, &x, &y, &vmax_q, &vmax_x, &sol_last, &n_failed, &mi,
+                  &t0_dot, &q_dot, &x_dot, &y_dot, &q_dot_out, &x_dot_out, &sol_dot};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+clik_status rollout_jacobian_impl(const clik_skill* s, bool nlp, int64_t N, int32_t steps, double dt,
+                                  const double* t0, int32_t t_stride, double* q, double* x, const double* y,
+                                  double vmax_q, double vmax_x, double* sol_last, int32_t* n_failed,
+                                  int32_t max_iter, double* jac, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_rjac : s->qp_rjac;
+  clik_status st = rollout_tangent_check(s, k, "Jacobian", nlp, N, steps, t0, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!jac) return fail(CLIK_ERR_INVALID, "jac is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0, ks = steps, mi = rollout_max_iter(s, nlp, max_iter);
+  void* args[] = {&n, &l, &ks, &dt, &t0, &ts, &q, &x, &y, &vmax_q, &vmax_x, &sol_last, &n_failed, &mi, &jac};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_qp_rollout_jvp(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                const double* t0_dot, const double* q_dot, const double* x_dot, const double* y_dot,
+                                double* q_dot_out, double* x_dot_out, double* sol_dot, void* stream) {
+  return rollout_jvp_impl(s, false, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed, sol_last,
+                          n_failed, max_iter, t0_dot, q_dot, x_dot, y_dot, q_dot_out, x_dot_out, sol_dot, stream);
+}
+
+clik_status clik_nlp_rollout_jvp(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                 double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                 const double* t0_dot, const double* q_dot, const double* x_dot, const double* y_dot,
+                                 double* q_dot_out, double* x_dot_out, double* sol_dot, void* stream) {
+  return rollout_jvp_impl(s, true, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed, sol_last,
+                          n_failed, max_iter, t0_dot, q_dot, x_dot, y_dot, q_dot_out, x_dot_out, sol_dot, stream);
+}
+
+clik_status clik_qp_rollout_jacobian(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                     int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                     double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                     double* jac, void* stream) {
+  return rollout_jacobian_impl(s, false, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed,
+                               sol_last, n_failed, max_iter, jac, stream);
+}
+
+clik_status clik_nlp_rollout_jacobian(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                      int32_t t_stride, double* q, double* x, const double* y,
+                                      double max_robot_speed, double max_virtual_speed, double* sol_last,
+                                      int32_t* n_failed, int32_t max_iter, double* jac, void* stream) {
+  return rollout_jacobian_impl(s, true, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed,
+                               sol_last, n_failed, max_iter, jac, stream);
 }
 
 clik_status clik_measure_fp64_peak(int32_t device, int32_t iters, double* tflops) {

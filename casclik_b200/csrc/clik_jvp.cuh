@@ -94,16 +94,19 @@ struct QpFace {
   unsigned up, lo;
   int W[NN], k;
   double lam[M], Q[NN * NN], R[NN * NN], s[NN], xs[NN];
-  __device__ __forceinline__ bool factor(long long ld, long long i, const double* __restrict__ t, int t_stride,
-                                         const double* __restrict__ q, const double* __restrict__ x,
-                                         const double* __restrict__ y, const double* __restrict__ sol,
-                                         const int* __restrict__ status, const unsigned* __restrict__ active) {
-    if (status[i] != QP_OK) return false;
-    duals_load<S, S::JVP_READ_T, S::JVP_READ_Q, S::JVP_READ_X, S::JVP_READ_Y>(ld, i, t, t_stride, q, x, y, tv, qv, xv,
-                                                                              yv);
+  // from values in registers: the inputs, the step's solution, status and working set
+  __device__ __forceinline__ bool factor(double t_, const double (&q_)[S::NQ > 0 ? S::NQ : 1],
+                                         const double (&x_)[S::NX > 0 ? S::NX : 1],
+                                         const double (&y_)[S::NY > 0 ? S::NY : 1], const double (&sol_)[NN], int st,
+                                         unsigned up_, unsigned lo_) {
+    if (st != QP_OK) return false;
+    tv = t_;
+    for (int j = 0; j < S::NQ; ++j) qv[j] = q_[j];
+    for (int j = 0; j < S::NX; ++j) xv[j] = x_[j];
+    for (int j = 0; j < S::NY; ++j) yv[j] = y_[j];
     S::eval_qp(tv, qv, xv, yv, d);
-    up = active[i];
-    lo = active[ld + i];
+    up = up_;
+    lo = lo_;
     if (!working_set_rows<NN, M>(up, lo, W, k, lam)) return false;
     for (int j = 0; j < NN; ++j) s[j] = 1.0 / sqrt(d.h[j]);
     for (int a = 0; a < k; ++a)
@@ -111,11 +114,23 @@ struct QpFace {
     if (!working_set_qr<NN>(k, Q, R)) return false;
     double sg[NN];
     for (int j = 0; j < NN; ++j) {
-      xs[j] = sol[(long long)j * ld + i];
+      xs[j] = sol_[j];
       sg[j] = s[j] * (d.h[j] * xs[j]);
     }
     working_set_solve<NN>(k, W, Q, R, sg, lam);
     return true;
+  }
+  // of instance i, from global memory
+  __device__ __forceinline__ bool factor(long long ld, long long i, const double* __restrict__ t, int t_stride,
+                                         const double* __restrict__ q, const double* __restrict__ x,
+                                         const double* __restrict__ y, const double* __restrict__ sol,
+                                         const int* __restrict__ status, const unsigned* __restrict__ active) {
+    if (status[i] != QP_OK) return false;
+    duals_load<S, S::JVP_READ_T, S::JVP_READ_Q, S::JVP_READ_X, S::JVP_READ_Y>(ld, i, t, t_stride, q, x, y, tv, qv, xv,
+                                                                              yv);
+    double sv[NN];
+    for (int j = 0; j < NN; ++j) sv[j] = sol[(long long)j * ld + i];
+    return factor(tv, qv, xv, yv, sv, QP_OK, active[i], active[ld + i]);
   }
   // x_dot from rho1 (stride c) and rho2
   __device__ __forceinline__ void solve(const double* r1, const double* r2u, const double* r2l, int c,
@@ -135,20 +150,22 @@ struct NlpFace {
   unsigned up, lo;
   int W[NN], k;
   double lam[M], Q[NN * NN], R[NN * NN], L[NH], xs[NN];
-  __device__ __forceinline__ bool factor(long long ld, long long i, const double* __restrict__ t, int t_stride,
-                                         const double* __restrict__ q, const double* __restrict__ x,
-                                         const double* __restrict__ y, const double* __restrict__ sol,
-                                         const int* __restrict__ status, const unsigned* __restrict__ active) {
-    if (status[i] != 0) return false;
-    duals_load<S, S::JVP_READ_T, S::JVP_READ_Q, S::JVP_READ_X, S::JVP_READ_Y>(ld, i, t, t_stride, q, x, y, tv, qv, xv,
-                                                                              yv);
+  __device__ __forceinline__ bool factor(double t_, const double (&q_)[S::NQ > 0 ? S::NQ : 1],
+                                         const double (&x_)[S::NX > 0 ? S::NX : 1],
+                                         const double (&y_)[S::NY > 0 ? S::NY : 1], const double (&sol_)[NN], int st,
+                                         unsigned up_, unsigned lo_) {
+    if (st != 0) return false;
+    tv = t_;
+    for (int j = 0; j < S::NQ; ++j) qv[j] = q_[j];
+    for (int j = 0; j < S::NX; ++j) xv[j] = x_[j];
+    for (int j = 0; j < S::NY; ++j) yv[j] = y_[j];
     NlpData<typename S::Base> d;
     S::eval_nlp_pre(tv, qv, xv, yv, d);
-    up = active[i];
-    lo = active[ld + i];
+    up = up_;
+    lo = lo_;
     double g[NN], H[NH], one[NN];
     for (int j = 0; j < NN; ++j) {
-      xs[j] = sol[(long long)j * ld + i];
+      xs[j] = sol_[j];
       one[j] = 1.0;
     }
     S::eval_nlp_fgH(d.P, xs, g, H);
@@ -163,6 +180,17 @@ struct NlpFace {
       nlp_lsolve<NN>(L, &Q[a * NN]);
     }
     return working_set_qr<NN>(k, Q, R);
+  }
+  __device__ __forceinline__ bool factor(long long ld, long long i, const double* __restrict__ t, int t_stride,
+                                         const double* __restrict__ q, const double* __restrict__ x,
+                                         const double* __restrict__ y, const double* __restrict__ sol,
+                                         const int* __restrict__ status, const unsigned* __restrict__ active) {
+    if (status[i] != 0) return false;
+    duals_load<S, S::JVP_READ_T, S::JVP_READ_Q, S::JVP_READ_X, S::JVP_READ_Y>(ld, i, t, t_stride, q, x, y, tv, qv, xv,
+                                                                              yv);
+    double sv[NN];
+    for (int j = 0; j < NN; ++j) sv[j] = sol[(long long)j * ld + i];
+    return factor(tv, qv, xv, yv, sv, 0, active[i], active[ld + i]);
   }
   __device__ __forceinline__ void solve(const double* r1, const double* r2u, const double* r2l, int c,
                                         double* xd) const {
@@ -256,6 +284,229 @@ __device__ __forceinline__ void nlp_jacobian(long long N, long long ld, const do
                                              const double* x, const double* y, const double* sol, const int* status,
                                              const unsigned* active, double* jac) {
   step_jacobian<S, NlpFace<S>>(N, ld, t, t_stride, q, x, y, sol, status, active, jac);
+}
+
+// ---- forward-mode derivative of the closed-loop rollouts ------------------------------------------------------
+//
+// The rollout of qp_rollout / nlp_rollout (the same step helpers, hence the same primal bits) with the tangent of
+// the state carried next to it.  p = (t0, q0, x0, y); at step k theta_k = (t0 + k dt, q_k, x_k, y), sol_k the
+// step's unclipped solution and active_k its working set.  Per step:
+//   s_dot_k = the step JVP above at (theta_k, sol_k, status_k, active_k) along theta_dot_k = (t0_dot, q_dot_k,
+//             x_dot_k, y_dot): exactly 0 for an all-zero theta_dot_k, NaN under the step JVP's rules; once NaN, the
+//             instance's tangent outputs are NaN from then on;
+//   v_dot_j  = s_dot_j where |sol_j| < vmax (vmax_q robot part, vmax_x virtual part), 0 where the clip holds (at
+//             the bound too); slack entries are not clipped;
+//   q_dot_{k+1} = q_dot_k + dt v_dot_q,  x_dot_{k+1} = x_dot_k + dt v_dot_x  (the rounding of the primal update).
+// The face of step k is factored from registers before the solution is clipped into the next step's start.
+// The Jacobian rollout carries P = d(q_k, x_k)/dp (NS x NT) instead: one eval_jac and one factorisation per step,
+// rho contracted with d theta_k / dp = [e_0; P; 0 I], then NT face solves.
+
+// The primal of one instance's QP rollout: qp_rollout_solve / qp_rollout_advance, as qp_rollout.  P = the step
+// skill (the struct qp_rollout is instantiated on), S = its JVP struct.
+template <class S, class P>
+struct QpRolloutState {
+  using Face = QpFace<S>;
+  static constexpr int NN = S::QN;
+  double xs[NN];             // the step's unclipped solution after solve(), clipped after advance()
+  unsigned mu = 0u, ml = 0u;  // working set of the previous step = warm start of the next
+  int st = QP_OK;
+  __device__ __forceinline__ QpRolloutState() {
+    for (int j = 0; j < NN; ++j) xs[j] = 0.0;
+  }
+  __device__ __forceinline__ void solve(double tv, const double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                        const double (&xv)[S::NX > 0 ? S::NX : 1],
+                                        const double (&yv)[S::NY > 0 ? S::NY : 1], int max_iter) {
+    st = qp_rollout_solve<P>(tv, qv, xv, yv, xs, mu, ml, max_iter);
+  }
+  __device__ __forceinline__ const double (&sol() const)[NN] { return xs; }
+  __device__ __forceinline__ void advance(double (&qv)[S::NQ > 0 ? S::NQ : 1], double (&xv)[S::NX > 0 ? S::NX : 1],
+                                          double vmax_q, double vmax_x, double dt, int& failed) {
+    qp_rollout_advance<P>(st, xs, qv, xv, vmax_q, vmax_x, dt, failed);
+  }
+  __device__ __forceinline__ double last(int j, int) const { return xs[j]; }
+};
+
+// The primal of one instance's NLP rollout: nlp_rollout_solve / nlp_rollout_advance, as nlp_rollout.
+template <class S, class P>
+struct NlpRolloutState {
+  using Face = NlpFace<S>;
+  static constexpr int NN = S::NN;
+  double v[NN], xs[NN];      // v: the step's solution and the next step's start; xs: v clipped
+  unsigned mu = 0u, ml = 0u;
+  int st = 0;
+  __device__ __forceinline__ NlpRolloutState() {
+    for (int j = 0; j < NN; ++j) v[j] = 0.0;
+  }
+  __device__ __forceinline__ void solve(double tv, const double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                        const double (&xv)[S::NX > 0 ? S::NX : 1],
+                                        const double (&yv)[S::NY > 0 ? S::NY : 1], int max_iter) {
+    st = nlp_rollout_solve<P>(tv, qv, xv, yv, v, mu, ml, max_iter);
+  }
+  __device__ __forceinline__ const double (&sol() const)[NN] { return v; }
+  __device__ __forceinline__ void advance(double (&qv)[S::NQ > 0 ? S::NQ : 1], double (&xv)[S::NX > 0 ? S::NX : 1],
+                                          double vmax_q, double vmax_x, double dt, int& failed) {
+    nlp_rollout_advance<P>(st, v, xs, qv, xv, vmax_q, vmax_x, dt, failed);
+  }
+  __device__ __forceinline__ double last(int j, int steps) const { return steps > 0 ? xs[j] : 0.0; }
+};
+
+// The clip mask of a step's tangent (entries j < NQ + NX of s_dot) and the Euler update of the state tangent.
+template <class S>
+__device__ __forceinline__ double clip_tangent(int j, double sol_j, double s_dot_j, double vmax_q, double vmax_x) {
+  return fabs(sol_j) < (j < S::NQ ? vmax_q : vmax_x) ? s_dot_j : 0.0;
+}
+
+// Tangent rollout (JAC false: q_dot_out, x_dot_out, sol_dot) or Jacobian rollout (JAC true: jac, entry (s, c) of
+// instance i at jac[(s*NT + c)*ld + i], s over (q, x), c over p), with the primal outputs of the rollout kernels.
+// R: QpRolloutState<S, P> or NlpRolloutState<S, P>.
+template <class S, class R, bool JAC>
+__device__ __forceinline__ void rollout_tangent(long long N, long long ld, int steps, double dt,
+                                                const double* __restrict__ t0, int t_stride, double* __restrict__ q,
+                                                double* __restrict__ x, const double* __restrict__ y, double vmax_q,
+                                                double vmax_x, double* __restrict__ sol_last,
+                                                int* __restrict__ n_failed, int max_iter,
+                                                const double* __restrict__ t_dot, const double* __restrict__ q_dot,
+                                                const double* __restrict__ x_dot, const double* __restrict__ y_dot,
+                                                double* __restrict__ q_dot_out, double* __restrict__ x_dot_out,
+                                                double* __restrict__ sol_dot, double* __restrict__ jac) {
+  using F = typename R::Face;
+  constexpr int NN = F::NN, M = F::M, NQ = S::NQ, NX = S::NX, NY = S::NY, NS = NQ + NX, NT = 1 + NS + NY;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride) {
+    double qv[NQ > 0 ? NQ : 1], xv[NX > 0 ? NX : 1], yv[NY > 0 ? NY : 1];
+    const double t0v = t0[(long long)t_stride * i];
+    for (int j = 0; j < NQ; ++j) qv[j] = q[(long long)j * ld + i];
+    for (int j = 0; j < NX; ++j) xv[j] = x[(long long)j * ld + i];
+    for (int j = 0; j < NY; ++j) yv[j] = y[(long long)j * ld + i];
+    double td, qd[NQ > 0 ? NQ : 1], xd[NX > 0 ? NX : 1], yd[NY > 0 ? NY : 1];   // JVP: the state's tangent
+    double sd[NN];                                                              // JVP: s_dot of the last step
+    double Pm[JAC ? NS * NT : 1];                                               // Jacobian: d(q, x)/dp
+    if constexpr (JAC) {
+      for (int a = 0; a < NS * NT; ++a) Pm[a] = 0.0;
+      for (int a = 0; a < NS; ++a) Pm[a * NT + 1 + a] = 1.0;
+    } else {
+      jvp_tangent<S>(ld, i, t_dot, q_dot, x_dot, y_dot, td, qd, xd, yd);
+      for (int j = 0; j < NN; ++j) sd[j] = 0.0;
+    }
+    bool dead = false;   // a NaN derivative: every later one is NaN
+    int failed = 0;
+    R r;
+    for (int k = 0; k < steps; ++k) {
+      const double tv = __dadd_rn(t0v, __dmul_rn(dt, (double)k));
+      r.solve(tv, qv, xv, yv, max_iter);
+      if constexpr (JAC) {
+        if (!dead) {
+          F f;
+          if (f.factor(tv, qv, xv, yv, r.sol(), r.st, r.mu, r.ml)) {
+            double r1[NN * NT], r2u[M * NT], r2l[M * NT];
+            S::eval_jac(f.tv, f.qv, f.xv, f.yv, f.xs, f.lam, r1, r2u, r2l);
+            // d rho / dp = d rho / d theta_k . d theta_k / dp, row by row in place
+            auto chain = [&](double* row) {
+              double out[NT];
+              for (int c = 0; c < NT; ++c) {
+                double acc = (c == 0 || c > NS) ? row[c] : 0.0;
+                for (int a = 0; a < NS; ++a) acc = fma(row[1 + a], Pm[a * NT + c], acc);
+                out[c] = acc;
+              }
+              for (int c = 0; c < NT; ++c) row[c] = out[c];
+            };
+            for (int j = 0; j < NN; ++j) chain(&r1[j * NT]);
+            for (int a = 0; a < M; ++a) {
+              chain(&r2u[a * NT]);
+              chain(&r2l[a * NT]);
+            }
+            for (int c = 0; c < NT; ++c) {
+              double col[NN];
+              f.solve(&r1[c], &r2u[c], &r2l[c], NT, col);
+              for (int a = 0; a < NS; ++a)
+                Pm[a * NT + c] = __dadd_rn(Pm[a * NT + c],
+                                           __dmul_rn(clip_tangent<S>(a, r.sol()[a], col[a], vmax_q, vmax_x), dt));
+            }
+          } else {
+            dead = true;
+          }
+        }
+      } else {
+        bool zero = td == 0.0;
+        for (int j = 0; j < NQ; ++j) zero = zero && qd[j] == 0.0;
+        for (int j = 0; j < NX; ++j) zero = zero && xd[j] == 0.0;
+        for (int j = 0; j < NY; ++j) zero = zero && yd[j] == 0.0;
+        if (zero) {
+          for (int j = 0; j < NN; ++j) sd[j] = 0.0;
+        } else if (!dead) {
+          F f;
+          if (f.factor(tv, qv, xv, yv, r.sol(), r.st, r.mu, r.ml)) {
+            double r1[NN], r2u[M], r2l[M];
+            S::eval_jvp(f.tv, f.qv, f.xv, f.yv, f.xs, f.lam, td, qd, xd, yd, r1, r2u, r2l);
+            f.solve(r1, r2u, r2l, 1, sd);
+            for (int j = 0; j < NS; ++j) sd[j] = clip_tangent<S>(j, r.sol()[j], sd[j], vmax_q, vmax_x);
+            for (int j = 0; j < NQ; ++j) qd[j] = __dadd_rn(qd[j], __dmul_rn(sd[j], dt));
+            for (int j = 0; j < NX; ++j) xd[j] = __dadd_rn(xd[j], __dmul_rn(sd[NQ + j], dt));
+          } else {
+            dead = true;
+          }
+        }
+      }
+      r.advance(qv, xv, vmax_q, vmax_x, dt, failed);
+    }
+    for (int j = 0; j < NQ; ++j) q[(long long)j * ld + i] = qv[j];
+    for (int j = 0; j < NX; ++j) x[(long long)j * ld + i] = xv[j];
+    if (sol_last != nullptr)
+      for (int j = 0; j < NN; ++j) sol_last[(long long)j * ld + i] = r.last(j, steps);
+    if (n_failed != nullptr) n_failed[i] = failed;
+    if constexpr (JAC) {
+      for (int a = 0; a < NS * NT; ++a) jac[(long long)a * ld + i] = dead ? NAN : Pm[a];
+    } else {
+      for (int j = 0; j < NQ; ++j) q_dot_out[(long long)j * ld + i] = dead ? NAN : qd[j];
+      for (int j = 0; j < NX; ++j) x_dot_out[(long long)j * ld + i] = dead ? NAN : xd[j];
+      if (sol_dot != nullptr)
+        for (int j = 0; j < NN; ++j) sol_dot[(long long)j * ld + i] = dead ? NAN : sd[j];
+    }
+  }
+}
+
+template <class S, class P>
+__device__ __forceinline__ void qp_rollout_jvp(long long N, long long ld, int steps, double dt, const double* t0,
+                                               int t_stride, double* q, double* x, const double* y, double vmax_q,
+                                               double vmax_x, double* sol_last, int* n_failed, int max_iter,
+                                               const double* t_dot, const double* q_dot, const double* x_dot,
+                                               const double* y_dot, double* q_dot_out, double* x_dot_out,
+                                               double* sol_dot) {
+  rollout_tangent<S, QpRolloutState<S, P>, false>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,
+                                                  n_failed, max_iter, t_dot, q_dot, x_dot, y_dot, q_dot_out,
+                                                  x_dot_out, sol_dot, nullptr);
+}
+
+template <class S, class P>
+__device__ __forceinline__ void nlp_rollout_jvp(long long N, long long ld, int steps, double dt, const double* t0,
+                                                int t_stride, double* q, double* x, const double* y, double vmax_q,
+                                                double vmax_x, double* sol_last, int* n_failed, int max_iter,
+                                                const double* t_dot, const double* q_dot, const double* x_dot,
+                                                const double* y_dot, double* q_dot_out, double* x_dot_out,
+                                                double* sol_dot) {
+  rollout_tangent<S, NlpRolloutState<S, P>, false>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,
+                                                   n_failed, max_iter, t_dot, q_dot, x_dot, y_dot, q_dot_out,
+                                                   x_dot_out, sol_dot, nullptr);
+}
+
+template <class S, class P>
+__device__ __forceinline__ void qp_rollout_jacobian(long long N, long long ld, int steps, double dt, const double* t0,
+                                                    int t_stride, double* q, double* x, const double* y,
+                                                    double vmax_q, double vmax_x, double* sol_last, int* n_failed,
+                                                    int max_iter, double* jac) {
+  rollout_tangent<S, QpRolloutState<S, P>, true>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,
+                                                 n_failed, max_iter, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                                 nullptr, nullptr, jac);
+}
+
+template <class S, class P>
+__device__ __forceinline__ void nlp_rollout_jacobian(long long N, long long ld, int steps, double dt, const double* t0,
+                                                     int t_stride, double* q, double* x, const double* y,
+                                                     double vmax_q, double vmax_x, double* sol_last, int* n_failed,
+                                                     int max_iter, double* jac) {
+  rollout_tangent<S, NlpRolloutState<S, P>, true>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,
+                                                  n_failed, max_iter, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                                  nullptr, nullptr, jac);
 }
 
 }  // namespace clik

@@ -254,6 +254,35 @@ __device__ __forceinline__ void nlp_step(long long N, long long ld, const double
   }
 }
 
+// One step of the closed-loop rollouts (nlp_rollout and the tangent rollouts of clik_jvp.cuh): the SQP
+// iteration at (tv, qv, xv, yv) from v, the previous step's solution, which it replaces; (mu, ml) = the last
+// subproblem's working set.  Returns the status.
+template <class S>
+__device__ __forceinline__ int nlp_rollout_solve(double tv, const double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                                 const double (&xv)[S::NX > 0 ? S::NX : 1],
+                                                 const double (&yv)[S::NY > 0 ? S::NY : 1], double (&v)[S::NN],
+                                                 unsigned& mu, unsigned& ml, int max_iter) {
+  NlpData<S> d;
+  S::eval_nlp_pre(tv, qv, xv, yv, d);
+  int it;
+  return nlp_solve<S>(d, v, &mu, &ml, &it, max_iter);
+}
+
+// Applies an NLP rollout step: an unsolved one applies zero velocity, is counted in failed and the next step
+// starts from zero; xs = v with the robot / virtual parts clipped.
+template <class S>
+__device__ __forceinline__ void nlp_rollout_advance(int st, double (&v)[S::NN], double (&xs)[S::NN],
+                                                    double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                                    double (&xv)[S::NX > 0 ? S::NX : 1], double vmax_q,
+                                                    double vmax_x, double dt, int& failed) {
+  if (st != NLP_OK) {
+    ++failed;
+    for (int j = 0; j < S::NN; ++j) v[j] = 0.0;
+  }
+  for (int j = 0; j < S::NN; ++j) xs[j] = v[j];
+  rollout_euler<S>(xs, qv, xv, vmax_q, vmax_x, dt);
+}
+
 // Closed-loop rollout (the loop of qp_rollout): each step starts from the previous step's solution,
 // v = clip(sol[:n], +-max_speed); q += v_rob*dt; x += v_virt*dt.  A step that is not solved applies zero
 // velocity, is counted in n_failed and the next step starts from zero.  sol_last: the last step's
@@ -275,24 +304,9 @@ __device__ __forceinline__ void nlp_rollout(long long N, long long ld, int steps
     int failed = 0;
     for (int k = 0; k < steps; ++k) {
       const double tv = __dadd_rn(t0v, __dmul_rn(dt, (double)k));
-      NlpData<S> d;
-      S::eval_nlp_pre(tv, qv, xv, yv, d);
       unsigned mu, ml;
-      int it;
-      const int st = nlp_solve<S>(d, v, &mu, &ml, &it, max_iter);
-      if (st != NLP_OK) {
-        ++failed;
-        for (int j = 0; j < S::NN; ++j) v[j] = 0.0;
-      }
-      for (int j = 0; j < S::NN; ++j) xs[j] = v[j];
-      for (int j = 0; j < S::NQ; ++j) {
-        xs[j] = fmax(fmin(xs[j], vmax_q), -vmax_q);
-        qv[j] = __dadd_rn(qv[j], __dmul_rn(xs[j], dt));
-      }
-      for (int j = 0; j < S::NX; ++j) {
-        xs[S::NQ + j] = fmax(fmin(xs[S::NQ + j], vmax_x), -vmax_x);
-        xv[j] = __dadd_rn(xv[j], __dmul_rn(xs[S::NQ + j], dt));
-      }
+      const int st = nlp_rollout_solve<S>(tv, qv, xv, yv, v, mu, ml, max_iter);
+      nlp_rollout_advance<S>(st, v, xs, qv, xv, vmax_q, vmax_x, dt, failed);
     }
     for (int j = 0; j < S::NQ; ++j) q[(long long)j * ld + i] = qv[j];
     for (int j = 0; j < S::NX; ++j) x[(long long)j * ld + i] = xv[j];

@@ -1052,6 +1052,76 @@ __device__ __forceinline__ void qp_step_tail(long long N, long long ld, const do
 
 #endif
 
+// One step of the closed-loop rollouts (qp_rollout and the tangent rollouts of clik_jvp.cuh): the QP at
+// (tv, qv, xv, yv), started from the working set (mu, ml) of the previous step, which it replaces.  Returns the
+// status (QP_INVALID for a non-finite solution); xs = the unclipped solution.
+template <class S>
+__device__ __forceinline__ int qp_rollout_solve(double tv, const double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                                const double (&xv)[S::NX > 0 ? S::NX : 1],
+                                                const double (&yv)[S::NY > 0 ? S::NY : 1], double (&xs)[S::QN],
+                                                unsigned& mu, unsigned& ml, int max_iter) {
+  int st;
+  if constexpr (S::QSTRUCT) {
+    QpSData<S> d;
+    S::eval_qps(tv, qv, xv, yv, d);
+    unsigned wu = mu, wl = ml;
+    bool solved = false;            // previous step's set -> this step's (usually one pass)
+    if (S::QP_CRASH) {
+      bool cycling = false;
+      bool ok = crash_guess<S>(d, &wu, &wl, xs, &cycling);
+      if (!ok && cycling && S::QP_CRASH_SINGLE) ok = crash_guess<S, CRASH_SINGLE_PASSES, true>(d, &wu, &wl, xs);
+      solved = ok && S::QP_CRASH_FINAL && all_finite(xs);
+    }
+    st = solved ? QP_OK : QP_MAXITER;
+    if (solved) { mu = wu; ml = wl; }
+#pragma unroll 1
+    for (int attempt = 0; attempt < 2 && !solved; ++attempt) {
+      if (attempt > 0) {
+        wu = wl = 0u;
+        S::eval_qps(tv, qv, xv, yv, d);
+      }
+      st = qp_structured<S>(d, xs, &mu, &ml, max_iter, wu, wl);
+      if (st == QP_OK || (wu | wl) == 0u) break;
+    }
+  } else {
+    QpData<S> d;
+    S::eval_qp(tv, qv, xv, yv, d);
+    st = qp_dual_active_set<S::QN, S::QM>(S::QN, S::QM, d.A, d.lb, d.ub, d.h, nullptr, xs, &mu, &ml,
+                                          max_iter);
+  }
+  if (st == QP_OK && !all_finite(xs)) st = QP_INVALID;
+  return st;
+}
+
+// The clip and the Euler update of a rollout step (QP and NLP): v = clip(xs[:n], +-max_speed) in place,
+// q += v_rob*dt, x += v_virt*dt.
+template <class S, int NN>
+__device__ __forceinline__ void rollout_euler(double (&xs)[NN], double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                              double (&xv)[S::NX > 0 ? S::NX : 1], double vmax_q, double vmax_x,
+                                              double dt) {
+  for (int j = 0; j < S::NQ; ++j) {
+    xs[j] = fmax(fmin(xs[j], vmax_q), -vmax_q);
+    qv[j] = __dadd_rn(qv[j], __dmul_rn(xs[j], dt));
+  }
+  for (int j = 0; j < S::NX; ++j) {
+    xs[S::NQ + j] = fmax(fmin(xs[S::NQ + j], vmax_x), -vmax_x);
+    xv[j] = __dadd_rn(xv[j], __dmul_rn(xs[S::NQ + j], dt));
+  }
+}
+
+// Applies a solved QP rollout step: an unsolved one (st != QP_OK) applies zero velocity and is counted in failed;
+// xs is left clipped, the next step's start.
+template <class S>
+__device__ __forceinline__ void qp_rollout_advance(int st, double (&xs)[S::QN], double (&qv)[S::NQ > 0 ? S::NQ : 1],
+                                                   double (&xv)[S::NX > 0 ? S::NX : 1], double vmax_q,
+                                                   double vmax_x, double dt, int& failed) {
+  if (st != QP_OK) {
+    ++failed;
+    for (int j = 0; j < S::QN; ++j) xs[j] = 0.0;
+  }
+  rollout_euler<S>(xs, qv, xv, vmax_q, vmax_x, dt);
+}
+
 // Closed-loop rollout with the QP controller: `steps` times  sol = solve(t0 + k*dt, q, x, y);
 // v = clip(sol[:n], +-max_speed); q += v_rob*dt; x += v_virt*dt  (the notebooks' simulation loop,
 // ur5_moe2016_example2.ipynb cell 12).  A step whose QP is not solved (status != 0; the reference
@@ -1075,48 +1145,8 @@ __device__ __forceinline__ void qp_rollout(long long N, long long ld, int steps,
     unsigned mu = 0u, ml = 0u;        // working set of the previous step = warm start of the next
     for (int k = 0; k < steps; ++k) {
       const double tv = __dadd_rn(t0v, __dmul_rn(dt, (double)k));
-      int st;
-      if constexpr (S::QSTRUCT) {
-        QpSData<S> d;
-        S::eval_qps(tv, qv, xv, yv, d);
-        unsigned wu = mu, wl = ml;
-        bool solved = false;            // previous step's set -> this step's (usually one pass)
-        if (S::QP_CRASH) {
-          bool cycling = false;
-          bool ok = crash_guess<S>(d, &wu, &wl, xs, &cycling);
-          if (!ok && cycling && S::QP_CRASH_SINGLE) ok = crash_guess<S, CRASH_SINGLE_PASSES, true>(d, &wu, &wl, xs);
-          solved = ok && S::QP_CRASH_FINAL && all_finite(xs);
-        }
-        st = solved ? QP_OK : QP_MAXITER;
-        if (solved) { mu = wu; ml = wl; }
-#pragma unroll 1
-        for (int attempt = 0; attempt < 2 && !solved; ++attempt) {
-          if (attempt > 0) {
-            wu = wl = 0u;
-            S::eval_qps(tv, qv, xv, yv, d);
-          }
-          st = qp_structured<S>(d, xs, &mu, &ml, max_iter, wu, wl);
-          if (st == QP_OK || (wu | wl) == 0u) break;
-        }
-      } else {
-        QpData<S> d;
-        S::eval_qp(tv, qv, xv, yv, d);
-        st = qp_dual_active_set<S::QN, S::QM>(S::QN, S::QM, d.A, d.lb, d.ub, d.h, nullptr, xs, &mu, &ml,
-                                              max_iter);
-      }
-      if (st == QP_OK && !all_finite(xs)) st = QP_INVALID;
-      if (st != QP_OK) {
-        ++failed;
-        for (int j = 0; j < S::QN; ++j) xs[j] = 0.0;
-      }
-      for (int j = 0; j < S::NQ; ++j) {
-        xs[j] = fmax(fmin(xs[j], vmax_q), -vmax_q);
-        qv[j] = __dadd_rn(qv[j], __dmul_rn(xs[j], dt));
-      }
-      for (int j = 0; j < S::NX; ++j) {
-        xs[S::NQ + j] = fmax(fmin(xs[S::NQ + j], vmax_x), -vmax_x);
-        xv[j] = __dadd_rn(xv[j], __dmul_rn(xs[S::NQ + j], dt));
-      }
+      const int st = qp_rollout_solve<S>(tv, qv, xv, yv, xs, mu, ml, max_iter);
+      qp_rollout_advance<S>(st, xs, qv, xv, vmax_q, vmax_x, dt, failed);
     }
     for (int j = 0; j < S::NQ; ++j) q[(long long)j * ld + i] = qv[j];
     for (int j = 0; j < S::NX; ++j) x[(long long)j * ld + i] = xv[j];

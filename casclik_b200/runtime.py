@@ -41,6 +41,7 @@ EXPORTS = (
     "clik_qp_duals", "clik_nlp_duals", "clik_qp_duals_host", "clik_nlp_duals_host",
     "clik_qp_solve_one_lam", "clik_nlp_solve_one_lam", "clik_qp_vjp", "clik_nlp_vjp",
     "clik_qp_jvp", "clik_nlp_jvp", "clik_qp_jacobian", "clik_nlp_jacobian",
+    "clik_qp_rollout_jvp", "clik_nlp_rollout_jvp", "clik_qp_rollout_jacobian", "clik_nlp_rollout_jacobian",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -134,6 +135,13 @@ def load_library():
     for name in ("clik_qp_jacobian", "clik_nlp_jacobian"):
         getattr(lib, name).restype = i32
         getattr(lib, name).argtypes = [vp, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]
+    rollout = [vp, i64, i32, ctypes.c_double, vp, i32, vp, vp, vp, ctypes.c_double, ctypes.c_double, vp, vp, i32]
+    for name in ("clik_qp_rollout_jvp", "clik_nlp_rollout_jvp"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = rollout + [vp, vp, vp, vp, vp, vp, vp, vp]
+    for name in ("clik_qp_rollout_jacobian", "clik_nlp_rollout_jacobian"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = rollout + [vp, vp]
     lib.clik_qp_solve_one_lam.restype = i32
     lib.clik_qp_solve_one_lam.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.clik_nlp_solve_one_lam.restype = i32

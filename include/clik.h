@@ -341,6 +341,51 @@ clik_status clik_nlp_jacobian(const clik_skill* skill, int64_t N, const double* 
                               const double* q, const double* x, const double* y, const double* sol,
                               const int32_t* status, const uint32_t* active, double* jac, void* stream);
 
+/* Forward-mode derivative of the closed-loop rollouts clik_qp_rollout / clik_nlp_rollout, for N instances.  The
+ * primal is exactly that rollout (same warm starts, failure rule, clip fmax(fmin(v, vmax), -vmax) and Euler update
+ * q + v*dt), and q, x, sol_last and n_failed are bit-identical to it; q and x are updated in place as there.
+ * Inputs p = (t0, q0, x0, y), n_theta = 1 + n_robot + n_virtual + n_input as clik_qp_jacobian.  At step k,
+ * theta_k = (t0 + k*dt, q_k, x_k, y) and theta_dot_k = (t0_dot, q_dot_k, x_dot_k, y_dot); then
+ *   s_dot_k = the step JVP (clik_qp_jvp / clik_nlp_jvp) at (theta_k, sol_k, status_k, active_k) along theta_dot_k,
+ *             sol_k the step's unclipped solution and active_k its working set: exactly 0 for an all-zero
+ *             theta_dot_k; otherwise NaN when status_k != 0 (a failed step that applied zero velocity included), A_W
+ *             is rank-deficient or (NLP) a Cholesky pivot is rejected; once NaN, every later tangent of the instance
+ *             is NaN, and so are all its tangent outputs;
+ *   v_dot_j = s_dot_j where |sol_j| < vmax (vmax_q robot part, vmax_x virtual part), 0 otherwise (at the bound the
+ *             clip holds); slack entries are not clipped;
+ *   q_dot_{k+1} = q_dot_k + dt*v_dot_q,  x_dot_{k+1} = x_dot_k + dt*v_dot_x (rounded as the primal update).
+ * As clik_qp_jvp this is the derivative of the face solution at the returned point: the NLP's dependence on its
+ * warm start (below its tol) is not differentiated.
+ *   clik_<kind>_rollout_jvp: the arguments of clik_<kind>_rollout, the tangent t0_dot [N], q_dot [n_robot * N],
+ *     x_dot [n_virtual * N], y_dot [n_input * N] (NULL = zero; not modified) and the outputs q_dot_out
+ *     [n_robot * N] and x_dot_out [n_virtual * N] (tangents of the final state, required) and sol_dot [qp_n * N]
+ *     (tangent of sol_last, may be NULL).  steps = 0 gives q_dot_out = q_dot, x_dot_out = x_dot, sol_dot = 0.
+ *   clik_<kind>_rollout_jacobian: jac = d(q_K, x_K)/dp, n_s = n_robot + n_virtual rows, entry (s, c) of instance i
+ *     at jac[(s * n_theta + c) * N + i]; column c is the tangent rollout along the unit tangent e_c.  One row
+ *     evaluation and one face factorisation per step: rho is contracted with the carried d theta_k/dp, then n_theta
+ *     face solves; an instance with a NaN tangent gets a block of NaN.
+ * The kernels are in images built with emit_skill(..., jvp=True, rollout_jvp=True) (manifest o[21]) only, for skills
+ * with a rollout kernel and 1..32 constraint rows: other images, and a NULL skill, fail with CLIK_ERR_INVALID.
+ * Device pointers only, row stride N, asynchronous on `stream`; one thread per instance. */
+clik_status clik_qp_rollout_jvp(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                const double* t0_dot, const double* q_dot, const double* x_dot, const double* y_dot,
+                                double* q_dot_out, double* x_dot_out, double* sol_dot, void* stream);
+clik_status clik_nlp_rollout_jvp(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                 double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                 const double* t0_dot, const double* q_dot, const double* x_dot, const double* y_dot,
+                                 double* q_dot_out, double* x_dot_out, double* sol_dot, void* stream);
+clik_status clik_qp_rollout_jacobian(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                     int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                     double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                     double* jac, void* stream);
+clik_status clik_nlp_rollout_jacobian(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                      int32_t t_stride, double* q, double* x, const double* y,
+                                      double max_robot_speed, double max_virtual_speed, double* sol_last,
+                                      int32_t* n_failed, int32_t max_iter, double* jac, void* stream);
+
 /* One host batch over several GPUs of the box: `skills[k]` is the same cubin loaded on device k
  * (clik_skill_load with desc.device = k); the batch is cut into n_skills contiguous shards (sizes differ
  * by at most one, shard k = [k*N/n .. )), each shard runs on its device from its own host thread (zero
