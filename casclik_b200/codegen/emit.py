@@ -339,14 +339,15 @@ def _switch(name, values, ret="int"):
 
 
 def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks=None, qp_fast_min_blocks=None,
-               nlp=None, nlp_tol=1e-10, vjp=False, jvp=False, rollout_jvp=False):
+               nlp=None, nlp_tol=1e-10, vjp=False, jvp=False, rollout_jvp=False, rollout_vjp=False):
     """-> (source text, meta dict).  `pinv`: PinvProgram or None, `qp`: QpProgram or None; or `nlp`:
     NlpProgram (an NLP-only image, stopping tolerance `nlp_tol`).  `vjp`: also append the reverse-mode
     derivative kernel of the QP / NLP step (clik_vjp.cuh) after the multiplier kernel, for skills that have
     one; everything emitted before it is the same text as with vjp=False.  `jvp`: likewise append the
     forward-mode derivative and Jacobian kernels (clik_jvp.cuh), after the VJP kernel when both are asked for.
     `rollout_jvp` (with `jvp`): then also the tangent and Jacobian rollouts (clik_jvp.cuh), for skills with a
-    rollout kernel.
+    rollout kernel.  `rollout_vjp` (with `vjp`): likewise the taped rollout and its reverse sweep
+    (clik_rollout_vjp.cuh), last.
     Tuning knobs (also settable through the environment for experiments): CLIK_BLOCK,
     CLIK_MINBLOCKS, CLIK_CONSTBANK (1), CLIK_FAST_SINCOS (1)."""
     if block_threads is None:
@@ -354,7 +355,7 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     if nlp is not None:
         if pinv is not None or qp is not None:
             raise ValueError("an NLP image holds the NLP kernels only")
-        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp, jvp, rollout_jvp)
+        return _emit_nlp(nlp, label, block_threads, nlp_tol, vjp, jvp, rollout_jvp, rollout_vjp)
     env_min_blocks = int(os.environ.get("CLIK_MINBLOCKS", "0"))
     if min_blocks is None:
         min_blocks = env_min_blocks
@@ -746,6 +747,9 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
     meta["rollout_jvp"] = bool(rollout_jvp) and meta["jvp"] and qp_rollout
     if meta["rollout_jvp"]:
         out.append(_ROLLOUT_JVP_MANIFEST % 1)
+    meta["rollout_vjp"] = bool(rollout_vjp) and meta["vjp"] and qp_rollout
+    if meta["rollout_vjp"]:
+        out.append(_ROLLOUT_VJP_MANIFEST % 1)
     out.append("}")
     if meta["duals"]:
         out += _emit_qp_duals(qp, sig, sincos_name, block_threads, meta["qp_structured"])
@@ -757,6 +761,8 @@ def emit_skill(pinv=None, qp=None, label="skill", block_threads=None, min_blocks
                          "SkillDuals" if meta["qp_structured"] else "Skill", meta["qp_read_masks"], meta)
     if meta["rollout_jvp"]:
         out += _emit_rollout_jvp("qp", block_threads)
+    if meta["rollout_vjp"]:
+        out += _emit_rollout_vjp("qp", block_threads)
     return "\n".join(out) + "\n", meta
 
 
@@ -927,6 +933,34 @@ def _emit_rollout_jvp(kind, block_threads):
             "}"]
 
 
+_ROLLOUT_VJP_MANIFEST = "  o[22] = %d;   // taped rollout and reverse sweep kernels (1 QP, 2 NLP)"
+
+
+def _emit_rollout_vjp(kind, block_threads):
+    """clik_<kind>_rollout_tape_kernel and clik_<kind>_rollout_vjp_kernel (clik_rollout_vjp.cuh), appended last: the
+    rollout of clik_<kind>_rollout_kernel on the step skill `Skill` writing its tape, and the reverse sweep over the
+    tape with the face and eval_vjp of `SkillVjp`."""
+    return ["", "// ---- reverse-mode derivative of the closed-loop rollout (clik_rollout_vjp.cuh) ----",
+            '#include "clik_rollout_vjp.cuh"',
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_rollout_tape_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, int steps, double dt, const double* t0, int t_stride, double* q, double* x,",
+            "    const double* y, double vmax_q, double vmax_x, double* sol_last, int* n_failed, int max_iter,",
+            "    double* tape_q, double* tape_x, double* tape_sol, int* tape_status, unsigned* tape_active) {",
+            "  clik::%s_rollout_tape<SkillVjp, Skill>(N, ld, steps, dt, t0, t_stride, q, x, y, vmax_q, vmax_x, sol_last,"
+            % kind,
+            "      n_failed, max_iter, tape_q, tape_x, tape_sol, tape_status, tape_active);",
+            "}",
+            'extern "C" __global__ void __launch_bounds__(%d) clik_%s_rollout_vjp_kernel(' % (block_threads, kind),
+            "    long long N, long long ld, int steps, double dt, const double* t0, int t_stride, const double* y,",
+            "    double vmax_q, double vmax_x, const double* tape_q, const double* tape_x, const double* tape_sol,",
+            "    const int* tape_status, const unsigned* tape_active, const double* q_bar_K, const double* x_bar_K,",
+            "    const double* sol_bar, double* t_bar, double* q_bar, double* x_bar, double* y_bar) {",
+            "  clik::%s_rollout_vjp<SkillVjp>(N, ld, steps, dt, t0, t_stride, y, vmax_q, vmax_x, tape_q, tape_x, tape_sol,"
+            % kind,
+            "      tape_status, tape_active, q_bar_K, x_bar_K, sol_bar, t_bar, q_bar, x_bar, y_bar);",
+            "}"]
+
+
 def nlp_hoisted(nlp):
     """The maximal decision-free subexpressions the cost graph (F, g, H) consumes: every non-constant
     argument without a decision symbol below it of a node that has one, and every output without one.
@@ -951,7 +985,7 @@ def nlp_hoisted(nlp):
     return P
 
 
-def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False, rollout_jvp=False):
+def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False, rollout_jvp=False, rollout_vjp=False):
     """Translation unit of the reactive-NLP controller (csrc/clik_nlp.cuh instantiated on the skill)."""
     const_table = [] if os.environ.get("CLIK_CONSTBANK", "1") == "1" else None
     sincos_name = "clik::sincos_fast" if os.environ.get("CLIK_FAST_SINCOS", "1") == "1" else "sincos"
@@ -1059,6 +1093,9 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False, rollout_jvp=
     meta["rollout_jvp"] = bool(rollout_jvp) and meta["jvp"]
     if meta["rollout_jvp"]:
         out.append(_ROLLOUT_JVP_MANIFEST % 2)
+    meta["rollout_vjp"] = bool(rollout_vjp) and meta["vjp"]
+    if meta["rollout_vjp"]:
+        out.append(_ROLLOUT_VJP_MANIFEST % 2)
     out.append("}")
     if meta["duals"]:
         out += ["", "// ---- constraint multipliers of the step's output (clik_duals.cuh) ----",
@@ -1074,6 +1111,8 @@ def _emit_nlp(nlp, label, block_threads, tol, vjp=False, jvp=False, rollout_jvp=
         out += _emit_jvp(nlp, "nlp", sig, sincos_name, block_threads, "Skill", meta["nlp_read_masks"], meta)
     if meta["rollout_jvp"]:
         out += _emit_rollout_jvp("nlp", block_threads)
+    if meta["rollout_vjp"]:
+        out += _emit_rollout_vjp("nlp", block_threads)
     return "\n".join(out) + "\n", meta
 
 

@@ -151,7 +151,9 @@ def vjp_image(ctrl, kind, device, which="vjp"):
     plus clik_<kind>_vjp_kernel, source ctrl._vjp_source()), "jvp" (emit_skill(..., jvp=True): the default image
     plus clik_<kind>_jvp_kernel and clik_<kind>_jacobian_kernel, source ctrl._jvp_source()) or "rollout_jvp"
     (emit_skill(..., jvp=True, rollout_jvp=True): the JVP image plus clik_<kind>_rollout_jvp_kernel and
-    clik_<kind>_rollout_jacobian_kernel, source ctrl._rollout_jvp_source()).  Built and loaded on
+    clik_<kind>_rollout_jacobian_kernel, source ctrl._rollout_jvp_source()) or "rollout_vjp" (emit_skill(...,
+    vjp=True, rollout_vjp=True): the VJP image plus clik_<kind>_rollout_tape_kernel and clik_<kind>_rollout_vjp_kernel,
+    source ctrl._rollout_vjp_source()).  Built and loaded on
     the first call, cached like every cubin, one handle per device: a controller that never asks for derivatives
     compiles nothing more."""
     attr = "_" + which
@@ -350,6 +352,136 @@ def rollout_jacobian(ctrl, kind, time_var0, robot_var, steps, dt, virtual_var, i
         skill.handle, b.N, int(steps), ctypes.c_double(float(dt)), b.tp, b.t_stride, b.qp, b.xp, b.yp,
         *_speeds(max_speed, max_virtual_speed), b.ptr(sol), b.ptr(failed), max_iter, b.ptr(jac), b.stream()))
     return {"sol": sol, "n_failed": failed, "jac": jac}
+
+
+def _rollout_tape(ctrl, kind, b, steps, dt, max_speed, max_virtual_speed, max_iter):
+    """clik_<kind>_rollout_tape for the Batch `b` (state updated in place, the rollout_batch bits) on the current
+    stream -> (sol, n_failed, tape).  The tape is a private buffer of the reverse sweep: step-major (steps, rows, N)
+    blocks in the step kernels' layout, allocated through torch, so that a request that does not fit fails there,
+    before any launch."""
+    steps = int(steps)
+    if steps < 0:
+        raise ValueError("steps must be >= 0")
+    torch, N = b.torch, b.N
+    f64 = lambda rows: torch.empty((steps, rows, N), dtype=torch.float64, device=b.device)  # noqa: E731
+    tape = {"q": f64(ctrl.skill_spec.n_robot_var), "x": f64(ctrl._nxv) if ctrl._nxv else None, "sol": f64(ctrl._qn),
+            "status": torch.empty((steps, N), dtype=torch.int32, device=b.device),
+            "active": torch.empty((steps, 2, N), dtype=torch.int32, device=b.device)}
+    sol, failed = b.empty(ctrl._qn), b.empty(0, "i32")
+    skill = vjp_image(ctrl, kind, b.device_index, "rollout_vjp")
+    runtime.check(getattr(runtime.load_library(), "clik_%s_rollout_tape" % kind)(
+        skill.handle, N, steps, ctypes.c_double(float(dt)), b.tp, b.t_stride, b.qp, b.xp, b.yp,
+        *_speeds(max_speed, max_virtual_speed), b.ptr(sol), b.ptr(failed), max_iter,
+        *[b.ptr(tape[k]) for k in ("q", "x", "sol", "status", "active")], b.stream()))
+    return sol, failed, tape
+
+
+def _cotangent(ctrl, b, a, rows, name):
+    """Validated cotangent (rows, N) of a rollout output: None (zero) or a CUDA float64 tensor on b's device."""
+    if a is None or rows == 0:
+        return None
+    if not runtime._is_torch(a) or a.device != b.device:
+        raise ValueError("%s must be a CUDA tensor on %s like robot_var" % (name, b.device))
+    if tuple(a.shape) != (rows, b.N):
+        raise ValueError("%s must have shape %s" % (name, (rows, b.N)))
+    a = a.contiguous()
+    runtime.dev_ptr(a, "f64", rows * b.N, name)
+    return a
+
+
+def _rollout_sweep(ctrl, kind, b, steps, dt, max_speed, max_virtual_speed, tape, q_bar, x_bar, sol_bar):
+    """clik_<kind>_rollout_vjp over `tape` on the current stream -> (t_bar (N,), q_bar0, x_bar0 | None,
+    y_bar | None)."""
+    nq = ctrl.skill_spec.n_robot_var
+    cot = [_cotangent(ctrl, b, a, r, n) for a, r, n in ((q_bar, nq, "q_bar"), (x_bar, ctrl._nxv, "x_bar"),
+                                                        (sol_bar, ctrl._qn, "sol_bar"))]
+    out = (b.empty(0), b.empty(nq), b.empty(ctrl._nxv) if ctrl._nxv else None, b.empty(ctrl._ny) if ctrl._ny else None)
+    skill = vjp_image(ctrl, kind, b.device_index, "rollout_vjp")
+    runtime.check(getattr(runtime.load_library(), "clik_%s_rollout_vjp" % kind)(
+        skill.handle, b.N, int(steps), ctypes.c_double(float(dt)), b.tp, b.t_stride, b.yp,
+        *_speeds(max_speed, max_virtual_speed), *[b.ptr(tape[k]) for k in ("q", "x", "sol", "status", "active")],
+        *[b.ptr(a) for a in cot], *[b.ptr(a) for a in out], b.stream()))
+    return out
+
+
+def rollout_vjp(ctrl, kind, time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed, max_virtual_speed,
+                max_iter, q_bar, x_bar, sol_bar):
+    """Shared body of ReactiveQPController / ReactiveNLPController.rollout_vjp: the taped rollout (state updated in
+    place, the rollout_batch bits), then the reverse sweep along (q_bar, x_bar, sol_bar), both on the current stream.
+    -> {"sol", "n_failed", "t_bar", "q_bar", "x_bar", "y_bar"}."""
+    b = _rollout_batch(ctrl, "rollout_vjp", time_var0, robot_var, virtual_var, input_var)
+    sol, failed, tape = _rollout_tape(ctrl, kind, b, steps, dt, max_speed, max_virtual_speed, max_iter)
+    tb, qb, xb, yb = _rollout_sweep(ctrl, kind, b, steps, dt, max_speed, max_virtual_speed, tape, q_bar, x_bar,
+                                    sol_bar)
+    return {"sol": sol, "n_failed": failed, "t_bar": tb, "q_bar": qb, "x_bar": xb, "y_bar": yb}
+
+
+_ROLLOUT_FUNCTION = []
+
+
+def _rollout_function():
+    """torch.autograd.Function of a closed-loop rollout: forward the taped rollout, backward the reverse sweep, jvp
+    rollout_jvp."""
+    if _ROLLOUT_FUNCTION:
+        return _ROLLOUT_FUNCTION[0]
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class ControllerRollout(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, ctrl, kind, t0, q, x, y, steps, dt, max_speed, max_virtual_speed, max_iter):
+            qK = q.detach().clone()
+            xK = x.detach().clone() if x is not None else None
+            b = _rollout_batch(ctrl, "rollout_batch_differentiable", t0, qK, xK, y)
+            sol, failed, tape = _rollout_tape(ctrl, kind, b, steps, dt, max_speed, max_virtual_speed, max_iter)
+            ctx.ctrl, ctx.kind, ctx.t0 = ctrl, kind, t0
+            ctx.args = (steps, dt, max_speed, max_virtual_speed, max_iter)
+            ctx.tape = tape
+            ctx.save_for_backward(q, x, y)
+            ctx.save_for_forward(q, x, y)
+            ctx.mark_non_differentiable(failed)
+            return qK, xK, sol, failed
+
+        @staticmethod
+        def jvp(ctx, _ctrl, _kind, t_dot, q_dot, x_dot, y_dot, *unused):
+            q, x, y = ctx.saved_tensors
+            ctrl, t0 = ctx.ctrl, ctx.t0
+            steps, dt, vq, vx, mi = ctx.args
+            c = lambda a: None if a is None else a.contiguous()  # noqa: E731
+            if not torch.is_tensor(t0):
+                t_dot = None
+            qs = q.detach().clone()
+            xs = x.detach().clone() if x is not None else None
+            r = rollout_jvp(ctrl, ctx.kind, t0, qs, steps, dt, xs, y, vq, vx, mi, c(t_dot), c(q_dot),
+                            c(x_dot) if x is not None else None, c(y_dot) if y is not None else None)
+            return r["q_dot"], r["x_dot"], r["sol_dot"], None
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, q_bar, x_bar, sol_bar, _unused):
+            q, x, y = ctx.saved_tensors
+            ctrl, t0 = ctx.ctrl, ctx.t0
+            steps, dt, vq, vx, _ = ctx.args
+            b = _rollout_batch(ctrl, "rollout_batch_differentiable", t0, q, x, y)
+            tb, qb, xb, yb = _rollout_sweep(ctrl, ctx.kind, b, steps, dt, vq, vx, ctx.tape, q_bar, x_bar, sol_bar)
+            ctx.tape = None
+            t_grad = None
+            if torch.is_tensor(t0):
+                t_grad = (tb.sum() if t0.numel() == 1 else tb).reshape(t0.shape).to(t0.dtype)
+            return (None, None, t_grad, qb, xb if x is not None else None, yb if y is not None else None,
+                    None, None, None, None, None)
+
+    _ROLLOUT_FUNCTION.append(ControllerRollout)
+    return ControllerRollout
+
+
+def rollout_batch_differentiable(ctrl, kind, time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                                 max_virtual_speed, max_iter):
+    """Shared body of the controllers' rollout_batch_differentiable: validated like rollout_vjp before anything is
+    built, then the autograd Function."""
+    _rollout_batch(ctrl, "rollout_batch_differentiable", time_var0, robot_var, virtual_var, input_var)
+    return _rollout_function().apply(ctrl, kind, time_var0, robot_var, virtual_var, input_var if ctrl._ny else None,
+                                     steps, dt, max_speed, max_virtual_speed, max_iter)
 
 
 _STEP_FUNCTION = []

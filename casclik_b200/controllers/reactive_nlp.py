@@ -22,7 +22,8 @@ from .. import sym as cs
 from ..codegen import NlpProgram, emit_skill
 from ..sym import dag
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              jacobian_batch, jvp_batch, rollout_jacobian, rollout_jvp, solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, rollout_batch_differentiable, rollout_jacobian, rollout_jvp,
+                              rollout_vjp, solve_batch_differentiable, vjp_batch)
 from .reactive_qp import _weights
 
 #: per-instance outcome of the NLP step (status array): the QP codes plus a stalled line search
@@ -58,6 +59,7 @@ class ReactiveNLPController(BaseController):
         self._vjp = None
         self._jvp = None
         self._rollout_jvp = None
+        self._rollout_vjp = None
         self._has_initial = False
         self.res = None
         self._prog = self._program()     # validates the cost and the problem size now
@@ -134,6 +136,7 @@ class ReactiveNLPController(BaseController):
         self._vjp = None
         self._jvp = None
         self._rollout_jvp = None
+        self._rollout_vjp = None
         if load:
             self._skill()
 
@@ -271,6 +274,25 @@ class ReactiveNLPController(BaseController):
         """rollout_batch with d(q_K, x_K)/d(t0, q0, x0, y), as ReactiveQPController.rollout_jacobian."""
         return rollout_jacobian(self, "nlp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
                                 max_virtual_speed, self._max_iter(max_iter))
+
+    def _rollout_vjp_source(self):
+        """Source of the rollout-VJP image: the VJP image plus the taped rollout and reverse sweep kernels."""
+        return emit_skill(nlp=self._prog, label=self.skill_spec.label, nlp_tol=float(self.options["tol"]), vjp=True,
+                          rollout_vjp=True)
+
+    def rollout_vjp(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                    max_virtual_speed=None, max_iter=None, q_bar=None, x_bar=None, sol_bar=None):
+        """rollout_batch followed by the reverse sweep of the closed loop, as ReactiveQPController.rollout_vjp; each
+        step's cotangent is pulled back with the vjp_batch of its solution (Hessian at sol, no shift: NaN where it
+        is not positive definite).  The dependence of a step on its warm start (below tol) is not differentiated."""
+        return rollout_vjp(self, "nlp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                           max_virtual_speed, self._max_iter(max_iter), q_bar, x_bar, sol_bar)
+
+    def rollout_batch_differentiable(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
+                                     max_speed=None, max_virtual_speed=None, max_iter=None):
+        """rollout_batch as a torch.autograd.Function, as ReactiveQPController.rollout_batch_differentiable."""
+        return rollout_batch_differentiable(self, "nlp", time_var0, robot_var, steps, dt, virtual_var, input_var,
+                                            max_speed, max_virtual_speed, self._max_iter(max_iter))
 
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None, warmstart_slack_var=None):

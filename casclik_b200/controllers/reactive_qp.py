@@ -23,7 +23,8 @@ from .. import build, runtime
 from .. import sym as cs
 from ..codegen import QpProgram, emit_skill
 from .base_controller import (BaseController, Batch, as_vector, dm_column, multipliers_batch, one_instance, run_step,
-                              jacobian_batch, jvp_batch, rollout_jacobian, rollout_jvp, set_overlap, solve_batch_differentiable, vjp_batch)
+                              jacobian_batch, jvp_batch, rollout_batch_differentiable, rollout_jacobian, rollout_jvp,
+                              rollout_vjp, set_overlap, solve_batch_differentiable, vjp_batch)
 from .qp_solver import ConicSolver
 
 
@@ -72,6 +73,7 @@ class ReactiveQPController(BaseController):
         self._vjp = None
         self._jvp = None
         self._rollout_jvp = None
+        self._rollout_vjp = None
         self._has_initial = False
         self.res = None
 
@@ -206,6 +208,7 @@ class ReactiveQPController(BaseController):
         self._vjp = None
         self._jvp = None
         self._rollout_jvp = None
+        self._rollout_vjp = None
         ins, names = self._input_list()
         H = cs.diag(cs.MX(cs.vertcat(*prog.h)))
         A = cs.MX(cs.vertcat(*[cs.horzcat(*row) for row in prog.A]))
@@ -406,6 +409,38 @@ class ReactiveQPController(BaseController):
         mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
         return rollout_jacobian(self, "qp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
                                 max_virtual_speed, mi)
+
+    def _rollout_vjp_source(self):
+        """Source of the rollout-VJP image: the VJP image plus the taped rollout and reverse sweep kernels."""
+        return emit_skill(qp=self._program(), label=self.skill_spec.label, vjp=True, rollout_vjp=True,
+                          qp_fast_min_blocks=self.kernel_meta.get("qp_fast_min_blocks"))
+
+    def rollout_vjp(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None, max_speed=None,
+                    max_virtual_speed=None, max_iter=None, q_bar=None, x_bar=None, sol_bar=None):
+        """rollout_batch (robot_var / virtual_var UPDATED IN PLACE, bit for bit the same states, `sol` and `n_failed`)
+        followed by the reverse sweep of the closed loop: the cotangents q_bar (n_robot, N), x_bar (n_virtual, N) of
+        the final state and sol_bar (nx, N) of `sol` (None is zero) are pulled back to p = (t0, q0, x0, y), one
+        step VJP per step on the step's own solution and working set, masked where the clip max_speed /
+        max_virtual_speed holds (DESIGN.md §4.9).  Returns {"sol", "n_failed", "t_bar" (N,), "q_bar" (n_robot, N),
+        "x_bar" (n_virtual, N) | None, "y_bar" (n_input, N) | None}, the exact adjoint of rollout_jvp; t_bar is per
+        instance also for a shared t0.  A zero cotangent gives exactly 0; an instance whose nonzero cotangent
+        reaches a step with status != 0 or a rank-deficient working set gets NaN everywhere.  The image is compiled
+        and loaded on the first call (one per device); the tape between the two launches takes
+        steps * N * (8 (n_robot + n_virtual + nx) + 12) bytes of device memory.  NumPy inputs and skills with more
+        than 32 constraint rows raise ValueError."""
+        mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
+        return rollout_vjp(self, "qp", time_var0, robot_var, steps, dt, virtual_var, input_var, max_speed,
+                           max_virtual_speed, mi, q_bar, x_bar, sol_bar)
+
+    def rollout_batch_differentiable(self, time_var0, robot_var, steps, dt, virtual_var=None, input_var=None,
+                                     max_speed=None, max_virtual_speed=None, max_iter=None):
+        """rollout_batch as a torch.autograd.Function on torch CUDA tensors: returns new tensors (q_K, x_K | None,
+        sol, n_failed) and modifies no input.  backward() runs the reverse sweep of rollout_vjp over the tape the
+        forward kept (once differentiable), forward-mode AD the tangent of rollout_jvp; n_failed is not
+        differentiable.  A 0-d / one-element tensor t0 gets the summed t_bar; a Python float t0 gets none."""
+        mi = int(max_iter if max_iter is not None else self.options.get("max_iter", 0) or 0)
+        return rollout_batch_differentiable(self, "qp", time_var0, robot_var, steps, dt, virtual_var, input_var,
+                                            max_speed, max_virtual_speed, mi)
 
     def solve(self, time_var, robot_var, virtual_var=None, input_var=None,
               warmstart_robot_vel_var=None, warmstart_virtual_vel_var=None,

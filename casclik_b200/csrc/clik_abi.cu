@@ -96,6 +96,7 @@ struct clik_skill {
   KernelInfo qp_vjp, nlp_vjp;       // reverse-mode derivative of the step (manifest o[19]: bit 0 QP, bit 1 NLP)
   KernelInfo qp_jvp, nlp_jvp, qp_jac, nlp_jac;   // forward-mode derivative and Jacobian (o[20]: bit 0 QP, bit 1 NLP)
   KernelInfo qp_rjvp, nlp_rjvp, qp_rjac, nlp_rjac;   // tangent and Jacobian rollouts (o[21]: bit 0 QP, bit 1 NLP)
+  KernelInfo qp_rtape, nlp_rtape, qp_rvjp, nlp_rvjp;   // taped rollout and reverse sweep (o[22]: bit 0 QP, bit 1 NLP)
   bool qp_split = true;  // CLIK_QP_SPLIT=0: always the single full kernel
   int qp_tail_pick = -1; // CLIK_QP_TAIL_PICK: 0 always the uncapped tail kernel, 1 always the capped one, -1 by batch size
   bool pinv_split = true;     // CLIK_PINV_SPLIT=0: run-time mode tail inside the one kernel (thread mapping)
@@ -534,6 +535,11 @@ clik_status clik_skill_load(const void* cubin, size_t len, const clik_skill_desc
   if (st == CLIK_OK && (rjvp & 1)) st = setup_kernel(s, "clik_qp_rollout_jacobian_kernel", &s->qp_rjac);
   if (st == CLIK_OK && (rjvp & 2)) st = setup_kernel(s, "clik_nlp_rollout_jvp_kernel", &s->nlp_rjvp);
   if (st == CLIK_OK && (rjvp & 2)) st = setup_kernel(s, "clik_nlp_rollout_jacobian_kernel", &s->nlp_rjac);
+  const int rvjp = hsz[22];    // taped rollout + reverse sweep (emit_skill(..., vjp=True, rollout_vjp=True))
+  if (st == CLIK_OK && (rvjp & 1)) st = setup_kernel(s, "clik_qp_rollout_tape_kernel", &s->qp_rtape);
+  if (st == CLIK_OK && (rvjp & 1)) st = setup_kernel(s, "clik_qp_rollout_vjp_kernel", &s->qp_rvjp);
+  if (st == CLIK_OK && (rvjp & 2)) st = setup_kernel(s, "clik_nlp_rollout_tape_kernel", &s->nlp_rtape);
+  if (st == CLIK_OK && (rvjp & 2)) st = setup_kernel(s, "clik_nlp_rollout_vjp_kernel", &s->nlp_rvjp);
   if (st != CLIK_OK) {
     cudaLibraryUnload(s->lib);
     delete s;
@@ -1442,6 +1448,119 @@ clik_status clik_nlp_rollout_jacobian(const clik_skill* s, int64_t N, int32_t st
                                       int32_t* n_failed, int32_t max_iter, double* jac, void* stream) {
   return rollout_jacobian_impl(s, true, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed,
                                sol_last, n_failed, max_iter, jac, stream);
+}
+
+}  // extern "C"
+
+// ---- reverse-mode derivative of the closed-loop rollouts (clik_rollout_vjp.cuh) -----------------------------
+namespace {
+
+clik_status rollout_vjp_kernel_check(const clik_skill* s, const KernelInfo& k, const char* what, bool nlp, int64_t N,
+                                     int32_t steps) {
+  if (!k.kernel)
+    return fail(CLIK_ERR_INVALID, "skill image has no %s %s kernel (build it with emit_skill(..., vjp=True, "
+                "rollout_vjp=True); at most 32 constraint rows)", nlp ? "NLP" : "QP", what);
+  if (N < 0) return fail(CLIK_ERR_INVALID, "N < 0");
+  if (steps < 0) return fail(CLIK_ERR_INVALID, "steps < 0");
+  return CLIK_OK;
+}
+
+clik_status tape_check(const clik_skill* s, int32_t steps, const double* tape_q, const double* tape_x,
+                       const double* tape_sol, const int32_t* tape_status, const uint32_t* tape_active) {
+  if (steps > 0 && (!tape_q || !tape_sol || !tape_status || !tape_active || (s->desc.n_virtual > 0 && !tape_x)))
+    return fail(CLIK_ERR_INVALID, "tape_q, tape_sol, tape_status, tape_active (and tape_x with virtual_var) are "
+                "required when steps > 0");
+  return CLIK_OK;
+}
+
+clik_status rollout_tape_impl(const clik_skill* s, bool nlp, int64_t N, int32_t steps, double dt, const double* t0,
+                              int32_t t_stride, double* q, double* x, const double* y, double vmax_q, double vmax_x,
+                              double* sol_last, int32_t* n_failed, int32_t max_iter, double* tape_q, double* tape_x,
+                              double* tape_sol, int32_t* tape_status, uint32_t* tape_active, void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_rtape : s->qp_rtape;
+  clik_status st = rollout_vjp_kernel_check(s, k, "taped rollout", nlp, N, steps);
+  if (st == CLIK_OK) st = check_common(s, N, t0, q, x, y);
+  if (st != CLIK_OK || N == 0) return st;
+  st = tape_check(s, steps, tape_q, tape_x, tape_sol, tape_status, tape_active);
+  if (st != CLIK_OK) return st;
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0, ks = steps, mi = rollout_max_iter(s, nlp, max_iter);
+  void* args[] = {&n, &l, &ks, &dt, &t0, &ts, &q, &x, &y, &vmax_q, &vmax_x, &sol_last, &n_failed, &mi,
+                  &tape_q, &tape_x, &tape_sol, &tape_status, &tape_active};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+clik_status rollout_vjp_impl(const clik_skill* s, bool nlp, int64_t N, int32_t steps, double dt, const double* t0,
+                             int32_t t_stride, const double* y, double vmax_q, double vmax_x, const double* tape_q,
+                             const double* tape_x, const double* tape_sol, const int32_t* tape_status,
+                             const uint32_t* tape_active, const double* q_bar_K, const double* x_bar_K,
+                             const double* sol_bar, double* t_bar, double* q_bar, double* x_bar, double* y_bar,
+                             void* stream) {
+  if (!s) return fail(CLIK_ERR_INVALID, "skill is NULL");
+  const KernelInfo& k = nlp ? s->nlp_rvjp : s->qp_rvjp;
+  clik_status st = rollout_vjp_kernel_check(s, k, "rollout VJP", nlp, N, steps);
+  if (st != CLIK_OK || N == 0) return st;
+  if (!t0) return fail(CLIK_ERR_INVALID, "t0 is required");
+  if (s->desc.n_input > 0 && !y) return fail(CLIK_ERR_INVALID, "skill reads input_var: y is required");
+  st = tape_check(s, steps, tape_q, tape_x, tape_sol, tape_status, tape_active);
+  if (st != CLIK_OK) return st;
+  if (!t_bar || !q_bar) return fail(CLIK_ERR_INVALID, "t_bar and q_bar are required");
+  if (s->desc.n_virtual > 0 && !x_bar) return fail(CLIK_ERR_INVALID, "skill has virtual_var: x_bar is required");
+  if (s->desc.n_input > 0 && !y_bar) return fail(CLIK_ERR_INVALID, "skill reads input_var: y_bar is required");
+  ON_DEVICE(s->desc.device);
+  long long n = N, l = N;
+  int ts = t_stride ? 1 : 0, ks = steps;
+  void* args[] = {&n, &l, &ks, &dt, &t0, &ts, &y, &vmax_q, &vmax_x, &tape_q, &tape_x, &tape_sol, &tape_status,
+                  &tape_active, &q_bar_K, &x_bar_K, &sol_bar, &t_bar, &q_bar, &x_bar, &y_bar};
+  CK(launch(k, grid_for(k, N), args, (cudaStream_t)stream, false));
+  return CLIK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+clik_status clik_qp_rollout_tape(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                 double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                 double* tape_q, double* tape_x, double* tape_sol, int32_t* tape_status,
+                                 uint32_t* tape_active, void* stream) {
+  return rollout_tape_impl(s, false, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed, sol_last,
+                           n_failed, max_iter, tape_q, tape_x, tape_sol, tape_status, tape_active, stream);
+}
+
+clik_status clik_nlp_rollout_tape(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                  int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                  double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                  double* tape_q, double* tape_x, double* tape_sol, int32_t* tape_status,
+                                  uint32_t* tape_active, void* stream) {
+  return rollout_tape_impl(s, true, N, steps, dt, t0, t_stride, q, x, y, max_robot_speed, max_virtual_speed, sol_last,
+                           n_failed, max_iter, tape_q, tape_x, tape_sol, tape_status, tape_active, stream);
+}
+
+clik_status clik_qp_rollout_vjp(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                int32_t t_stride, const double* y, double max_robot_speed, double max_virtual_speed,
+                                const double* tape_q, const double* tape_x, const double* tape_sol,
+                                const int32_t* tape_status, const uint32_t* tape_active, const double* q_bar_K,
+                                const double* x_bar_K, const double* sol_bar, double* t_bar, double* q_bar,
+                                double* x_bar, double* y_bar, void* stream) {
+  return rollout_vjp_impl(s, false, N, steps, dt, t0, t_stride, y, max_robot_speed, max_virtual_speed, tape_q, tape_x,
+                          tape_sol, tape_status, tape_active, q_bar_K, x_bar_K, sol_bar, t_bar, q_bar, x_bar, y_bar,
+                          stream);
+}
+
+clik_status clik_nlp_rollout_vjp(const clik_skill* s, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, const double* y, double max_robot_speed, double max_virtual_speed,
+                                 const double* tape_q, const double* tape_x, const double* tape_sol,
+                                 const int32_t* tape_status, const uint32_t* tape_active, const double* q_bar_K,
+                                 const double* x_bar_K, const double* sol_bar, double* t_bar, double* q_bar,
+                                 double* x_bar, double* y_bar, void* stream) {
+  return rollout_vjp_impl(s, true, N, steps, dt, t0, t_stride, y, max_robot_speed, max_virtual_speed, tape_q, tape_x,
+                          tape_sol, tape_status, tape_active, q_bar_K, x_bar_K, sol_bar, t_bar, q_bar, x_bar, y_bar,
+                          stream);
 }
 
 clik_status clik_measure_fp64_peak(int32_t device, int32_t iters, double* tflops) {

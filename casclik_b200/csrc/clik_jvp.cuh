@@ -140,6 +140,18 @@ struct QpFace {
     jvp_face_solve<NN>(k, W, Q, R, up, r2u, r2l, c, z);
     for (int j = 0; j < NN; ++j) xd[j] = s[j] * z[j];
   }
+  // the adjoint solve of qp_vjp (the same operations in the same order) for the cotangent xb: K [u; v] = [xb; 0]
+  __device__ __forceinline__ void adjoint(const double (&xb)[NN], double (&u)[NN], double (&v)[M]) const {
+    for (int r = 0; r < M; ++r) v[r] = 0.0;
+    double sg[NN];
+    for (int j = 0; j < NN; ++j) sg[j] = s[j] * -xb[j];
+    working_set_solve<NN>(k, W, Q, R, sg, v);
+    for (int j = 0; j < NN; ++j) {
+      double acc = xb[j];
+      for (int a = 0; a < k; ++a) acc = fma(-d.A[W[a] * NN + j], v[W[a]], acc);
+      u[j] = acc / d.h[j];
+    }
+  }
 };
 
 // The NLP face factorisation of instance i (as nlp_vjp): lam, grad^2 F(x*) = L L' and the QR of L^-1 A_W'.
@@ -153,7 +165,7 @@ struct NlpFace {
   __device__ __forceinline__ bool factor(double t_, const double (&q_)[S::NQ > 0 ? S::NQ : 1],
                                          const double (&x_)[S::NX > 0 ? S::NX : 1],
                                          const double (&y_)[S::NY > 0 ? S::NY : 1], const double (&sol_)[NN], int st,
-                                         unsigned up_, unsigned lo_) {
+                                         unsigned up_, unsigned lo_, double* aw = nullptr) {
     if (st != 0) return false;
     tv = t_;
     for (int j = 0; j < S::NQ; ++j) qv[j] = q_[j];
@@ -177,6 +189,8 @@ struct NlpFace {
     if (!working_set_rows<NN, M>(up, lo, W, k, v)) return false;
     for (int a = 0; a < k; ++a) {
       for (int j = 0; j < NN; ++j) Q[a * NN + j] = d.A[W[a] * NN + j];
+      if (aw != nullptr)   // the rows of A_W, for NlpAdjointFace
+        for (int j = 0; j < NN; ++j) aw[a * NN + j] = Q[a * NN + j];
       nlp_lsolve<NN>(L, &Q[a * NN]);
     }
     return working_set_qr<NN>(k, Q, R);
@@ -198,6 +212,36 @@ struct NlpFace {
     nlp_lsolve<NN>(L, xd);
     jvp_face_solve<NN>(k, W, Q, R, up, r2u, r2l, c, xd);
     nlp_ltsolve<NN>(L, xd);
+  }
+};
+
+// NlpFace that also keeps the rows of A_W, for the adjoint solve of nlp_vjp (the forward-mode kernels do not need
+// them and keep the plain NlpFace).
+template <class S>
+struct NlpAdjointFace : NlpFace<S> {
+  using Base = NlpFace<S>;
+  static constexpr int NN = Base::NN, M = Base::M;
+  double AW[NN * NN];
+  __device__ __forceinline__ bool factor(double t_, const double (&q_)[S::NQ > 0 ? S::NQ : 1],
+                                         const double (&x_)[S::NX > 0 ? S::NX : 1],
+                                         const double (&y_)[S::NY > 0 ? S::NY : 1], const double (&sol_)[NN], int st,
+                                         unsigned up_, unsigned lo_) {
+    return Base::factor(t_, q_, x_, y_, sol_, st, up_, lo_, AW);
+  }
+  // the adjoint solve of nlp_vjp (the same operations in the same order): u = L^-T L^-1 (xb - A_W' v)
+  __device__ __forceinline__ void adjoint(const double (&xb)[NN], double (&u)[NN], double (&v)[M]) const {
+    for (int r = 0; r < M; ++r) v[r] = 0.0;
+    double sg[NN];
+    for (int j = 0; j < NN; ++j) sg[j] = -xb[j];
+    nlp_lsolve<NN>(this->L, sg);
+    working_set_solve<NN>(this->k, this->W, this->Q, this->R, sg, v);
+    for (int j = 0; j < NN; ++j) {
+      double acc = xb[j];
+      for (int a = 0; a < this->k; ++a) acc = fma(-AW[a * NN + j], v[this->W[a]], acc);
+      u[j] = acc;
+    }
+    nlp_lsolve<NN>(this->L, u);
+    nlp_ltsolve<NN>(this->L, u);
   }
 };
 

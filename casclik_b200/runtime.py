@@ -42,6 +42,7 @@ EXPORTS = (
     "clik_qp_solve_one_lam", "clik_nlp_solve_one_lam", "clik_qp_vjp", "clik_nlp_vjp",
     "clik_qp_jvp", "clik_nlp_jvp", "clik_qp_jacobian", "clik_nlp_jacobian",
     "clik_qp_rollout_jvp", "clik_nlp_rollout_jvp", "clik_qp_rollout_jacobian", "clik_nlp_rollout_jacobian",
+    "clik_qp_rollout_tape", "clik_nlp_rollout_tape", "clik_qp_rollout_vjp", "clik_nlp_rollout_vjp",
     "clik_skill_set_staging", "clik_skill_get_staging",
     "clik_measure_fp64_peak", "clik_flush_l2", "clik_device_count", "clik_abi_version",
     "clik_last_error",
@@ -142,6 +143,13 @@ def load_library():
     for name in ("clik_qp_rollout_jacobian", "clik_nlp_rollout_jacobian"):
         getattr(lib, name).restype = i32
         getattr(lib, name).argtypes = rollout + [vp, vp]
+    for name in ("clik_qp_rollout_tape", "clik_nlp_rollout_tape"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = rollout + [vp, vp, vp, vp, vp, vp]
+    for name in ("clik_qp_rollout_vjp", "clik_nlp_rollout_vjp"):
+        getattr(lib, name).restype = i32
+        getattr(lib, name).argtypes = [vp, i64, i32, ctypes.c_double, vp, i32, vp, ctypes.c_double, ctypes.c_double,
+                                       vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.clik_qp_solve_one_lam.restype = i32
     lib.clik_qp_solve_one_lam.argtypes = [vp, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.clik_nlp_solve_one_lam.restype = i32

@@ -386,6 +386,55 @@ clik_status clik_nlp_rollout_jacobian(const clik_skill* skill, int64_t N, int32_
                                       double max_robot_speed, double max_virtual_speed, double* sol_last,
                                       int32_t* n_failed, int32_t max_iter, double* jac, void* stream);
 
+/* Reverse-mode derivative of the closed-loop rollouts clik_qp_rollout / clik_nlp_rollout, for N instances: the exact
+ * adjoint of clik_<kind>_rollout_jvp.  Inputs p = (t0, q0, x0, y) and the primal as there; the caller supplies the
+ * cotangents q_bar_K [n_robot * N], x_bar_K [n_virtual * N] of the final state and sol_bar [qp_n * N] of sol_last
+ * (NULL = zero).  Two launches:
+ *   clik_<kind>_rollout_tape: the arguments of clik_<kind>_rollout (q, x, sol_last, n_failed bit-identical to it; q
+ *     and x updated in place) and a tape of `steps` blocks, step-major, each in the SoA layout of the step kernels
+ *     (row stride N): tape_q [steps * n_robot * N] and tape_x [steps * n_virtual * N] the state at the start of step
+ *     k, tape_sol [steps * qp_n * N] its unclipped solution, tape_status [steps * N] and tape_active
+ *     [steps * 2 * N] its status and working set.  Step k of the tape is a valid input of clik_<kind>_vjp with
+ *     t = t0 + k*dt.  Size: steps * N * (8 * (n_robot + n_virtual + qp_n) + 12) bytes.
+ *   clik_<kind>_rollout_vjp: the sweep over that tape (the same N, steps, dt, t0, t_stride, y and speed limits).
+ *     With a_q = q_bar_K, a_x = x_bar_K, for k = steps-1 ... 0:
+ *       s_bar_k = m_k * (dt*[a_q; a_x; 0] + [k = steps-1]*sol_bar), m_kj = 1 where |sol_kj| < vmax (vmax_q robot
+ *                 part, vmax_x virtual part), 0 where the clip holds (at the bound too); slack entries are 1;
+ *       theta_bar_k = clik_<kind>_vjp at (theta_k, sol_k, status_k, active_k) along s_bar_k: exactly 0 for an
+ *                 all-zero s_bar_k (the face is not factored); otherwise NaN when status_k != 0 (a failed step that
+ *                 applied zero velocity included), A_W is rank-deficient or (NLP) a Cholesky pivot is rejected,
+ *                 and then every cotangent output of the instance is NaN;
+ *       a_q += theta_bar_k.q,  a_x += theta_bar_k.x,  t_bar += theta_bar_k.t,  y_bar += theta_bar_k.y.
+ *     Outputs (required): t_bar [N] (per instance also for a shared t0), q_bar = a_q [n_robot * N], x_bar = a_x
+ *     [n_virtual * N], y_bar [n_input * N].  steps = 0 gives q_bar = q_bar_K, x_bar = x_bar_K, t_bar = y_bar = 0.
+ * As clik_qp_vjp this is the derivative of the face solutions at the returned points: the NLP's dependence on its
+ * warm start is not differentiated.  The kernels are in images built with emit_skill(..., vjp=True,
+ * rollout_vjp=True) (manifest o[22]) only, for skills with a rollout kernel and 1..32 constraint rows.
+ * CLIK_ERR_INVALID for a NULL skill, an image without the kernel, steps < 0, a NULL tape pointer with steps > 0 and
+ * a NULL required input or output.  Device pointers only, asynchronous on `stream`; one thread per instance. */
+clik_status clik_qp_rollout_tape(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                 double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                 double* tape_q, double* tape_x, double* tape_sol, int32_t* tape_status,
+                                 uint32_t* tape_active, void* stream);
+clik_status clik_nlp_rollout_tape(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                  int32_t t_stride, double* q, double* x, const double* y, double max_robot_speed,
+                                  double max_virtual_speed, double* sol_last, int32_t* n_failed, int32_t max_iter,
+                                  double* tape_q, double* tape_x, double* tape_sol, int32_t* tape_status,
+                                  uint32_t* tape_active, void* stream);
+clik_status clik_qp_rollout_vjp(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                int32_t t_stride, const double* y, double max_robot_speed, double max_virtual_speed,
+                                const double* tape_q, const double* tape_x, const double* tape_sol,
+                                const int32_t* tape_status, const uint32_t* tape_active, const double* q_bar_K,
+                                const double* x_bar_K, const double* sol_bar, double* t_bar, double* q_bar,
+                                double* x_bar, double* y_bar, void* stream);
+clik_status clik_nlp_rollout_vjp(const clik_skill* skill, int64_t N, int32_t steps, double dt, const double* t0,
+                                 int32_t t_stride, const double* y, double max_robot_speed, double max_virtual_speed,
+                                 const double* tape_q, const double* tape_x, const double* tape_sol,
+                                 const int32_t* tape_status, const uint32_t* tape_active, const double* q_bar_K,
+                                 const double* x_bar_K, const double* sol_bar, double* t_bar, double* q_bar,
+                                 double* x_bar, double* y_bar, void* stream);
+
 /* One host batch over several GPUs of the box: `skills[k]` is the same cubin loaded on device k
  * (clik_skill_load with desc.device = k); the batch is cut into n_skills contiguous shards (sizes differ
  * by at most one, shard k = [k*N/n .. )), each shard runs on its device from its own host thread (zero
